@@ -241,6 +241,24 @@ WORKLOADS = {
     "rollout": (16384, "PPO rollout loop on the device: MlpPolicy.act_into + step_into per step, trex_gae at the end (BASELINE.json configs[3])"),
 }
 ACTION_SETS = 16  # pre-generated action sets cycled through the timed steps
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this much
+
+
+def dump_outputs(out_dir, arrays):
+    """Write the arrays one step returns (one row per environment) as ``out_dir/<name>.npy`` in float32, so that two builds
+    can be compared output for output.  When they exceed DUMP_BYTES together, every array keeps the same fixed, seeded
+    sample of environments, whose indices go to ``env_index.npy``."""
+    host = {k: v.detach().cpu().numpy().astype(np.float32) for k, v in arrays.items()}
+    n = len(next(iter(host.values())))
+    row_bytes = sum(a[0].nbytes for a in host.values())
+    if n * row_bytes > DUMP_BYTES:
+        keep = (DUMP_BYTES - 4096) // (row_bytes + 8)
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        host = {k: a[idx] for k, a in host.items()}
+        host["env_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def source_hash():
@@ -342,6 +360,10 @@ def run_rollout(args, rank, world, local, dev, use_dist, barrier):
         dist.all_reduce(t_ms, op=dist.ReduceOp.MAX)
     total_ms = float(t_ms.item())
     st = sim.stats()
+    if args.dump_outputs and rank == 0:  # the rows of the loop's last env step
+        dump_outputs(args.dump_outputs, {"obs": buf.obs[T], "action": buf.actions[T - 1], "reward": buf.rewards[T - 1], "done": buf.dones[T],
+                                         "value": buf.values[T - 1], "neglogp": buf.neglogp[T - 1],
+                                         "advantage": buf.advantages[T - 1], "return": buf.returns[T - 1]})
     if rank == 0:
         launches = sim.kernel_launches - l0 + T + 2  # + one policy kernel per step, the bootstrap value, the GAE scan
         line = {
@@ -413,9 +435,11 @@ def run_ours(args):
     for k in range(args.steps):
         flush.fill_(float(k))  # L2 flush between timed steps (not timed)
         evs[k][0].record()
-        step_fn(acts[(phase0 + args.warmup + k) % ring])
+        out = step_fn(acts[(phase0 + args.warmup + k) % ring])
         evs[k][1].record()
     barrier()
+    if args.dump_outputs and rank == 0:  # before the spread and e2e steps overwrite the simulator-owned buffers
+        dump_outputs(args.dump_outputs, dict(zip(("obs", "reward", "done"), out)))
     launches = sim.kernel_launches - launches0
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
     st = sim.stats()
@@ -535,13 +559,16 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed env steps of the loop that gives the value and --dump-outputs (default 20; with --workload rollout the rollout "
+                         "horizon, default 2048).  After it, the e2e figures time 2 x K more steps through the host entry points, and "
+                         "--spread-steps more are timed for the spread")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="random", choices=sorted(WORKLOADS), help="default: BASELINE.json configs[2], the headline")
     ap.add_argument("--envs-per-gpu", type=int, default=0, help="0 = the workload's own batch size (65,536 for the headline)")
     ap.add_argument("--spread-steps", type=int, default=-1, help="extra individually timed steps for the step-time spread (default: 200 for the headline at N=1, else 0)")
-    ap.add_argument("--rollout-horizon", type=int, default=2048)
+    ap.add_argument("--rollout-horizon", type=int, default=None, help="env steps of the timed rollout loop (default: --steps if given, else 2048)")
     ap.add_argument("--substeps", type=int, default=5)
     ap.add_argument("--horizon", type=int, default=0, help="max episode steps (0 = reference behaviour: never terminate)")
     ap.add_argument("--no-contacts", action="store_true", help="literal reference URDF (no collision shapes)")
@@ -549,7 +576,21 @@ def main():
     ap.add_argument("--warps-per-block", type=int, default=0)
     ap.add_argument("--graph", action="store_true", help="device-resident value through the CUDA-graph replay of the step (TrexBatchSim.step_graph)")
     ap.add_argument("--preroll", type=int, default=300, help="untimed env-steps from the reset state before warm-up, so the batch is in its steady regime (on the floor, in contact)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned (rank 0's environments) as "
+                    "DIR/<name>.npy in float32; past 64 MB, a fixed seeded sample of the environments")
     args = ap.parse_args()
+    if args.impl == "ours" and args.workload == "rollout":
+        # the rollout loop is the timed window: its horizon is the number of timed steps
+        if args.steps is not None and args.rollout_horizon is not None and args.steps != args.rollout_horizon:
+            ap.error("--steps and --rollout-horizon both set the timed steps of the rollout loop; give one of them")
+        given = [v for v in (args.rollout_horizon, args.steps) if v is not None]
+        args.steps = args.rollout_horizon = given[0] if given else 2048
+    elif args.steps is None:
+        args.steps = 20
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours: the reference arm times host workers and returns no arrays")
     if args.warmup < 3:
         args.warmup = 3
     if args.spread_steps < 0:

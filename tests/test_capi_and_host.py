@@ -34,24 +34,31 @@ def test_library_exports_every_declared_symbol():
     assert b"sm_100a" in L.trex_version()
 
 
+_NO_CPU_FALLBACK = """
+import ctypes
+import pytest
+from trex_gym_b200 import _native
+from trex_gym_b200.model_compiler import load_builtin
+from trex_gym_b200.sim import TrexBatchSim
+
+with pytest.raises(RuntimeError):
+    TrexBatchSim(4)
+# the C entry point itself also fails loudly instead of computing on the host
+L = _native.lib()
+blob = load_builtin().blob()
+h = ctypes.c_void_p()
+rc = L.trex_create(blob, len(blob), 4, 0, None, ctypes.byref(h))
+assert rc != 0 and not h.value
+assert b"CUDA" in L.trex_last_error() or b"cuda" in L.trex_last_error()
+"""
+
+
 def test_no_cpu_fallback():
-    import torch
-
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from trex_gym_b200 import _native
-    from trex_gym_b200.model_compiler import load_builtin
-    from trex_gym_b200.sim import TrexBatchSim
-
-    with pytest.raises(RuntimeError):
-        TrexBatchSim(4)
-    # the C entry point itself also fails loudly instead of computing on the host
-    L = _native.lib()
-    blob = load_builtin().blob()
-    h = ctypes.c_void_p()
-    rc = L.trex_create(blob, len(blob), 4, 0, None, ctypes.byref(h))
-    assert rc != 0 and not h.value
-    assert b"CUDA" in L.trex_last_error() or b"cuda" in L.trex_last_error()
+    """Without a visible GPU, both the Python class and the C entry point refuse to run.  The check runs in a child
+    process with every GPU hidden, so it also runs on a machine that has one."""
+    out = subprocess.run([sys.executable, "-c", _NO_CPU_FALLBACK], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                         capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
 
 
 def test_product_never_imports_oracle():
@@ -136,6 +143,44 @@ def test_f_alg_formula():
     assert abs(bench.f_alg(5, 60, 0) - 0.98e6) < 0.02e6
     assert abs(bench.f_alg(5, 60, 8) - 1.85e6) < 0.03e6
     assert abs(bench.f_alg(5, 10, 0) - 0.42e6) < 0.02e6
+
+
+def test_dump_outputs_writes_float32_and_samples_past_the_limit(tmp_path, monkeypatch):
+    import torch
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    obs = torch.arange(40 * 75, dtype=torch.float32).reshape(40, 75)
+    done = torch.arange(40, dtype=torch.uint8) % 2
+    bench.dump_outputs(str(tmp_path / "all"), {"obs": obs, "done": done})
+    assert sorted(os.listdir(tmp_path / "all")) == ["done.npy", "obs.npy"]
+    got = np.load(tmp_path / "all" / "done.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, done.numpy())
+    # past the limit: the same seeded rows of every array, the same ones on every call
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4096 + 10 * 76 * 4 + 80)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"obs": obs, "done": done})
+    idx = np.load(tmp_path / "a" / "env_index.npy")
+    assert idx.dtype == np.float64 and len(idx) == 10 and len(set(idx)) == 10
+    assert np.array_equal(np.load(tmp_path / "a" / "obs.npy"), obs.numpy()[idx.astype(int)])
+    assert np.array_equal(np.load(tmp_path / "a" / "done.npy"), done.numpy()[idx.astype(int)])
+    for name in ("env_index", "obs", "done"):
+        assert np.array_equal(np.load(tmp_path / "a" / (name + ".npy")), np.load(tmp_path / "b" / (name + ".npy")))
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= bench.DUMP_BYTES
+
+
+def test_bench_step_count_and_dump_arguments():
+    """--steps is the number of timed steps: for the rollout workload it is the rollout horizon, a second, different count
+    is refused; --steps 0 and a dump from the reference arm (which returns no arrays) are refused."""
+    def run(*a):
+        return subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + list(a), capture_output=True, text=True, timeout=120)
+
+    for a, msg in ((["--workload", "rollout", "--steps", "4", "--rollout-horizon", "8"], "--rollout-horizon"),
+                   (["--steps", "0"], "--steps must be at least 1"),
+                   (["--impl", "reference", "--steps", "1", "--dump-outputs", "x"], "--dump-outputs applies to --impl ours")):
+        out = run(*a)
+        assert out.returncode == 2 and msg in out.stderr, (a, out.stderr[-500:])
 
 
 def test_reference_arm_prints_contract_line():

@@ -273,3 +273,28 @@ def test_pipelined_groups_do_not_change_results(model):
     mask[::3] = 1
     obs = [s.reset(mask).clone() for s in sims]
     assert all(torch.equal(obs[0], x) for x in obs[1:])
+
+
+@pytest.mark.parametrize("workload,envs,rows", [("c2", 0, 4096), ("rollout", 256, 256)])
+def test_bench_dump_outputs_end_to_end(tmp_path, workload, envs, rows):
+    """bench.py --dump-outputs: the timed loop runs exactly --steps steps, the last one's outputs land in DIR as float32
+    with one row per environment, and two runs with the same arguments write the same arrays."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    for d in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", workload, "--envs-per-gpu", str(envs),
+                              "--steps", "3", "--warmup", "3", "--preroll", "5", "--no-cpu-baseline", "--spread-steps", "0",
+                              "--dump-outputs", str(tmp_path / d)], capture_output=True, text=True, timeout=900)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == 3
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert {"obs.npy", "reward.npy", "done.npy"} <= set(names) and names == sorted(os.listdir(tmp_path / "b"))
+    for f in names:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float32 and a.shape[0] == rows and np.isfinite(a).all(), f
+        assert np.array_equal(a, b), f
+    assert np.load(tmp_path / "a" / "obs.npy").shape == (rows, 75)

@@ -1,5 +1,6 @@
 """Model compiler / loader shim: golden numbers of SURVEY.md section 7.1 and Appendix B, regeneration of the
-checked-in blob from the reference URDF (skipped where /root/reference does not exist, e.g. the GPU box)."""
+checked-in blob from the reference URDF (skipped unless TREX_GYM_REFERENCE names a trex-gym checkout: the reference's
+URDF, meshes and parser are not part of this repository)."""
 import json
 import os
 import sys
@@ -7,9 +8,9 @@ import sys
 import numpy as np
 import pytest
 
-REF = "/root/reference"
+REF = os.environ.get("TREX_GYM_REFERENCE", "")
 URDF = os.path.join(REF, "assets", "trex.urdf")
-needs_ref = pytest.mark.skipif(not os.path.isfile(URDF), reason="reference checkout not present")
+needs_ref = pytest.mark.skipif(not (REF and os.path.isfile(URDF)), reason="reference checkout not present (set TREX_GYM_REFERENCE)")
 
 
 def test_golden_numbers(model):
@@ -177,6 +178,13 @@ def test_reference_parser_tests_pass_through_shim():
         assert res.wasSuccessful(), name
         ran += res.testsRun
     assert ran >= 5
+
+
+def test_topology_header_matches_checked_in_model(model):
+    """The kernels' compile-time topology (csrc/trex_topology.h) is the one of the checked-in blob."""
+    from trex_gym_b200.model_compiler import TOPOLOGY_HEADER, emit_topology_header
+
+    assert open(TOPOLOGY_HEADER).read() == emit_topology_header(model)
 
 
 @needs_ref
