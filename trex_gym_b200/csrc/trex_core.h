@@ -11,7 +11,7 @@
 //   lane 25            floating base body; lanes 25..30 own base velocity coordinates 0..5
 //   lane 31            spare
 // * tree passes (kinematics, bias forces, articulated inertias, accelerations) run
-//   level-synchronously: a lane is a body, parents/children talk through warp shuffles;
+//   level-synchronously: a lane is a body, parents/children talk through warp shuffles or shared-memory rows;
 // * the inverse joint-space inertia is built column-per-lane (31 unit-impulse passes run
 //   concurrently, one per lane, reading the per-body data as shared-memory broadcasts).
 //   M^-1 is symmetric, so lane d ends up holding exactly the coefficients it needs to
@@ -132,6 +132,14 @@ struct Uniform {
   int head_depth;
 };
 
+// Lane-major rows read with 128-bit loads: a stride of 4 x an odd number of floats puts the eight lanes of a quarter warp
+// (one 128-bit shared-memory wavefront) on eight different 16-byte bank groups (a stride of 16 would pair lane i with i + 2).
+#define TREX_PACK 20  // k.pack: E (9), U (6), invD, r0 (3), parent lane (int bits)
+#define TREX_XROW 28  // x.rows: articulated inertia (21) and bias force (6) in the parent's frame, 1 float of padding
+static_assert(TREX_PACK % 8 == 4 && TREX_XROW % 8 == 4, "row strides must be 4 x an odd number of floats");
+// 128-bit store of four consecutive floats by every lane (the predicate of st4_if is always true and folds away)
+TREX_FN void st4_every_lane(float* p, vi idx, const vf v[4]) { st4_if(p, idx, v, lane_id() >= 0); }
+
 // per-warp shared memory slab.  The kinematics-phase arrays (k) and the contact-row arrays (c) are
 // never live at the same time and share storage; 13.7 KB per warp at KMAX = 16 -> 16 warps per SM (two per CTA).
 struct alignas(16) WarpShared {
@@ -148,7 +156,7 @@ struct alignas(16) WarpShared {
       float invD[32];
       float Rw[9][32];    // world -> body rotation
       float xw[3][32];    // body origin, world
-      float pack[32][16]; // per body lane: E (9), U (6), invD -- the same data body-major, for 128-bit broadcast loads
+      float pack[32][TREX_PACK];  // per body lane: E (9), U (6), invD, r0 (3), parent lane -- body-major, for 128-bit loads
     } k;
     struct {
       float dV[3 * TREX_KMAX][32];   // rows 3*c + {0 normal, 1 t1, 2 t2}: M^-1 J^T, indexed by lane
@@ -156,21 +164,24 @@ struct alignas(16) WarpShared {
       unsigned char slot[TREX_KMAX][32];  // which Jc entry each lane multiplies its velocity coordinate with
       unsigned char inv[TREX_KW][16];     // inverse of slot: lane (coordinate) of each Jc entry
     } c;
-    struct {                  // exchange with the four-environments-per-warp inward pass (front kernel, 4-warp CTAs):
+    struct {                  // the inward pass (both variants) and its exchange with the four-environments-per-warp pass:
       float keep[28][32];     // k.E .. k.xw stay live (k.pack is written after the pass)
       float pA[6][32];        // bias force per body lane (in), later unused
       float cc[5][32];        // Coriolis terms c0 c1 c3 c4 and the joint damping torque (in)
       float uu[32];           // tau - S^T pA per joint (out)
-      float Ip[21][32];       // articulated inertia of each body in its parent's frame (scratch between levels)
-      float pp[6][32];        // ... and its bias force
+      float rows[32][TREX_XROW];  // per body lane: its articulated inertia and bias force in the parent's frame, handed
+                                  // from the children to the parent between levels
       float base[32];         // [0:21] articulated inertia of the base, [21:27] its bias force (out)
     } x;
   };
 };
 static_assert(sizeof(((WarpShared*)0)->x) <= sizeof(((WarpShared*)0)->c), "exchange area must fit the union");
-static_assert(sizeof(((WarpShared*)0)->x.keep) == 28 * 128, "exchange area must start behind k.E .. k.xw");
+static_assert(sizeof(((WarpShared*)0)->x.keep) == offsetof(WarpShared, k.pack) - offsetof(WarpShared, k.E),
+              "exchange area must start behind k.E .. k.xw");
+static_assert(offsetof(WarpShared, x.rows) % 16 == 0 && offsetof(WarpShared, k.pack) % 16 == 0 && sizeof(WarpShared) % 16 == 0,
+              "rows of 128-bit accesses");
 // link-damping partial wrenches live in dV rows beyond the kinematics-phase arrays
-#define TREX_PART_ROW 44  // row (of 32 floats) inside the union where the 6 damping partial rows live
+#define TREX_PART_ROW 48  // row (of 32 floats) inside the union where the 6 damping partial rows live
 static_assert(sizeof(((WarpShared*)0)->k) <= TREX_PART_ROW * 128, "partials must not overlap the kinematics arrays");
 static_assert(sizeof(((WarpShared*)0)->c) >= (TREX_PART_ROW + 6) * 128, "contact-row storage too small for the damping scratch");
 
@@ -439,7 +450,7 @@ TREX_FN void inward_packed(const Uniform& P, const float* mdl, const int* mdli, 
   const vi eo = e * (int)(sizeof(WarpShared) / sizeof(float));
   constexpr int O_E = offsetof(WarpShared, k.E) / 4, O_U = offsetof(WarpShared, k.U) / 4, O_ID = offsetof(WarpShared, k.invD) / 4;
   constexpr int O_PA = offsetof(WarpShared, x.pA) / 4, O_CC = offsetof(WarpShared, x.cc) / 4, O_UU = offsetof(WarpShared, x.uu) / 4;
-  constexpr int O_IP = offsetof(WarpShared, x.Ip) / 4, O_PP = offsetof(WarpShared, x.pp) / 4, O_BASE = offsetof(WarpShared, x.base) / 4;
+  constexpr int O_ROWS = offsetof(WarpShared, x.rows) / 4, O_BASE = offsetof(WarpShared, x.base) / 4;
   // the body this lane handles at each level: the i-th of depth d (depth 0: the base, lane 0 of the group)
   vi blv[MAX_DEPTH + 1];
   blv[0] = seli(i == 0, vi(25), vi(-1));
@@ -488,9 +499,11 @@ TREX_FN void inward_packed(const Uniform& P, const float* mdl, const int* mdli, 
         const vi cl = (children >> (6 * sidx)) & 63;
         const vb ok = has && (cl != 63);
         const vi cls = seli(ok, cl, bl);
-        // (select, not a 0/1 factor: a row that was never written may hold anything, 0 * NaN included)
-        TREX_UNROLL for (int k = 0; k < 21; k++) IA[k] = IA[k] + sel(ok, ld(sb, eo + cls + (O_IP + k * 32)), 0.0f);
-        TREX_UNROLL for (int k = 0; k < 6; k++) pA[k] = pA[k] + sel(ok, ld(sb, eo + cls + (O_PP + k * 32)), 0.0f);
+        // (+0 without the child, not a 0/1 factor: a row that was never written may hold anything, 0 * NaN included)
+        vf row[TREX_XROW];
+        TREX_UNROLL for (int j = 0; j < TREX_XROW / 4; j++) ld4_if(sb, eo + O_ROWS + cls * TREX_XROW + 4 * j, ok, row + 4 * j);
+        TREX_UNROLL for (int k = 0; k < 21; k++) IA[k] = IA[k] + row[k];
+        TREX_UNROLL for (int k = 0; k < 6; k++) pA[k] = pA[k] + row[21 + k];
       }
     }
     if (d == 0) {  // the base: hand its articulated inertia and bias force to the environment's warp
@@ -520,10 +533,10 @@ TREX_FN void inward_packed(const Uniform& P, const float* mdl, const int* mdli, 
     const vf s = ut * iD;
     TREX_UNROLL for (int a = 0; a < 6; a++)  // (row 2 of Ia is zero)
       pa[a] = a == 2 ? pA[a] + Ut[a] * s : pA[a] + (Ia[SI(a, 0)] * c0 + Ia[SI(a, 1)] * c1 + Ia[SI(a, 3)] * c3 + Ia[SI(a, 4)] * c4) + Ut[a] * s;
-    vf Ip[21], pp[6];
-    to_parent(E, r0, Ia, pa, Ip, pp);
-    TREX_UNROLL for (int k = 0; k < 21; k++) st_if(sb, eo + bl + (O_IP + k * 32), Ip[k], has);
-    TREX_UNROLL for (int k = 0; k < 6; k++) st_if(sb, eo + bl + (O_PP + k * 32), pp[k], has);
+    vf row[TREX_XROW];  // Ip (21), pp (6), padding
+    to_parent(E, r0, Ia, pa, row, row + 21);
+    row[27] = 0.0f;
+    TREX_UNROLL for (int j = 0; j < TREX_XROW / 4; j++) st4_if(sb, eo + O_ROWS + bl * TREX_XROW + 4 * j, row + 4 * j, has);
     warp_sync();
   }
 #undef TREX_LOAD_LEVEL_CONSTANTS
@@ -564,8 +577,11 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
   TREX_UNROLL for (int k = 0; k < 9; k++) E[k] = sel(is_base, vbroadcast(Rb[k]), E[k]);
   vf Rw[9], xw[3], v[6];
   forward_pass<true>(mdl, mdli, lane, R, Rb, E, Rw, xw, v);
-  TREX_UNROLL for (int k = 0; k < 9; k++) { st(S.k.E[k], lane, E[k]); st(S.k.Rw[k], lane, Rw[k]); }
+  TREX_UNROLL for (int k = 0; k < 9; k++) st(S.k.Rw[k], lane, Rw[k]);
   TREX_UNROLL for (int k = 0; k < 3; k++) st(S.k.xw[k], lane, xw[k]);
+  if (PACKED) {  // input of inward_packed
+    TREX_UNROLL for (int k = 0; k < 9; k++) st(S.k.E[k], lane, E[k]);
+  }
 
   TREX_TICK(0)
   // ---- 3. bias forces: p = v x* (I v) - gravity wrench + angular damping ------------------
@@ -691,10 +707,17 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
     const vf s = ut * iD;
     TREX_UNROLL for (int i = 0; i < 6; i++)  // (row 2 of Ia is zero)
       pa[i] = i == 2 ? pA[i] + Ut[i] * s : pA[i] + (Ia[SI(i, 0)] * c0 + Ia[SI(i, 1)] * c1 + Ia[SI(i, 3)] * c3 + Ia[SI(i, 4)] * c4) + Ut[i] * s;
-    vf Ip[21], pp[6];
-    to_parent(E, r0, Ia, pa, Ip, pp);
-    // parents (depth d-1) gather from their children (all at depth d); only as many child slots as any body
-    // of that depth has (tree constant), accumulated with a 0/1 mask through one FMA per element
+    vf row[TREX_XROW];  // Ip (21), pp (6), padding
+    to_parent(E, r0, Ia, pa, row, row + 21);
+    row[27] = 0.0f;
+    // parents (depth d-1) gather from their children (all at depth d) through the lane-major rows of x.rows (seven
+    // 128-bit accesses per row); only as many child slots as any body of that depth has (tree constant), accumulated
+    // with a 0/1 mask through one FMA per element.  Every lane publishes its row and a lane without that child reads
+    // back its own, written this level: its masked FMA adds 0 * its own value, never 0 * a stale NaN.
+    float* rows = &S.x.rows[0][0];
+    warp_sync();  // the previous level's gather is done with the rows
+    TREX_UNROLL for (int j = 0; j < TREX_XROW / 4; j++) st4_every_lane(rows, lane * TREX_XROW + 4 * j, row + 4 * j);
+    warp_sync();
     const vb parent_now = depth == (d - 1);
     const int nslots = P.max_children[d - 1];
     TREX_ROLLED for (int sidx = 0; sidx < nslots; sidx++) {
@@ -702,27 +725,29 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
       const vb ok = parent_now && (cl != 63);
       const vi cls = seli(ok, cl, lane);
       const vf okf = sel(ok, 1.0f, 0.0f);
-      TREX_UNROLL for (int k = 0; k < 21; k++) IA[k] = vfma(okf, shflv(Ip[k], cls), IA[k]);
-      TREX_UNROLL for (int k = 0; k < 6; k++) pA[k] = vfma(okf, shflv(pp[k], cls), pA[k]);
+      vf ch[TREX_XROW];
+      TREX_UNROLL for (int j = 0; j < TREX_XROW / 4; j++) ld4(rows, cls * TREX_XROW + 4 * j, ch + 4 * j);
+      TREX_UNROLL for (int k = 0; k < 21; k++) IA[k] = vfma(okf, ch[k], IA[k]);
+      TREX_UNROLL for (int k = 0; k < 6; k++) pA[k] = vfma(okf, ch[21 + k], pA[k]);
     }
   }
   float ia0[21], pA0[6], a0[6];
   if (PACKED) {
     TREX_UNROLL for (int k = 0; k < 21; k++) ia0[k] = ldu(S.x.base, k);
     TREX_UNROLL for (int k = 0; k < 6; k++) pA0[k] = ldu(S.x.base, 21 + k);
-    warp_sync();  // pack overwrites the exchange area
   } else {
     TREX_UNROLL for (int k = 0; k < 21; k++) ia0[k] = lane_value(IA[k], 25);
     TREX_UNROLL for (int k = 0; k < 6; k++) pA0[k] = lane_value(pA[k], 25);
-    TREX_UNROLL for (int k = 0; k < 6; k++) st(S.k.U[k], lane, U[k]);
-    st(S.k.invD, lane, invD);
   }
+  warp_sync();  // pack overwrites the exchange area
   {
-    vf pk[16];
+    vf pk[TREX_PACK];
     TREX_UNROLL for (int k = 0; k < 9; k++) pk[k] = E[k];
     TREX_UNROLL for (int k = 0; k < 6; k++) pk[9 + k] = U[k];
     pk[15] = invD;
-    st16(&S.k.pack[0][0], lane * 16, pk);
+    TREX_UNROLL for (int k = 0; k < 3; k++) pk[16 + k] = r0[k];
+    pk[19] = vi2f_bits(plane);
+    TREX_UNROLL for (int j = 0; j < TREX_PACK / 4; j++) st4_every_lane(&S.k.pack[0][0], lane * TREX_PACK + 4 * j, pk + 4 * j);
   }
 
   TREX_TICK(2)
@@ -780,13 +805,18 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
     TREX_UNROLL for (int k = 0; k < 6; k++) z[k] = sel(is_joint, U[k] * invD, 0.0f);
     vf Ydep[MAX_DEPTH + 1];
     TREX_UNROLL for (int dd = 0; dd <= MAX_DEPTH; dd++) Ydep[dd] = sel(is_joint && (depth == dd), 1.0f, 0.0f);
-    vi cur = lane;
+    // E, r0 and the parent lane of the body the walk has reached (while it is active): this lane's own to begin
+    // with, then the parent's pack row, loaded in the step before for its U and 1/D
+    vf Ec[9], rc[3];
+    vi par = plane;
+    TREX_UNROLL for (int k = 0; k < 9; k++) Ec[k] = E[k];
+    TREX_UNROLL for (int k = 0; k < 3; k++) rc[k] = r0[k];
     TREX_ROLLED for (int s = 0; s < MAX_DEPTH; s++) {
       const vb active = is_joint && ((depth - s) >= 1);
-      const vi cs = seli(active, cur, lane);
-      vf Ec[9], rc[3];
-      TREX_UNROLL for (int k = 0; k < 9; k++) Ec[k] = ld(S.k.E[k], cs);
-      TREX_UNROLL for (int k = 0; k < 3; k++) rc[k] = ldg_ro(mdl, cs + (F_R0 + k) * 32);
+      const vb par_joint = active && (par != 25);
+      const vi ps = seli(par_joint, par, lane);
+      vf pr[TREX_PACK];
+      TREX_UNROLL for (int j = 0; j < TREX_PACK / 4; j++) ld4(&S.k.pack[0][0], ps * TREX_PACK + 4 * j, pr + 4 * j);
       vf fn[3], ff[3];
       TREX_UNROLL for (int i = 0; i < 3; i++) {
         fn[i] = Ec[i] * z[0] + Ec[3 + i] * z[1] + Ec[6 + i] * z[2];
@@ -797,19 +827,16 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
       zn[1] = fn[1] + (rc[2] * ff[0] - rc[0] * ff[2]);
       zn[2] = fn[2] + (rc[0] * ff[1] - rc[1] * ff[0]);
       zn[3] = ff[0]; zn[4] = ff[1]; zn[5] = ff[2];
-      const vi par = ldi(mdli, cs + IF_PARENT_LANE * 32);
-      const vb par_joint = active && (par != 25);
-      const vi ps = seli(par_joint, par, lane);
       // at a joint parent: Y = -S^T z ; z += U * Y / D
       const vf Yp = -zn[2];
-      const vf sc = Yp * ld(S.k.invD, ps);
-      TREX_UNROLL for (int k = 0; k < 6; k++) {
-        const vf up = ld(S.k.U[k], ps);
-        z[k] = sel(active, sel(par_joint, zn[k] + up * sc, zn[k]), z[k]);
-      }
+      const vf sc = Yp * pr[15];
+      TREX_UNROLL for (int k = 0; k < 6; k++) z[k] = sel(active, sel(par_joint, zn[k] + pr[9 + k] * sc, zn[k]), z[k]);
       const vi pd = depth - s - 1;
       TREX_UNROLL for (int dd = 1; dd <= MAX_DEPTH; dd++) Ydep[dd] = sel(par_joint && (pd == dd), Yp, Ydep[dd]);
-      cur = seli(active, par, cur);
+      // the walk stays active only while it is below a joint parent, so the row just loaded is the next step's
+      TREX_UNROLL for (int k = 0; k < 9; k++) Ec[k] = pr[k];
+      TREX_UNROLL for (int k = 0; k < 3; k++) rc[k] = pr[16 + k];
+      par = vf2i_bits(pr[19]);
     }
     // base-coordinate lanes: unit torque / force on the base, rotated into base coordinates
     {
@@ -834,7 +861,7 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
       const int bl = b - 1;
       const int dep = P.depth[b];
       float pk[16];
-      ldu16(&S.k.pack[0][0], bl * 16, pk);  // four 128-bit broadcast loads
+      ldu16(&S.k.pack[0][0], bl * TREX_PACK, pk);  // four 128-bit broadcast loads
       const float* Eb = pk;
       const float* Ub = pk + 9;
       const float iDb = pk[15];
