@@ -111,7 +111,10 @@ typedef struct trex_config {
                                 (persistent 4-warp CTAs, tcgen05.ld 32x32b as a lane-private scratchpad: the shared-memory instance
                                 runs at 69 % of the shared-memory data pipe's wavefront peak), TREX_CONTACT_SHARED in shared memory.
                                 Results are bit-identical. */
-  int32_t reserved[7];       /* must be zero */
+  int32_t env_params;        /* 0 (default): every environment simulates the model's own constants.  1: the handle owns a
+                                per-environment parameter record (trex_set_env_params below) and runs the kernel instances that
+                                read it; rows start as the model's constants, which reproduce the env_params = 0 results bit for bit */
+  int32_t reserved[6];       /* must be zero */
 } trex_config;
 
 typedef struct trex_stats {
@@ -160,6 +163,33 @@ int trex_reset_host(trex_handle* h, float* obs_host);
 /* Simulator-state checkpoint / parity hooks: copy the environment records out / in (device pointers). */
 int trex_get_state(trex_handle* h, float* state_dev, void* stream);
 int trex_set_state(trex_handle* h, const float* state_dev, void* stream);
+/* Per-environment dynamics parameters (handles created with trex_config.env_params = 1; TREX_ERR_INVALID otherwise).
+ * The record is float32 [N][TREX_ENV_PARAM_DIM], one row per environment; each element replaces, for that environment only,
+ * what a pybullet client sets with the call named beside it:
+ *   [0:25]  mass scale of the body of joint k (pybullet link order, fixed links merged in)   changeDynamics(mass=, localInertiaDiagonal=)
+ *   [25]    mass scale of the base body                                                        changeDynamics(-1, mass=, localInertiaDiagonal=)
+ *           (uniform density scaling: mass, first moment, inertia, angular-damping tensor and link-damping masses; the COM stays)
+ *   [26]    friction coefficient of the foot-floor contacts (the combined value)               changeDynamics(lateralFriction=)
+ *   [27]    motor position gain kp, [28] velocity gain kd                                      setJointMotorControlArray(positionGains=, velocityGains=)
+ *   [29]    motor max torque, N m                                                              setJointMotorControlArray(forces=)
+ *   [30]    motor impulse bound = [29] * dt, computed in double by the library (the value passed is ignored)
+ *   [31]    reserved, 0
+ * Defaults (every row after trex_create): scales 1, then the model's friction, motor_kp, motor_kd, motor_max_torque.  Reset
+ * steps keep zero motor gains, as with env_params = 0; mass scales and friction apply to them.
+ * trex_get_state / trex_set_state do not carry the record: a checkpoint saves it with trex_get_env_params. */
+#define TREX_ENV_PARAM_DIM 32
+/* rows of params_dev [N][32] (device) -> the record: all rows, or (mask_dev uint8[N] on the device, optional) those with
+ * mask != 0; element 30 is recomputed.  Stream ordered, capturable. */
+int trex_set_env_params(trex_handle* h, const float* params_dev, const uint8_t* mask_dev, void* stream);
+int trex_get_env_params(trex_handle* h, float* params_dev, void* stream);
+/* Randomizer (domain randomization): while set, every reset of an environment -- trex_reset (masked too) and the auto-reset on
+ * done -- first draws its row: element k = lo[k] + u (hi[k] - lo[k]), u in [0,1) from Philox4x32-10 keyed by the seed and
+ * counted by (env_offset + env, episode, k / 4), so rows do not depend on the number of GPUs and lo == hi gives lo exactly;
+ * element 30 follows from the drawn 29.  Host arrays of 32 floats: lo <= hi, finite, mass scales > 0, friction, gains and
+ * torque >= 0, elements 30 and 31 zero.  NULL / NULL turns the randomizer off.  Synchronises the device (resets already
+ * enqueued use the previous ranges); a CUDA graph keeps the setting it was captured with. */
+int trex_set_env_param_ranges(trex_handle* h, const float* lo32_host, const float* hi32_host);
+
 /* per-env diagnostics of the last step: head xyz (trex_robot.py:330-335), the three penalty terms
  * logged at trex_env.py:193-195 (lifting, station keeping, energy), PGS iterations, contacts. */
 int trex_get_aux(trex_handle* h, float* aux_dev, void* stream);

@@ -17,11 +17,13 @@ NUM_JOINTS = 25
 OBS_DIM = 75
 STATE_DIM = 160
 AUX_DIM = 8
+ENV_PARAM_DIM = 32  # per-environment parameter row (include/trex_b200.h, trex_set_env_params)
 
 EXPORTED_SYMBOLS = (
     "trex_create", "trex_destroy", "trex_reset", "trex_step", "trex_step_host", "trex_step_host_async", "trex_host_wait",
     "trex_reset_host",
     "trex_get_state", "trex_set_state", "trex_get_aux", "trex_get_joint_limits",
+    "trex_set_env_params", "trex_get_env_params", "trex_set_env_param_ranges",
     "trex_fill_random_actions", "trex_get_stats", "trex_measure_fp32_peak", "trex_gae", "trex_normalize",
     "trex_policy_param_count", "trex_policy_forward", "trex_kernel_launches", "trex_num_envs",
     "trex_last_error", "trex_version",
@@ -46,7 +48,8 @@ class TrexConfig(ctypes.Structure):
         ("heavy_memory", ctypes.c_int32),
         ("chunk_envs", ctypes.c_int32),
         ("contact_memory", ctypes.c_int32),
-        ("reserved", ctypes.c_int32 * 7),
+        ("env_params", ctypes.c_int32),
+        ("reserved", ctypes.c_int32 * 6),
     ]
 
 
@@ -121,6 +124,12 @@ def lib():
         f = getattr(L, name)
         f.restype = ctypes.c_int
         f.argtypes = [vp, fp, vp]
+    L.trex_set_env_params.restype = ctypes.c_int
+    L.trex_set_env_params.argtypes = [vp, fp, u8p, vp]
+    L.trex_get_env_params.restype = ctypes.c_int
+    L.trex_get_env_params.argtypes = [vp, fp, vp]
+    L.trex_set_env_param_ranges.restype = ctypes.c_int
+    L.trex_set_env_param_ranges.argtypes = [vp, fp, fp]
     L.trex_get_joint_limits.restype = ctypes.c_int
     L.trex_get_joint_limits.argtypes = [vp, fp, fp]
     L.trex_fill_random_actions.restype = ctypes.c_int

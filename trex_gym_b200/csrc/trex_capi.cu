@@ -36,6 +36,9 @@ static_assert(TREX_STATE_DIM == TREX_STATE_STRIDE, "state record size");
 static_assert(TREX_AUX_DIM == TREX_AUX_STRIDE, "aux record size");
 #endif
 static_assert(trex::F_COUNT == 32, "float field table");
+static_assert(TREX_ENV_PARAM_DIM == TREX_ENVP_DIM && TREX_ENVP_DIM == (int)trex_host::ENVP_DIM &&
+              (int)trex::EP_MAX_IMPULSE == (int)trex_host::ENVP_MAX_IMPULSE && (int)trex::EP_MU == (int)trex_host::ENVP_MU &&
+              (int)trex::EP_MAX_TORQUE == (int)trex_host::ENVP_MAX_TORQUE, "parameter row layout");
 
 namespace {
 
@@ -57,13 +60,15 @@ int fail(int code, const char* fmt, const char* detail = "") {
 // ------------------------------------------------------------------------------------------------
 // one warp per environment: dynamics front end of one physics substep (+ the whole substep when the solve is not deferred).
 // PACKED (4 warps per CTA): the inward pass of the CTA's four environments is done by warp 0, four environments at a time.
-template <int WARPS, bool PACKED>
+// ENVP (trex_config.env_params): every environment's mass scales, friction and motor settings come from its row of envp
+// (indexed like state); without it envp is unused and the instance is the one the library had before the record existed.
+template <int WARPS, bool PACKED, bool ENVP>
 __global__ void __launch_bounds__(32 * WARPS, TREX_MIN_BLOCKS / WARPS)
 trex_front_kernel(const trex::Uniform P, const float* __restrict__ mdl, const int* __restrict__ mdli,
                   const float* __restrict__ tasks, const float* __restrict__ cand_p, const int* __restrict__ cand_lane,
                   float* __restrict__ state, float* __restrict__ work, float* __restrict__ workh, const float* __restrict__ action,
                   int* __restrict__ list, int* __restrict__ list_count, const int* __restrict__ heavy_hint, int heavy_div, int n_envs,
-                  int first_round) {
+                  int first_round, const float* __restrict__ envp) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   trex::WarpShared* slabs = reinterpret_cast<trex::WarpShared*>(smem_raw);
   const int warp = threadIdx.x >> 5;
@@ -83,11 +88,12 @@ trex_front_kernel(const trex::Uniform P, const float* __restrict__ mdl, const in
 #ifdef TREX_PHASES
   const long long t_entry = clock64();
 #endif
-  const int front_result = trex::front_phase<PACKED>(P, mdl, mdli, tasks, cand_p, cand_lane, slabs[warp], state + (size_t)env * TREX_STATE_STRIDE,
+  const int front_result = trex::front_phase<PACKED, ENVP>(P, mdl, mdli, tasks, cand_p, cand_lane, slabs[warp], state + (size_t)env * TREX_STATE_STRIDE,
                                                   work ? work + (size_t)env * TREX_WORK_STRIDE : nullptr, action + (size_t)env * trex::NJ,
                                                   first_round != 0, slabs, warp, valid_mask,
                                                   // class 5 (more than TREX_KC contacts) always goes to its own solver unless heavy_share_div asks for the batch-dependent rule
-                                                  (workh != nullptr && (heavy_div <= 0 || (long long)(*heavy_hint) * heavy_div <= (long long)n_envs)) ? workh + (size_t)env * TREX_HEAVY_STRIDE : nullptr);
+                                                  (workh != nullptr && (heavy_div <= 0 || (long long)(*heavy_hint) * heavy_div <= (long long)n_envs)) ? workh + (size_t)env * TREX_HEAVY_STRIDE : nullptr,
+                                                  ENVP ? envp + (size_t)env * TREX_ENVP_DIM : nullptr);
   const int deferred = front_result & 255, n_contacts = front_result >> 8;
   // append to the list of its class of deferred environments (any order: the solver's lane groups are independent):
   // class 0 = contact-free substeps, classes 1..4 = 1 / 2 / 3-4 / 5-8 contacts, 5 = more; list c at list + c * n_envs, counters + 64 * c
@@ -111,10 +117,10 @@ trex_front_kernel(const trex::Uniform P, const float* __restrict__ mdl, const in
 // registers per thread -- 16 instead of 12 warps per SM contact-free, 12 instead of 8 for a 1-2-contact instance: +11 % and
 // +30 % step time.  And the contact instance held to 6 / 4 warps per SM by extra shared memory: +1 % / +10 %.  These kernels
 // are not bound by the number of resident warps.)
-template <int WARPS, int KC, int CLO, int CHI>
+template <int WARPS, int KC, int CLO, int CHI, bool ENVP>
 __global__ void __launch_bounds__(32 * WARPS, (KC ? TREX_SOLVEC_MIN_BLOCKS : TREX_SOLVE_MIN_BLOCKS) / WARPS)
 trex_solve_kernel(const trex::Uniform P, float* __restrict__ state, const float* __restrict__ work,
-                  const int* __restrict__ list, const int* __restrict__ list_count, int n_envs) {
+                  const int* __restrict__ list, const int* __restrict__ list_count, int n_envs, const float* __restrict__ envp) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* scratch = reinterpret_cast<float*>(smem_raw) + (threadIdx.x >> 5) * TREX_SOLVE_SCRATCH(KC);
   const int warp = threadIdx.x >> 5;
@@ -136,16 +142,17 @@ trex_solve_kernel(const trex::Uniform P, float* __restrict__ state, const float*
   if (first >= count) return;
   int envs[4] = {0, 0, 0, 0}, pending = 0;
   for (int e = 0; e < 4 && first + e < count; e++) { envs[e] = list[first + e]; pending |= 1 << e; }
-  trex::solve_phase<KC>(P, scratch, work, state, envs, pending);
+  trex::solve_phase<KC, false, ENVP>(P, scratch, work, state, envs, pending, tmem_t(), envp);
 }
 
 // The contact solver with its Delassus blocks and sweep responses in TENSOR MEMORY (solve4<TREX_KC, true>): persistent 4-warp
 // CTAs (the four warps of a CTA reach the four 32-lane quarters of its tensor-memory columns), 256 columns per CTA, two CTAs =
 // 8 warps per SM.  Warps pull tasks (four environments of one class, heaviest class first) from a counter.
-template <int CLO, int CHI>
+template <int CLO, int CHI, bool ENVP>
 __global__ void __launch_bounds__(128, 2)
 trex_solve_tm_kernel(const trex::Uniform P, float* __restrict__ state, const float* __restrict__ work,
-                     const int* __restrict__ list, const int* __restrict__ list_count, int* __restrict__ next_task, int n_envs) {
+                     const int* __restrict__ list, const int* __restrict__ list_count, int* __restrict__ next_task, int n_envs,
+                     const float* __restrict__ envp) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int warp = threadIdx.x >> 5;
   float* scratch = reinterpret_cast<float*>(smem_raw) + warp * TREX_SOLVE_SCRATCH_TM(TREX_KC);
@@ -169,7 +176,7 @@ trex_solve_tm_kernel(const trex::Uniform P, float* __restrict__ state, const flo
     const int count = list_count[64 * c], first = 4 * t;
     int envs[4] = {0, 0, 0, 0}, pending = 0;
     for (int e = 0; e < 4 && first + e < count; e++) { envs[e] = lst[first + e]; pending |= 1 << e; }
-    trex::solve_phase<TREX_KC, true>(P, scratch, work, state, envs, pending, tm);
+    trex::solve_phase<TREX_KC, true, ENVP>(P, scratch, work, state, envs, pending, tm, envp);
     __syncwarp();
   }
   tmem_free_cta<TREX_S4_TMEM_COLS>(tm.base - ((uint32_t)(warp & 3) << 21));
@@ -181,11 +188,11 @@ trex_solve_tm_kernel(const trex::Uniform P, float* __restrict__ state, const flo
 //   TM = true : 4-warp CTAs, the Delassus matrices in TENSOR MEMORY (256 columns per CTA: 2 CTAs = 8 warps per SM),
 //               11.4 KB of shared memory per warp
 //   TM = false: 1-warp CTAs, the Delassus matrices in shared memory (29.8 KB per warp): they fill the shared memory left
-template <int WARPS, bool TM>
+template <int WARPS, bool TM, bool ENVP>
 __global__ void __launch_bounds__(32 * WARPS)
 trex_heavy_kernel(const trex::Uniform P, float* __restrict__ state, const float* __restrict__ work, const float* __restrict__ workh,
                   const int* __restrict__ list, const int* __restrict__ list_count, const int* __restrict__ seen, int* __restrict__ hint,
-                  int* __restrict__ next_task) {
+                  int* __restrict__ next_task, const float* __restrict__ envp) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int warp = threadIdx.x >> 5;
   float* scratch = reinterpret_cast<float*>(smem_raw) + warp * (TM ? TREX_SOLVE2_SCRATCH_TM : TREX_SOLVE2_SCRATCH);
@@ -204,29 +211,42 @@ trex_heavy_kernel(const trex::Uniform P, float* __restrict__ state, const float*
     if (i >= count) break;
     const bool two = i + 1 < count;
     const int envs[2] = {list[i], two ? list[i + 1] : 0};
-    trex::heavy_phase<TM>(P, scratch, tm, work, workh, state, envs, two ? 3 : 1);
+    trex::heavy_phase<TM, ENVP>(P, scratch, tm, work, workh, state, envs, two ? 3 : 1, envp);
     __syncwarp();
   }
   if (TM) tmem_free_cta<TREX_S2_TMEM_COLS>(tm.base - ((uint32_t)(warp & 3) << 21));
 }
 
 // one warp per environment: reward / done / auto-reset / observations (mode 0), or reset only (mode 1, optional mask)
-template <int WARPS>
+// ENVP: mass scales and friction of each environment's row apply to its reset step; ranges != nullptr: every reset first draws
+// the environment's row (the randomizer; dt = physics substep in double, for the impulse bound)
+template <int WARPS, bool ENVP>
 __global__ void __launch_bounds__(32 * WARPS, TREX_MIN_BLOCKS / WARPS)
 trex_tail_kernel(const trex::Uniform P, const float* __restrict__ mdl, const int* __restrict__ mdli,
                  const float* __restrict__ tasks, const float* __restrict__ cand_p, const int* __restrict__ cand_lane,
                  float* __restrict__ state, float* __restrict__ obs, float* __restrict__ reward, uint8_t* __restrict__ done,
-                 float* __restrict__ aux, const uint8_t* __restrict__ mask, int n_envs, int mode) {
+                 float* __restrict__ aux, const uint8_t* __restrict__ mask, int n_envs, int mode, float* envp,
+                 const float* __restrict__ ranges, double dt) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   trex::WarpShared* slabs = reinterpret_cast<trex::WarpShared*>(smem_raw);
   const int warp = threadIdx.x >> 5;
   const int env = blockIdx.x * WARPS + warp;
   if (env >= n_envs) return;
   if (mode == 1 && mask != nullptr && mask[env] == 0) return;
-  trex::tail_phase(P, mdl, mdli, tasks, cand_p, cand_lane, slabs[warp], state + (size_t)env * TREX_STATE_STRIDE,
+  trex::tail_phase<ENVP>(P, mdl, mdli, tasks, cand_p, cand_lane, slabs[warp], state + (size_t)env * TREX_STATE_STRIDE,
                    obs ? obs + (size_t)env * (3 * trex::NJ) : nullptr, (mode == 0 && reward) ? reward + env : nullptr,
                    (mode == 0 && done) ? done + env : nullptr, (mode == 0 && aux) ? aux + (size_t)env * TREX_AUX_STRIDE : nullptr,
-                   mode == 1, (long long)env);
+                   mode == 1, (long long)env, ENVP ? envp + (size_t)env * TREX_ENVP_DIM : nullptr, ranges, dt);
+}
+
+// trex_set_env_params: rows (all, or those with mask != 0) from the caller's buffer, the impulse bound recomputed in double
+__global__ void __launch_bounds__(256)
+trex_set_env_params_kernel(float* __restrict__ envp, const float* __restrict__ src, const uint8_t* __restrict__ mask, double dt, int n_envs) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const int env = i / TREX_ENVP_DIM, k = i % TREX_ENVP_DIM;
+  if (env >= n_envs || (mask != nullptr && mask[env] == 0)) return;
+  const float* row = src + (size_t)env * TREX_ENVP_DIM;
+  envp[i] = k == trex::EP_MAX_IMPULSE ? (float)((double)row[trex::EP_MAX_TORQUE] * dt) : row[k];
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -411,6 +431,11 @@ struct trex_handle {
   int heavy_mode = 0;           // 0: both instances concurrently; 1: shared memory only; 2: tensor memory only (TREX_HEAVY_MODE, measurement aid)
   int64_t launches = 0;
   int64_t env_steps = 0;
+  // per-environment dynamics parameters (trex_config.env_params = 1): d_envp [n_envs][TREX_ENVP_DIM]; the randomizer's ranges
+  // d_envp_ranges (lo [32] | hi [32]) are used while ranges_on
+  bool envp_on = false, ranges_on = false;
+  float *d_envp = nullptr, *d_envp_ranges = nullptr;
+  double dt = 0.0;              // physics substep in double (the motor impulse bound = torque * dt)
 };
 
 namespace {
@@ -436,7 +461,7 @@ struct HostIO {
   uint8_t* done;
 };
 
-template <int WF, int WS>
+template <int WF, int WS, bool ENVP>
 int launch_step(trex_handle* h, const float* action, float* obs, float* reward, uint8_t* done, const uint8_t* mask,
                 int mode, cudaStream_t st, const HostIO* io = nullptr) {
   static const size_t extra_c = getenv("TREX_SOLVEC_EXTRA_SMEM") ? (size_t)atoi(getenv("TREX_SOLVEC_EXTRA_SMEM")) : 0;  // measurement aid: fewer resident warps
@@ -450,13 +475,13 @@ int launch_step(trex_handle* h, const float* action, float* obs, float* reward, 
   std::lock_guard<std::mutex> guard(configure_lock);
   if (!configured[h->device & 15]) {
     int rc;
-    if ((rc = configure_kernel(trex_front_kernel<WF, WF == 4>, smem_f)) != TREX_OK) return rc;
-    if ((rc = configure_kernel(trex_solve_kernel<WS, 0, 0, 0>, smem_s)) != TREX_OK) return rc;
-    if ((rc = configure_kernel(trex_solve_kernel<WS, TREX_KC, 1, TREX_CLASS_HEAVY - 1>, smem_c)) != TREX_OK) return rc;
-    if ((rc = configure_kernel(trex_solve_tm_kernel<1, TREX_CLASS_HEAVY - 1>, smem_ct)) != TREX_OK) return rc;
-    if ((rc = configure_kernel(trex_heavy_kernel<1, false>, smem_h)) != TREX_OK) return rc;
-    if ((rc = configure_kernel(trex_heavy_kernel<4, true>, smem_ht)) != TREX_OK) return rc;
-    if ((rc = configure_kernel(trex_tail_kernel<WF>, smem_f)) != TREX_OK) return rc;
+    if ((rc = configure_kernel(trex_front_kernel<WF, WF == 4, ENVP>, smem_f)) != TREX_OK) return rc;
+    if ((rc = configure_kernel(trex_solve_kernel<WS, 0, 0, 0, ENVP>, smem_s)) != TREX_OK) return rc;
+    if ((rc = configure_kernel(trex_solve_kernel<WS, TREX_KC, 1, TREX_CLASS_HEAVY - 1, ENVP>, smem_c)) != TREX_OK) return rc;
+    if ((rc = configure_kernel(trex_solve_tm_kernel<1, TREX_CLASS_HEAVY - 1, ENVP>, smem_ct)) != TREX_OK) return rc;
+    if ((rc = configure_kernel(trex_heavy_kernel<1, false, ENVP>, smem_h)) != TREX_OK) return rc;
+    if ((rc = configure_kernel(trex_heavy_kernel<4, true, ENVP>, smem_ht)) != TREX_OK) return rc;
+    if ((rc = configure_kernel(trex_tail_kernel<WF, ENVP>, smem_f)) != TREX_OK) return rc;
     configured[h->device & 15] = true;
   }
   if (h->n_pipes > 1) CUDA_TRY(cudaEventRecord(h->ev_start, st));
@@ -491,10 +516,11 @@ int launch_step(trex_handle* h, const float* action, float* obs, float* reward, 
     float* state = h->d_state + e0 * TREX_STATE_STRIDE;
     float* work = h->d_work ? h->d_work + q.work_slot * TREX_WORK_STRIDE : nullptr;
     float* workh = h->d_workh ? h->d_workh + q.work_slot * TREX_HEAVY_STRIDE : nullptr;
+    float* envp = ENVP ? h->d_envp + e0 * TREX_ENVP_DIM : nullptr;  // rows indexed like state
     for (int r = 0; r < n_rounds; r++) {
-      trex_front_kernel<WF, WF == 4><<<grid1, 32 * WF, smem_f, s>>>(Pc, h->d_mdl, h->d_mdli, h->d_tasks, h->d_cand_p, h->d_cand_lane,
+      trex_front_kernel<WF, WF == 4, ENVP><<<grid1, 32 * WF, smem_f, s>>>(Pc, h->d_mdl, h->d_mdli, h->d_tasks, h->d_cand_p, h->d_cand_lane,
                                                           state, work, workh, action + e0 * trex::NJ, q.d_list, q.d_list_count + r,
-                                                          q.d_list_count + 64 * (TREX_NCLASS + 2), h->heavy_div, count, r == 0);
+                                                          q.d_list_count + 64 * (TREX_NCLASS + 2), h->heavy_div, count, r == 0, envp);
       CUDA_TRY(cudaGetLastError());
       h->launches++;
       if (stagger && c == 0 && r == 0) CUDA_TRY(cudaEventRecord(h->ev_stagger, s));
@@ -516,15 +542,15 @@ int launch_step(trex_handle* h, const float* action, float* obs, float* reward, 
         int* hint = q.d_list_count + 64 * (TREX_NCLASS + 2);
         CUDA_TRY(cudaStreamWaitEvent(q.side, q.ev_fork, 0));
         if (h->heavy_mode != 1) {  // the tensor-memory instance first: its CTAs take their two slots per SM ...
-          trex_heavy_kernel<4, true><<<h->heavy_grid_tm, 128, smem_ht, q.side>>>(Pc, state, work, workh, lst, cnt, q.d_list_count + 64 * TREX_NCLASS + r, hint, next_task);
+          trex_heavy_kernel<4, true, ENVP><<<h->heavy_grid_tm, 128, smem_ht, q.side>>>(Pc, state, work, workh, lst, cnt, q.d_list_count + 64 * TREX_NCLASS + r, hint, next_task, envp);
           CUDA_TRY(cudaGetLastError());
           h->launches++;
         }
         if (h->heavy_mode != 2) {  // ... and the shared-memory instance fills what is left of the shared memory
           cudaStream_t sh = h->heavy_mode == 0 ? q.side3 : q.side;
           if (h->heavy_mode == 0) CUDA_TRY(cudaStreamWaitEvent(q.side3, q.ev_fork, 0));
-          trex_heavy_kernel<1, false><<<h->heavy_mode == 0 ? h->heavy_grid_mixed : h->heavy_grid, 32, smem_h, sh>>>(
-              Pc, state, work, workh, lst, cnt, q.d_list_count + 64 * TREX_NCLASS + r, h->heavy_mode == 0 ? nullptr : hint, next_task);
+          trex_heavy_kernel<1, false, ENVP><<<h->heavy_mode == 0 ? h->heavy_grid_mixed : h->heavy_grid, 32, smem_h, sh>>>(
+              Pc, state, work, workh, lst, cnt, q.d_list_count + 64 * TREX_NCLASS + r, h->heavy_mode == 0 ? nullptr : hint, next_task, envp);
           CUDA_TRY(cudaGetLastError());
           h->launches++;
           if (h->heavy_mode == 0) {
@@ -535,18 +561,18 @@ int launch_step(trex_handle* h, const float* action, float* obs, float* reward, 
         CUDA_TRY(cudaEventRecord(q.ev_join, q.side));
       }
       if (contacts && h->solve_tm) {
-        trex_solve_tm_kernel<1, TREX_CLASS_HEAVY - 1><<<h->solve_tm_grid, 128, smem_ct, s>>>(Pc, state, work, q.d_list, q.d_list_count + r,
-                                                                                         q.d_list_count + 64 * (TREX_NCLASS + 3) + r, count);
+        trex_solve_tm_kernel<1, TREX_CLASS_HEAVY - 1, ENVP><<<h->solve_tm_grid, 128, smem_ct, s>>>(Pc, state, work, q.d_list, q.d_list_count + r,
+                                                                                         q.d_list_count + 64 * (TREX_NCLASS + 3) + r, count, envp);
         CUDA_TRY(cudaGetLastError());
         h->launches++;
       } else if (contacts) {
-        trex_solve_kernel<WS, TREX_KC, 1, TREX_CLASS_HEAVY - 1><<<grid4 + 4, 32 * WS, smem_c, s>>>(Pc, state, work, q.d_list, q.d_list_count + r, count);
+        trex_solve_kernel<WS, TREX_KC, 1, TREX_CLASS_HEAVY - 1, ENVP><<<grid4 + 4, 32 * WS, smem_c, s>>>(Pc, state, work, q.d_list, q.d_list_count + r, count, envp);
         CUDA_TRY(cudaGetLastError());
         h->launches++;
       }
       cudaStream_t s0 = split ? q.side2 : s;
       if (split) CUDA_TRY(cudaStreamWaitEvent(q.side2, q.ev_fork, 0));
-      trex_solve_kernel<WS, 0, 0, 0><<<grid4, 32 * WS, smem_s, s0>>>(Pc, state, work, q.d_list, q.d_list_count + r, count);
+      trex_solve_kernel<WS, 0, 0, 0, ENVP><<<grid4, 32 * WS, smem_s, s0>>>(Pc, state, work, q.d_list, q.d_list_count + r, count, envp);
       CUDA_TRY(cudaGetLastError());
       h->launches++;
       if (split) {
@@ -555,10 +581,11 @@ int launch_step(trex_handle* h, const float* action, float* obs, float* reward, 
       }
       if (heavy) CUDA_TRY(cudaStreamWaitEvent(s, q.ev_join, 0));
     }
-    trex_tail_kernel<WF><<<grid1, 32 * WF, smem_f, s>>>(Pc, h->d_mdl, h->d_mdli, h->d_tasks, h->d_cand_p, h->d_cand_lane,
+    trex_tail_kernel<WF, ENVP><<<grid1, 32 * WF, smem_f, s>>>(Pc, h->d_mdl, h->d_mdli, h->d_tasks, h->d_cand_p, h->d_cand_lane,
                                                         h->d_state + e0 * TREX_STATE_STRIDE, obs ? obs + e0 * 3 * trex::NJ : nullptr,
                                                         reward ? reward + e0 : nullptr, done ? done + e0 : nullptr,
-                                                        h->d_aux + e0 * TREX_AUX_STRIDE, mask ? mask + e0 : nullptr, count, mode);
+                                                        h->d_aux + e0 * TREX_AUX_STRIDE, mask ? mask + e0 : nullptr, count, mode, envp,
+                                                        ENVP && h->ranges_on ? h->d_envp_ranges : nullptr, h->dt);
     CUDA_TRY(cudaGetLastError());
     h->launches++;
     if (io) {
@@ -576,10 +603,13 @@ int launch_step(trex_handle* h, const float* action, float* obs, float* reward, 
 
 int dispatch_step(trex_handle* h, const float* action, float* obs, float* reward, uint8_t* done, const uint8_t* mask,
                   int mode, cudaStream_t st, const HostIO* io = nullptr) {
-  switch (h->warps_per_block) {
-    case 1: return launch_step<1, 2>(h, action, obs, reward, done, mask, mode, st, io);
-    case 2: return launch_step<2, 1>(h, action, obs, reward, done, mask, mode, st, io);
-    case 4: return launch_step<4, 4>(h, action, obs, reward, done, mask, mode, st, io);
+  switch (h->warps_per_block * 2 + (h->envp_on ? 1 : 0)) {
+    case 2: return launch_step<1, 2, false>(h, action, obs, reward, done, mask, mode, st, io);
+    case 4: return launch_step<2, 1, false>(h, action, obs, reward, done, mask, mode, st, io);
+    case 8: return launch_step<4, 4, false>(h, action, obs, reward, done, mask, mode, st, io);
+    case 3: return launch_step<1, 2, true>(h, action, obs, reward, done, mask, mode, st, io);
+    case 5: return launch_step<2, 1, true>(h, action, obs, reward, done, mask, mode, st, io);
+    case 9: return launch_step<4, 4, true>(h, action, obs, reward, done, mask, mode, st, io);
     default: return fail(TREX_ERR_INVALID, "warps_per_block must be 1, 2 or 4%s");
   }
 }
@@ -660,7 +690,12 @@ int trex_create(const void* model_blob, size_t bytes, int32_t n_envs, int32_t de
       return fail(TREX_ERR_INVALID, "trex_config.heavy_memory must be one of TREX_HEAVY_*%s");
     }
     h->heavy_mode = cfg->heavy_memory;
-    for (int i = 0; i < 7; i++)
+    if (cfg->env_params != 0 && cfg->env_params != 1) {
+      delete h;
+      return fail(TREX_ERR_INVALID, "trex_config.env_params must be 0 or 1%s");
+    }
+    h->envp_on = cfg->env_params == 1;
+    for (int i = 0; i < 6; i++)
       if (cfg->reserved[i] != 0) {
         delete h;
         return fail(TREX_ERR_INVALID, "trex_config.reserved must be zero%s");
@@ -685,14 +720,15 @@ int trex_create(const void* model_blob, size_t bytes, int32_t n_envs, int32_t de
     if (h->n_pipes > h->n_chunks) h->n_pipes = h->n_chunks;
   }
   trex_host::fill_uniform(h->T, h->C, h->P);
+  h->dt = trex_host::substep_dt(h->T, h->C.num_substeps);
   {
     // trex_heavy_kernel strides over its list with a fixed grid: exactly the CTAs that are resident at once (a larger
     // grid would run its surplus CTAs as a second wave after the first has walked the whole list)
     int sms = 148, per_sm = 7;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-    cudaFuncSetAttribute(trex_heavy_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(float) * TREX_SOLVE2_SCRATCH));
-    cudaFuncSetAttribute(trex_heavy_kernel<1, false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, trex_heavy_kernel<1, false>, 32, sizeof(float) * TREX_SOLVE2_SCRATCH) != cudaSuccess || per_sm < 1)
+    cudaFuncSetAttribute(trex_heavy_kernel<1, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(float) * TREX_SOLVE2_SCRATCH));
+    cudaFuncSetAttribute(trex_heavy_kernel<1, false, false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, trex_heavy_kernel<1, false, false>, 32, sizeof(float) * TREX_SOLVE2_SCRATCH) != cudaSuccess || per_sm < 1)
       per_sm = 7;
     if (sms > 0) {
       h->heavy_grid = sms * per_sm;
@@ -760,6 +796,15 @@ int trex_create(const void* model_blob, size_t bytes, int32_t n_envs, int32_t de
   CTRY(cudaMemset(h->d_aux, 0, N * TREX_AUX_STRIDE * sizeof(float)));
   // (the staging buffers of the host-buffer entry points are allocated on first use: ensure_host_path)
   CTRY(cudaMalloc((void**)&h->d_stats, sizeof(DevStats)));
+  if (h->envp_on) {  // every row starts as the model's own constants
+    float row[TREX_ENVP_DIM];
+    trex_host::default_env_params(h->T, h->C.num_substeps, row);
+    std::vector<float> rows(N * TREX_ENVP_DIM);
+    for (size_t i = 0; i < rows.size(); i++) rows[i] = row[i % TREX_ENVP_DIM];
+    CTRY(cudaMalloc((void**)&h->d_envp, rows.size() * sizeof(float)));
+    CTRY(cudaMemcpy(h->d_envp, rows.data(), rows.size() * sizeof(float), cudaMemcpyHostToDevice));
+    CTRY(cudaMalloc((void**)&h->d_envp_ranges, 2 * TREX_ENVP_DIM * sizeof(float)));
+  }
 #undef CTRY
   // all environments start from the reference reset (TrexBulletEnv.__init__ calls reset(), trex_env.py:92)
   rc = trex_reset(h, nullptr, nullptr, nullptr);
@@ -778,6 +823,7 @@ void trex_destroy(trex_handle* h) {
   cudaFree(h->d_mdl); cudaFree(h->d_mdli); cudaFree(h->d_tasks); cudaFree(h->d_cand_p); cudaFree(h->d_cand_lane);
   cudaFree(h->d_work); cudaFree(h->d_workh);
   cudaFree(h->d_lower); cudaFree(h->d_upper); cudaFree(h->d_state); cudaFree(h->d_aux); cudaFree(h->d_stats);
+  cudaFree(h->d_envp); cudaFree(h->d_envp_ranges);
   for (int b = 0; b < 2; b++) {
     cudaFree(h->d_action[b]); cudaFree(h->d_obs[b]); cudaFree(h->d_reward[b]); cudaFree(h->d_done[b]);
     if (h->ev_step_done[b]) cudaEventDestroy(h->ev_step_done[b]);
@@ -930,6 +976,46 @@ int trex_set_state(trex_handle* h, const float* state_dev, void* stream) {
   CUDA_TRY(cudaSetDevice(h->device));
   CUDA_TRY(cudaMemcpyAsync(h->d_state, state_dev, (size_t)h->n_envs * TREX_STATE_STRIDE * sizeof(float), cudaMemcpyDeviceToDevice,
                            (cudaStream_t)stream));
+  return TREX_OK;
+}
+
+int trex_set_env_params(trex_handle* h, const float* params_dev, const uint8_t* mask_dev, void* stream) {
+  if (!h || !params_dev) return fail(TREX_ERR_INVALID, "NULL argument%s");
+  if (!h->envp_on) return fail(TREX_ERR_INVALID, "trex_set_env_params: the handle was created with env_params = 0%s");
+  CUDA_TRY(cudaSetDevice(h->device));
+  const int total = h->n_envs * TREX_ENVP_DIM;
+  trex_set_env_params_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(h->d_envp, params_dev, mask_dev, h->dt, h->n_envs);
+  CUDA_TRY(cudaGetLastError());
+  h->launches++;
+  return TREX_OK;
+}
+
+int trex_get_env_params(trex_handle* h, float* params_dev, void* stream) {
+  if (!h || !params_dev) return fail(TREX_ERR_INVALID, "NULL argument%s");
+  if (!h->envp_on) return fail(TREX_ERR_INVALID, "trex_get_env_params: the handle was created with env_params = 0%s");
+  CUDA_TRY(cudaSetDevice(h->device));
+  CUDA_TRY(cudaMemcpyAsync(params_dev, h->d_envp, (size_t)h->n_envs * TREX_ENVP_DIM * sizeof(float), cudaMemcpyDeviceToDevice,
+                           (cudaStream_t)stream));
+  return TREX_OK;
+}
+
+int trex_set_env_param_ranges(trex_handle* h, const float* lo32_host, const float* hi32_host) {
+  if (!h) return fail(TREX_ERR_INVALID, "handle is NULL%s");
+  if (!h->envp_on) return fail(TREX_ERR_INVALID, "trex_set_env_param_ranges: the handle was created with env_params = 0%s");
+  if (!lo32_host && !hi32_host) {
+    h->ranges_on = false;
+    return TREX_OK;
+  }
+  if (!lo32_host || !hi32_host) return fail(TREX_ERR_INVALID, "trex_set_env_param_ranges: pass both ranges or neither%s");
+  if (const char* why = trex_host::check_env_param_ranges(lo32_host, hi32_host)) return fail(TREX_ERR_INVALID, "trex_set_env_param_ranges: %s", why);
+  CUDA_TRY(cudaSetDevice(h->device));
+  float both[2 * TREX_ENVP_DIM];
+  memcpy(both, lo32_host, TREX_ENVP_DIM * sizeof(float));
+  memcpy(both + TREX_ENVP_DIM, hi32_host, TREX_ENVP_DIM * sizeof(float));
+  // resets already enqueued (on any stream) finish with the old ranges before the new ones land
+  CUDA_TRY(cudaDeviceSynchronize());
+  CUDA_TRY(cudaMemcpy(h->d_envp_ranges, both, sizeof both, cudaMemcpyHostToDevice));
+  h->ranges_on = true;
   return TREX_OK;
 }
 

@@ -218,6 +218,19 @@ struct StepStats {
 #define MDL(f) ldg_ro(mdl, lane + (f) * 32)
 #define MDLI(f) ldi(mdli, lane + (f) * 32)
 
+// ---- per-environment dynamics parameters (trex_config.env_params = 1; the ENVP instances of the kernels) ----------------
+// One row of 32 floats per environment, lane L reads element L (one 128-byte access per warp):
+//   [0, 25)  mass scale of the body of joint L (body L + 1)    [25] mass scale of the base body
+//   [26] friction coefficient   [27] motor kp   [28] motor kd   [29] motor max torque (N m)
+//   [30] motor impulse bound = [29] * dt, rounded from double (written by the library only)   [31] reserved, 0
+// A mass scale multiplies the body's mass, first moment, rotational inertia, angular-damping tensor and the masses of its
+// link-damping tasks (uniform density scaling: the COM stays).  Lanes 26..31 hold no body and keep scale 1.
+#define TREX_ENVP_DIM 32  // (trex_model.h mirrors the layout for the host: ENVP_*)
+enum { EP_MASS_BASE = 25, EP_MU = 26, EP_KP = 27, EP_KD = 28, EP_MAX_TORQUE = 29, EP_MAX_IMPULSE = 30 };
+// the randomizer's Philox key word (the reset sampler uses 0xfa11: the two streams stay independent)
+#define TREX_ENVP_PHILOX_KEY 0xe9a5u
+TREX_FN vf envp_mass_scale(const float* envp, vi lane) { return ld_if(envp, seli(lane <= EP_MASS_BASE, lane, 0), lane <= EP_MASS_BASE, 1.0f); }
+
 // btClamp semantics: comparison based, so a NaN stays a NaN (fmin/fmax would launder it into a bound)
 TREX_FN vf clampv(vf x, float lo, float hi) { return sel(x < lo, lo, sel(x > hi, hi, x)); }
 TREX_FN float clampf(float x, float lo, float hi) { return x < lo ? lo : (x > hi ? hi : x); }
@@ -442,7 +455,11 @@ TREX_FN void finish_substep(const Uniform& P, vi lane, EnvRegs& R, vf dv, vf lam
 // shared slabs (WarpShared::x); children hand their transformed inertia to the parent through the slab as well.
 // Same operations in the same order as the one-environment pass: bit-identical results.
 // ------------------------------------------------------------------------------------------
-TREX_FN void inward_packed(const Uniform& P, const float* mdl, const int* mdli, WarpShared* slabs, int valid_mask) {
+// ENVP: envp_cta = parameter row of the CTA's first environment (the four rows are consecutive); the level constants of a
+// body are scaled by its mass scale in its environment's row
+template <bool ENVP = false>
+TREX_FN void inward_packed(const Uniform& P, const float* mdl, const int* mdli, WarpShared* slabs, int valid_mask,
+                           const float* envp_cta = nullptr) {
   const vi lane = lane_id();
   const vi e = lane >> 3, i = lane & 7;
   const vb env_ok = ((vi(valid_mask) >> e) & 1) != 0;
@@ -456,11 +473,13 @@ TREX_FN void inward_packed(const Uniform& P, const float* mdl, const int* mdli, 
   blv[0] = seli(i == 0, vi(25), vi(-1));
   TREX_UNROLL for (int d = 1; d <= MAX_DEPTH; d++) blv[d] = ldi(mdli, i + (IF_LEVEL + d - 1) * 32);
   // model constants of the body, loaded one level ahead (global loads off the level-to-level dependence chain)
-  vf n_mass, n_mc[3], n_I3[6], n_r0[3];
+  vf n_mass, n_mc[3], n_I3[6], n_r0[3], n_sc = 1.0f;
   vi n_children;
+  const vi ep_row = seli(env_ok, e, 0) * TREX_ENVP_DIM;
 #define TREX_LOAD_LEVEL_CONSTANTS(BL)                                                       \
   {                                                                                         \
     const vi b_ = (BL);                                                                     \
+    if (ENVP) n_sc = ld(envp_cta, ep_row + b_);                                             \
     n_mass = ldg_ro(mdl, b_ + F_MASS * 32);                                                 \
     TREX_UNROLL for (int k = 0; k < 3; k++) n_mc[k] = ldg_ro(mdl, b_ + (F_MC + k) * 32);    \
     TREX_UNROLL for (int k = 0; k < 6; k++) n_I3[k] = ldg_ro(mdl, b_ + (F_I + k) * 32);     \
@@ -478,10 +497,10 @@ TREX_FN void inward_packed(const Uniform& P, const float* mdl, const int* mdli, 
     const vi bl = seli(has, bl0, 0);
     // own spatial inertia (model constants) and the bias force computed by the environment's own warp
     vf mc[3], I3[6], r0[3], pA[6];
-    const vf mass = n_mass;
+    const vf mass = ENVP ? n_mass * n_sc : n_mass;
     const vi children = n_children;
-    TREX_UNROLL for (int k = 0; k < 3; k++) { mc[k] = n_mc[k]; r0[k] = n_r0[k]; }
-    TREX_UNROLL for (int k = 0; k < 6; k++) I3[k] = n_I3[k];
+    TREX_UNROLL for (int k = 0; k < 3; k++) { mc[k] = ENVP ? n_mc[k] * n_sc : n_mc[k]; r0[k] = n_r0[k]; }
+    TREX_UNROLL for (int k = 0; k < 6; k++) I3[k] = ENVP ? n_I3[k] * n_sc : n_I3[k];
     if (d > 0) TREX_LOAD_LEVEL_CONSTANTS(seli(env_ok && (bln >= 0), bln, 0))
     TREX_UNROLL for (int k = 0; k < 6; k++) pA[k] = ld(sb, eo + bl + (O_PA + k * 32));
     vf IA[21];
@@ -552,11 +571,12 @@ TREX_FN void inward_packed(const Uniform& P, const float* mdl, const int* mdli, 
 // environments of that class (0: contact-free, 1: 1-2 contacts, 2: 3-4, 3: 5-8).
 // PACKED (front kernel with 4-warp CTAs): the inward pass of the CTA's four environments is done by warp 0
 // (inward_packed) between two CTA barriers; cta_slabs = slab of warp 0, valid_mask = which warps hold an environment.
-template <bool PACKED = false>
+// ENVP: envp = this environment's parameter row (mass scales and friction; the caller passes the row's motor settings)
+template <bool PACKED = false, bool ENVP = false>
 TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const float* tasks, const float* cand_p,
                      const int* cand_lane, WarpShared& S, EnvRegs& R, float kp, float kd, float max_imp,
                      StepStats& stats, float* work, WarpShared* cta_slabs = nullptr, int warp_in_cta = 0, int valid_mask = 0,
-                     float* workh = nullptr) {
+                     float* workh = nullptr, const float* envp = nullptr) {
   const vi lane = lane_id();
   const vb is_joint = lane < NJ;
   const vb is_base = lane == 25;
@@ -585,10 +605,11 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
 
   TREX_TICK(0)
   // ---- 3. bias forces: p = v x* (I v) - gravity wrench + angular damping ------------------
-  const vf mass = MDL(F_MASS);
+  const vf msc = ENVP ? envp_mass_scale(envp, lane) : vf(1.0f);  // this lane's body's mass scale
+  const vf mass = ENVP ? MDL(F_MASS) * msc : MDL(F_MASS);
   vf mc[3], I3[6];
-  TREX_UNROLL for (int k = 0; k < 3; k++) mc[k] = MDL(F_MC + k);
-  TREX_UNROLL for (int k = 0; k < 6; k++) I3[k] = MDL(F_I + k);
+  TREX_UNROLL for (int k = 0; k < 3; k++) mc[k] = ENVP ? MDL(F_MC + k) * msc : MDL(F_MC + k);
+  TREX_UNROLL for (int k = 0; k < 6; k++) I3[k] = ENVP ? MDL(F_I + k) * msc : MDL(F_I + k);
   vf pA[6];
   {
     const vf wx = v[0], wy = v[1], wz = v[2], lx = v[3], ly = v[4], lz = v[5];
@@ -613,7 +634,7 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
     pA[3] -= mass * gx; pA[4] -= mass * gy; pA[5] -= mass * gz;
     // angular damping of every URDF link of the body: (sum R I R^T) w (k + k|w|)
     vf dr[6];
-    TREX_UNROLL for (int k = 0; k < 6; k++) dr[k] = MDL(F_DROT + k);
+    TREX_UNROLL for (int k = 0; k < 6; k++) dr[k] = ENVP ? MDL(F_DROT + k) * msc : MDL(F_DROT + k);
     const vf wn = vsqrt(wx * wx + wy * wy + wz * wz);
     const vf ka = P.k_ang + P.k_ang * wn;
     pA[0] += (dr[0] * wx + dr[1] * wy + dr[2] * wz) * ka;
@@ -625,12 +646,13 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
     const vi dl = MDLI(IF_DAMP_LANE);
     vf bv[6];
     TREX_UNROLL for (int k = 0; k < 6; k++) bv[k] = shflv(v[k], dl);
+    const vf tsc = ENVP ? shflv(msc, dl) : vf(1.0f);  // mass scale of the body whose links this lane evaluates
     vf acc[6];
     TREX_UNROLL for (int k = 0; k < 6; k++) acc[k] = 0.0f;
     // (latency bound: four table loads feed ~25 dependent operations per round -- several rounds in flight)
     _Pragma("unroll 5") for (int rd = 0; rd < P.n_rounds; rd++) {
       const float* t = tasks + rd * 4 * 32;
-      const vf rx = ldg_ro(t, lane), ry = ldg_ro(t, lane + 32), rz = ldg_ro(t, lane + 64), m = ldg_ro(t, lane + 96);
+      const vf rx = ldg_ro(t, lane), ry = ldg_ro(t, lane + 32), rz = ldg_ro(t, lane + 64), m = ENVP ? ldg_ro(t, lane + 96) * tsc : ldg_ro(t, lane + 96);
       const vf cx = bv[3] + (bv[1] * rz - bv[2] * ry);
       const vf cy = bv[4] + (bv[2] * rx - bv[0] * rz);
       const vf cz = bv[5] + (bv[0] * ry - bv[1] * rx);
@@ -679,7 +701,7 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
     TREX_UNROLL for (int k = 0; k < 6; k++) st(S.x.pA[k], lane, pA[k]);
     st(S.x.cc[0], lane, c0); st(S.x.cc[1], lane, c1); st(S.x.cc[2], lane, c3); st(S.x.cc[3], lane, c4); st(S.x.cc[4], lane, tau_j);
     cta_sync();
-    if (warp_in_cta == 0) inward_packed(P, mdl, mdli, cta_slabs, valid_mask);
+    if (warp_in_cta == 0) inward_packed<ENVP>(P, mdl, mdli, cta_slabs, valid_mask, ENVP ? envp - TREX_ENVP_DIM * warp_in_cta : nullptr);
     cta_sync();
     TREX_UNROLL for (int k = 0; k < 6; k++) U[k] = sel(is_joint, ld(S.k.U[k], lane), 0.0f);
     invD = sel(is_joint, ld(S.k.invD, lane), 0.0f);
@@ -1149,6 +1171,7 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
         }
         st_if(cw, sb + 9, c_lam[0], own);
         st_if(cw, sb + 10, vi2f(ldi(S.ccand, ls)), own);
+        if (ENVP) st_if(cw, sb + 11, vbroadcast(ldu(envp, EP_MU)), own);  // the environment's friction coefficient
         st_if(cw, vi(o_nc), vbroadcast((float)n_act), lane == 0);
       }
       TREX_ROLLED for (int r = 0; r < 3 * n_act; r++) st(cw, lane + (r * 32 + o_bt), ld(S.c.dV[r], lane));
@@ -1326,7 +1349,7 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
       const vi sl = ldb(S.c.slot[c], lane);
       const vf jA = warp_sum(ld(S.c.Jc[3 * c + 1], sl) * dv);
       const vf jB = warp_sum(ld(S.c.Jc[3 * c + 2], sl) * dv);
-      const vf lim = P.mu * c_lam[0];
+      const vf lim = (ENVP ? ldu(envp, EP_MU) : P.mu) * c_lam[0];
       vf dB = c_rhs[2] - jB * c_jdi[2];
       const vf sumB = c_lam[2] + dB;
       vf dA = c_rhs[1] - jA * c_jdi[1];
@@ -1361,7 +1384,7 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
   {  // active-set signature of this substep's solve (see StepStats)
     const uint32_t Lm = vballot(is_joint && ((lam_lo > 0.0f) || (lam_hi > 0.0f)));
     const uint32_t Mm = vballot(is_joint && (vabs(lam_m) >= max_imp));
-    const vf lim = P.mu * c_lam[0];
+    const vf lim = (ENVP ? ldu(envp, EP_MU) : P.mu) * c_lam[0];
     const vb hasc = lane < n_act;
     const uint32_t Nm = vballot(hasc && (c_lam[0] > 0.0f));
     const uint32_t Fm = vballot(hasc && (c_lam[0] > 0.0f) && ((c_lam[1] * c_lam[1] + c_lam[2] * c_lam[2]) >= TREX_CONE_EDGE * (lim * lim)));
@@ -1460,6 +1483,28 @@ TREX_FN void reset_pose(const Uniform& P, const float* mdl, vi lane, WarpShared&
   warp_sync();
 }
 
+// Randomizer of the per-environment parameters, at every reset of an environment: element L of its row is
+//   lo_L + u_L (hi_L - lo_L)   (one fused multiply-add: lo == hi gives lo exactly)
+// with u from Philox4x32-10 keyed by (seed, TREX_ENVP_PHILOX_KEY), counter (global env id, episode, block L >> 2), word L & 3
+// -- the reset sampler's counters with a different key, so rows depend on neither the number of GPUs nor the reset-pose stream.
+// Element 30 (the motor impulse bound) is then derived from the drawn torque in double, as the model's own bound is.
+// ranges: lo [32] then hi [32]; dt: the physics substep in double.
+TREX_FN void draw_env_params(const Uniform& P, vi lane, const float* ranges, float* envp, long long env_id, float episode, double dt) {
+  const unsigned long long gid = (unsigned long long)(P.env_offset + env_id);
+  const vi c0 = vi((int)(unsigned)(gid & 0xffffffffull)), c1 = vi((int)(unsigned)(gid >> 32)), c2 = vi((int)episode);
+  vf u[4];
+  philox4_uniform(c0, c1, c2, lane >> 2, P.seed, TREX_ENVP_PHILOX_KEY, u);
+  const vi wsel = lane & 3;
+  const vf ul = sel(wsel == 0, u[0], sel(wsel == 1, u[1], sel(wsel == 2, u[2], u[3])));
+  const vf lo = ld(ranges, lane), hi = ld(ranges, lane + TREX_ENVP_DIM);
+  vf x = vfma(ul, hi - lo, lo);
+  const float imp = (float)((double)lane_value(x, EP_MAX_TORQUE) * dt);
+  x = sel(lane == EP_MAX_IMPULSE, vbroadcast(imp), x);
+  warp_sync();
+  st(envp, lane, x);
+  warp_sync();
+}
+
 // ------------------------------------------------------------------------------------------
 // solve4: projected Gauss-Seidel for up to FOUR contact-free environments in one warp.
 //
@@ -1504,7 +1549,7 @@ TREX_TOPO_FN bool limit_order_matches_motor_order() {
 #define S4_TM_COLS(KC) (S4_TM_BK(KC) + 84)
 template <int B, bool FWD, int KC, bool TM>
 TREX_FN void s4_motor_block(vf (&w)[4], vf (&lam_m)[4], const vf (&g)[4][NJ], vf (&cu)[3], vi glx, vi dead, vi bt_own, const float* Bs,
-                            tmem_t tm, float max_imp) {
+                            tmem_t tm, vf max_imp) {
   constexpr int n = (4 * B + 4 <= NJ) ? 4 : NJ - 4 * B;
   vf bk[3][4];  // responses of the owned contact's three rows at this block's four joints
   if (KC > 0) TREX_UNROLL for (int k = 0; k < 3; k++) {
@@ -1563,8 +1608,9 @@ TREX_FN void s4_motor_block(vf (&w)[4], vf (&lam_m)[4], const vf (&g)[4][NJ], vf
 // loads do not go through it.
 #define TREX_SOLVE_SCRATCH_TM(KC) (4 * TREX_BT_SIZE(KC) + 4 * (32 + 4 * (KC)) + 128 * TREX_LIMIT_SLOTS(KC))
 // envs[g] = index (relative to work0 / rec0) of the environment served by lane group g, valid when pending bit g is set.
-template <int KC, bool TM = false>
-TREX_FN vi solve4(const Uniform& P, float* scratch, const float* work0, float* rec0, const int envs[4], int pending, float max_imp,
+// max_imp: motor impulse bound (per lane group).  ENVP: each contact's friction coefficient comes from word 11 of its scalars.
+template <int KC, bool TM = false, bool ENVP = false>
+TREX_FN vi solve4(const Uniform& P, float* scratch, const float* work0, float* rec0, const int envs[4], int pending, vf max_imp,
                   tmem_t tm = tmem_t()) {
   static_assert((KC == 0 || KC == 1 || KC == 2 || KC == 4 || KC == 8) && KC <= TREX_KC, "one contact per lane of a group");
   static_assert(!TM || KC == TREX_KC, "the tensor-memory instance serves all contact classes of solve4");
@@ -1613,6 +1659,7 @@ TREX_FN vi solve4(const Uniform& P, float* scratch, const float* work0, float* r
   vi ccand = 0;
   vb cown = gact && !gact;
   int kmax = 0;
+  vf mu_own = 0.0f;  // ENVP: friction coefficient of the owned contact's environment
   if (KC > 0) {
     const vi nc = seli(gact, vf2i(ld(work0, woff + W_NC)), 0);
     kmax = lane_value_i(warp_maxi(nc), 0);
@@ -1623,6 +1670,7 @@ TREX_FN vi solve4(const Uniform& P, float* scratch, const float* work0, float* r
       cjdi[k] = ld_if(work0, sb + (3 + k), cown, 0.0f);
       cdd[k] = ld_if(work0, sb + (6 + k), cown, 0.0f);
     }
+    if (ENVP) mu_own = ld_if(work0, sb + 11, cown, 0.0f);
     cl[0] = ld_if(work0, sb + 9, cown, 0.0f);  // warm start
     ccand = seli(cown, vf2i(ld_if(work0, sb + 10, cown, 0.0f)), 0);
     // Bt: rows 3c+k of the record (32 floats each) -> rows of 33; one float4 per lane and step, 8 per row
@@ -1732,7 +1780,7 @@ TREX_FN vi solve4(const Uniform& P, float* scratch, const float* work0, float* r
     }                                                                                                  \
   }
 #define MB_(b, fwd) s4_motor_block<b, fwd, KC, TM>(w, lam_m, g, cu, glx, dead, bt_own, Bs, tm, max_imp);
-  vf mu_l = P.mu;
+  vf mu_l = ENVP ? mu_own : vf(P.mu);
   TREX_ROLLED for (int it = 0; it < P.iters; it++) {
     // every 4th sweep (TREX_REBUILD_MASK) rebuild w (and u) exactly from the impulses (bounds the FP32 drift of the incremental updates):
     // w_k = rhs_m,k - sigma_k lam_l,k + sum_j g[k][j] Lambda_j - jdi_k sum_r B[r][k] lambda_r
@@ -1968,7 +2016,7 @@ TREX_FN vi solve4(const Uniform& P, float* scratch, const float* work0, float* r
     }
     vi NF = 0;
     if (KC > 0) {
-      const vf lim = P.mu * cl[0];
+      const vf lim = (ENVP ? mu_own : vf(P.mu)) * cl[0];
       const vb pos = cown && (cl[0] > 0.0f);
       NF = seli(pos, vi(1) << gl, vi(0)) |
            seli(pos && ((cl[1] * cl[1] + cl[2] * cl[2]) >= TREX_CONE_EDGE * (lim * lim)), vi(65536) << gl, vi(0));
@@ -2025,7 +2073,7 @@ template <bool TM>
 TREX_FN void s2_ready_a(vf (&a)[4]) { if (TM) tmem_wait4(a); }
 
 template <int B, bool FWD>
-TREX_FN void s2_motor_block(vf (&w)[2], vf (&lam_m)[2], const vf (&g)[2][NJ], vf (&cu)[3], vi glx, vi dead, vi bp_own, const float* Sc, float max_imp) {
+TREX_FN void s2_motor_block(vf (&w)[2], vf (&lam_m)[2], const vf (&g)[2][NJ], vf (&cu)[3], vi glx, vi dead, vi bp_own, const float* Sc, vf max_imp) {
   constexpr int n = (2 * B + 2 <= NJ) ? 2 : NJ - 2 * B;
   vf bk[3][2];  // responses of the owned contact's three rows at this block's joints
   TREX_UNROLL for (int k = 0; k < 3; k++) ld2(Sc, bp_own + (k * TREX_S2_BS + 2 * B), bk[k]);
@@ -2049,9 +2097,9 @@ TREX_FN void s2_motor_block(vf (&w)[2], vf (&lam_m)[2], const vf (&g)[2][NJ], vf
 }
 
 // envs[g] = index (relative to work0 / workh0 / rec0) of the environment served by lane group g, valid when pending bit g is set.
-template <bool TM>
+template <bool TM, bool ENVP = false>
 TREX_FN vi solve2(const Uniform& P, float* scratch, tmem_t tm, const float* work0, const float* workh0, float* rec0, const int envs[2],
-                  int pending, float max_imp) {
+                  int pending, vf max_imp) {
   constexpr int NR = TREX_S2_NR, BS = TREX_S2_BS, LS = TREX_S2_LS, AOFF = 0, BOFF = TM ? 0 : NR * NR;
   constexpr int ENV = TM ? TREX_S2_ENV_TM : TREX_S2_ENV;
   const vi lane = lane_id();
@@ -2106,6 +2154,7 @@ TREX_FN vi solve2(const Uniform& P, float* scratch, tmem_t tm, const float* work
     }
     cl[0] = ld_if(workh0, sb + 9, cown, 0.0f);  // warm start
   }
+  const vf mu_own = ENVP ? ld_if(workh0, hoff + gl * 16 + (H_CS + 11), cown, 0.0f) : vf(P.mu);  // ENVP: the environment's friction
   const vi ccand = seli(cown, vf2i(ld_if(workh0, hoff + gl * 16 + (H_CS + 10), cown, 0.0f)), 0);
   {
     const vi nr = nc * 3;
@@ -2194,7 +2243,7 @@ TREX_FN vi solve2(const Uniform& P, float* scratch, tmem_t tm, const float* work
     }                                                                                                  \
   }
 #define MB_(b, fwd) s2_motor_block<b, fwd>(w, lam_m, g, cu, glx, dead, bp_own, Sc, max_imp);
-  vf mu_l = P.mu;
+  vf mu_l = ENVP ? mu_own : vf(P.mu);
   TREX_ROLLED for (int it = 0; it < P.iters; it++) {
     // every 16th sweep (TREX_S2_REBUILD_MASK) rebuild w and u exactly from the impulses (also the warm-started initial state):
     // w_k = rhs_m,k - sigma_k lam_l,k + sum_j g[k][j] Lambda_j - jdi_k sum_r B[r][k] lambda_r
@@ -2423,7 +2472,7 @@ TREX_FN vi solve2(const Uniform& P, float* scratch, tmem_t tm, const float* work
     }
     vi NF = 0;
     {
-      const vf lim = P.mu * cl[0];
+      const vf lim = (ENVP ? mu_own : vf(P.mu)) * cl[0];
       const vb pos = cown && (cl[0] > 0.0f);
       NF = seli(pos, vi(1) << gl, vi(0)) |
            seli(pos && ((cl[1] * cl[1] + cl[2] * cl[2]) >= TREX_CONE_EDGE * (lim * lim)), vi(65536) << gl, vi(0));
@@ -2491,10 +2540,12 @@ static_assert(ST_SIG == ST_ACC_ITERS + 3, "front_phase stores the four accumulat
 // articulated inertias, accelerations, velocity update, M^-1, row setup, contact detection.  With more than TREX_KC
 // contacts the substep is finished here (one-environment solver + integration); otherwise the solver inputs go to
 // `work` and the function returns 1 + class (solve_phase finishes the substep).   action: [25] name-sorted (trex_robot.py:311-314)
-template <bool PACKED = false>
+// ENVP: envp = the environment's parameter row (mass scales, friction, motor gains and impulse bound)
+template <bool PACKED = false, bool ENVP = false>
 TREX_FN int front_phase(const Uniform& P, const float* mdl, const int* mdli, const float* tasks, const float* cand_p,
                          const int* cand_lane, WarpShared& S, float* rec, float* work, const float* action, bool first_round,
-                         WarpShared* cta_slabs = nullptr, int warp_in_cta = 0, int valid_mask = 0, float* workh = nullptr) {
+                         WarpShared* cta_slabs = nullptr, int warp_in_cta = 0, int valid_mask = 0, float* workh = nullptr,
+                         const float* envp = nullptr) {
   const vi lane = lane_id();
   const vb is_joint = lane < NJ;
   const vi slot = seli(is_joint, MDLI(IF_OBS_SLOT), 0);
@@ -2509,8 +2560,10 @@ TREX_FN int front_phase(const Uniform& P, const float* mdl, const int* mdli, con
 #ifdef TREX_PHASES
   for (int i = 0; i < 8; i++) st.phase[i] = 0.0f;
 #endif
-  const int deferred = substep<PACKED>(P, mdl, mdli, tasks, cand_p, cand_lane, S, R, P.kp, P.kd, P.max_impulse, st, work, cta_slabs,
-                                       warp_in_cta, valid_mask, workh);
+  const float kp = ENVP ? ldu(envp, EP_KP) : P.kp, kd = ENVP ? ldu(envp, EP_KD) : P.kd;
+  const float max_imp = ENVP ? ldu(envp, EP_MAX_IMPULSE) : P.max_impulse;
+  const int deferred = substep<PACKED, ENVP>(P, mdl, mdli, tasks, cand_p, cand_lane, S, R, kp, kd, max_imp, st, work, cta_slabs,
+                                             warp_in_cta, valid_mask, workh, envp);
   store_env(rec, lane, S, R);  // deferred: positions unchanged, velocities after the unconstrained update
   const float it0 = first_round ? 0.0f : ldu(rec, ST_ACC_ITERS), ov0 = first_round ? 0.0f : ldu(rec, ST_ACC_OVERFLOW);
   vf acc = 0.0f;
@@ -2531,11 +2584,19 @@ TREX_FN int front_phase(const Uniform& P, const float* mdl, const int* mdli, con
 }
 
 // solve_phase: the deferred solves of up to four environments (any four: the groups are independent)
-template <int KC, bool TM = false>
+// ENVP: envp0 = parameter rows indexed like rec0 (the motor impulse bound of each group's environment)
+template <int KC, bool TM = false, bool ENVP = false>
 TREX_FN void solve_phase(const Uniform& P, float* scratch, const float* work0, float* rec0, const int envs[4], int pending,
-                         tmem_t tm = tmem_t()) {
+                         tmem_t tm = tmem_t(), const float* envp0 = nullptr) {
   const vi lane = lane_id();
-  const vi itd = solve4<KC, TM>(P, scratch, work0, rec0, envs, pending, P.max_impulse, tm);
+  vf max_imp = P.max_impulse;
+  if (ENVP) {
+    const vi g = lane >> 3;
+    const vi ge = seli(g == 0, vi(envs[0]), seli(g == 1, vi(envs[1]), seli(g == 2, vi(envs[2]), vi(envs[3]))));
+    const vb gp = ((vi(pending) >> g) & 1) != 0;
+    max_imp = ld_if(envp0, seli(gp, ge, 0) * TREX_ENVP_DIM + EP_MAX_IMPULSE, gp, 0.0f);
+  }
+  const vi itd = solve4<KC, TM, ENVP>(P, scratch, work0, rec0, envs, pending, max_imp, tm);
   // iterations executed per environment -> its accumulator (lane 8e holds group e's count)
   const vi grp = lane >> 3;
   const vb wr = ((lane & 7) == 0) && ((((vi(pending)) >> grp) & 1) != 0);
@@ -2545,11 +2606,18 @@ TREX_FN void solve_phase(const Uniform& P, float* scratch, const float* work0, f
 }
 
 // heavy_phase: the deferred solves of up to two environments with more than TREX_KC contacts (any two)
-template <bool TM = false>
+template <bool TM = false, bool ENVP = false>
 TREX_FN void heavy_phase(const Uniform& P, float* scratch, tmem_t tm, const float* work0, const float* workh0, float* rec0, const int envs[2],
-                         int pending) {
+                         int pending, const float* envp0 = nullptr) {
   const vi lane = lane_id();
-  const vi itd = solve2<TM>(P, scratch, tm, work0, workh0, rec0, envs, pending, P.max_impulse);
+  vf max_imp = P.max_impulse;
+  if (ENVP) {
+    const vi g = lane >> 4;
+    const vi ge = seli(g == 0, vi(envs[0]), vi(envs[1]));
+    const vb gp = ((vi(pending) >> g) & 1) != 0;
+    max_imp = ld_if(envp0, seli(gp, ge, 0) * TREX_ENVP_DIM + EP_MAX_IMPULSE, gp, 0.0f);
+  }
+  const vi itd = solve2<TM, ENVP>(P, scratch, tm, work0, workh0, rec0, envs, pending, max_imp);
   const vi grp = lane >> 4;
   const vb wr = ((lane & 15) == 0) && ((((vi(pending)) >> grp) & 1) != 0);
   const vi genv = seli(grp == 0, vi(envs[0]), vi(envs[1]));
@@ -2562,9 +2630,13 @@ TREX_FN void heavy_phase(const Uniform& P, float* scratch, tmem_t tm, const floa
 // zero-force motors, ONE physics step), observations (trex_robot.py:359-365), diagnostics.
 // force_reset: only the reset (trex_reset).
 //   obs : [75] q | qd | motor torque   aux : [TREX_AUX_STRIDE] head xyz, lifting/station/energy, PGS iterations, contacts
+// ENVP: envp = the environment's parameter row (mass scales and friction apply to the reset step; its motor gains stay zero).
+// ranges != nullptr: the randomizer is on -- every reset first draws a new row (draw_env_params).
+template <bool ENVP = false>
 TREX_FN void tail_phase(const Uniform& P, const float* mdl, const int* mdli, const float* tasks, const float* cand_p,
                         const int* cand_lane, WarpShared& S, float* rec, float* obs, float* reward, uint8_t* done,
-                        float* aux, bool force_reset, long long env_id) {
+                        float* aux, bool force_reset, long long env_id, float* envp = nullptr, const float* ranges = nullptr,
+                        double dt = 0.0) {
   const vi lane = lane_id();
   const vb is_joint = lane < NJ;
   const vi slot = seli(is_joint, MDLI(IF_OBS_SLOT), 0);
@@ -2600,12 +2672,13 @@ TREX_FN void tail_phase(const Uniform& P, const float* mdl, const int* mdli, con
   if (force_reset || is_done) {
     const float episode = ldu(rec, ST_EPISODE);
     reset_pose(P, mdl, lane, S, R, env_id, episode);
+    if (ENVP && ranges != nullptr) draw_env_params(P, lane, ranges, envp, env_id, episode, dt);
     StepStats rs;
     rs.iters = 0; rs.contacts = 0; rs.overflow = 0; rs.sig = 0u;
 #ifdef TREX_PHASES
     for (int i = 0; i < 8; i++) rs.phase[i] = 0.0f;
 #endif
-    substep(P, mdl, mdli, tasks, cand_p, cand_lane, S, R, 0.0f, 0.0f, 0.0f, rs, nullptr);
+    substep<false, ENVP>(P, mdl, mdli, tasks, cand_p, cand_lane, S, R, 0.0f, 0.0f, 0.0f, rs, nullptr, nullptr, 0, 0, nullptr, envp);
     store_env(rec, lane, S, R);
     vf meta = 0.0f;
     meta = sel(lane == 1, vbroadcast(episode + 1.0f), meta);

@@ -303,4 +303,36 @@ static inline void fill_uniform(const ModelTables& T, const EnvConfig& C, U& P) 
   }
 }
 
+// ---- per-environment parameter rows (layout: trex_core.h, TREX_ENVP_DIM) ---------------------------------------------
+enum { ENVP_DIM = 32, ENVP_MASS_BASE = 25, ENVP_MU = 26, ENVP_KP = 27, ENVP_KD = 28, ENVP_MAX_TORQUE = 29, ENVP_MAX_IMPULSE = 30 };
+
+// physics substep in double: the motor impulse bound is torque * this, rounded once to float
+static inline double substep_dt(const ModelTables& T, int num_substeps) {
+  return T.params[P_TIME_STEP] / (num_substeps < 1 ? 1 : num_substeps);
+}
+
+// the row that reproduces the model's own constants: unit mass scales, and friction, gains and bounds as fill_uniform rounds them
+static inline void default_env_params(const ModelTables& T, int num_substeps, float row[ENVP_DIM]) {
+  const double* p = T.params;
+  for (int k = 0; k < ENVP_DIM; k++) row[k] = k <= ENVP_MASS_BASE ? 1.0f : 0.0f;
+  row[ENVP_MU] = (float)p[P_FRICTION];
+  row[ENVP_KP] = (float)p[P_KP];
+  row[ENVP_KD] = (float)p[P_KD];
+  row[ENVP_MAX_TORQUE] = (float)p[P_MAX_TORQUE];
+  row[ENVP_MAX_IMPULSE] = (float)(p[P_MAX_TORQUE] * substep_dt(T, num_substeps));
+}
+
+// randomizer ranges: lo <= hi, all finite, mass scales > 0, friction / gains / torque >= 0, elements 30-31 zero.
+// Returns nullptr when valid, else what is wrong.
+static inline const char* check_env_param_ranges(const float lo[ENVP_DIM], const float hi[ENVP_DIM]) {
+  for (int k = 0; k < ENVP_DIM; k++) {
+    if (!(lo[k] - lo[k] == 0.0f) || !(hi[k] - hi[k] == 0.0f)) return "ranges must be finite";
+    if (!(lo[k] <= hi[k])) return "every low bound must be <= its high bound";
+    if (k <= ENVP_MASS_BASE && !(lo[k] > 0.0f)) return "mass scales must be > 0";
+    if (k > ENVP_MASS_BASE && k < ENVP_MAX_IMPULSE && !(lo[k] >= 0.0f)) return "friction, kp, kd and max torque must be >= 0";
+    if (k >= ENVP_MAX_IMPULSE && (lo[k] != 0.0f || hi[k] != 0.0f)) return "elements 30 and 31 of the ranges must be zero";
+  }
+  return nullptr;
+}
+
 }  // namespace trex_host

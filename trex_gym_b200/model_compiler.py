@@ -872,6 +872,31 @@ def with_params(model: CompiledModel, **overrides) -> CompiledModel:
     return CompiledModel(sections, meta)
 
 
+def with_body_mass_scale(model: CompiledModel, scales) -> CompiledModel:
+    """Copy of ``model`` with the mass of every merged body scaled: uniform density scaling, what pybullet's
+    ``changeDynamics(mass=s * m, localInertiaDiagonal=s * I)`` does to each URDF link of the body.  The COM stays; the
+    mass, first moment, rotational inertia, angular-damping tensor and link-damping task masses of the body, and the
+    mass and principal inertia of each of its links, are multiplied by the body's scale.
+
+    ``scales``: 26 factors in the order of a per-environment parameter row (``TrexBatchSim.set_env_params``):
+    ``scales[L]`` for the body of joint ``L`` (body ``L + 1``), ``scales[25]`` for the base."""
+    s = np.asarray(scales, np.float64).reshape(-1)
+    nb = int(model.sections["mb_n_bodies"][0])
+    if s.shape != (nb,) or not np.all(np.isfinite(s)) or np.any(s <= 0):
+        raise ValueError("scales must be %d finite factors > 0" % nb)
+    by_body = np.concatenate([s[nb - 1:], s[:nb - 1]])  # body index order: base first
+    S = OrderedDict(model.sections)
+    S["mb_mass"] = model.sections["mb_mass"] * by_body
+    for name, width in (("mb_mc", 3), ("mb_I", 6), ("mb_damp_rot", 6)):
+        S[name] = (model.sections[name].reshape(nb, width) * by_body[:, None]).reshape(-1)
+    task_body = model.sections["mb_task_body"]
+    link_scale = by_body[task_body]  # one task per URDF link, in link order
+    S["mb_task_m"] = model.sections["mb_task_m"] * link_scale
+    S["full_mass"] = model.sections["full_mass"] * link_scale
+    S["full_inertia"] = (model.sections["full_inertia"].reshape(-1, 3) * link_scale[:, None]).reshape(-1)
+    return CompiledModel(S, dict(model.meta))
+
+
 def emit_topology_header(model: CompiledModel) -> str:
     """C header with the merged tree as compile-time constants.
 

@@ -27,7 +27,8 @@ class TrexBatchSim:
                  drift_weight: float = 0.002, max_episode_steps: int = 0, contacts: bool = True,
                  seed: int = 0, warps_per_block: int | None = None, reset_mode: int = 0, env_offset: int = 0,
                  deferred_solve: bool = True, defer_contacts: bool = True, heavy_solver: bool = True,
-                 heavy_share_div: int = 0, pipelines: int = 0, heavy_memory: int = 0, chunk_envs: int = 0, contact_memory: int = 0):
+                 heavy_share_div: int = 0, pipelines: int = 0, heavy_memory: int = 0, chunk_envs: int = 0, contact_memory: int = 0,
+                 env_params: bool = False):
         if not torch.cuda.is_available():
             raise RuntimeError("trex_gym_b200 needs a CUDA device (no CPU fallback)")
         dev = torch.device(device if not isinstance(device, int) else "cuda:%d" % device)
@@ -58,6 +59,8 @@ class TrexBatchSim:
         cfg.pipelines = int(pipelines)  # 0 = default; independent groups of environments on separate streams
         cfg.contact_memory = int(contact_memory)  # _native.CONTACT_TENSOR (default) / CONTACT_SHARED: where solve4 keeps its contact stash
         cfg.chunk_envs = int(chunk_envs)  # 0 = default; L2-resident work records (include/trex_b200.h), -1 = off
+        cfg.env_params = int(bool(env_params))  # per-environment dynamics parameters (set_env_params)
+        self.env_params = bool(env_params)
         blob = self.model.blob()
         h = ctypes.c_void_p()
         idx = dev.index if dev.index is not None else torch.cuda.current_device()
@@ -205,6 +208,101 @@ class TrexBatchSim:
         obs = np.empty((self.num_envs, _native.OBS_DIM), np.float32)
         _native.check(self._L.trex_reset_host(self._h, ctypes.c_void_p(obs.ctypes.data)), "trex_reset_host")
         return obs
+
+    # -- per-environment dynamics parameters (env_params=True) ------------------------------------------------
+    # A row has 32 floats (include/trex_b200.h): [0:25] mass scale of the body of joint k (pybullet link order), [25] of the
+    # base, [26] friction, [27] kp, [28] kd, [29] max torque (N m), [30] impulse bound (derived), [31] reserved.
+    _ROW_FIELDS = {"friction": 26, "kp": 27, "kd": 28, "max_torque": 29}
+
+    def _body_index(self, name) -> int:
+        """Row element of a body named by its joint (``meta["body_joint_names"]``) or ``"base"``."""
+        if name == "base":
+            return 25
+        names = self.model.meta["body_joint_names"]
+        if name not in names[1:]:
+            raise ValueError("unknown body %r: use 'base' or a name of meta['body_joint_names']" % (name,))
+        return names.index(name) - 1
+
+    def default_env_params(self) -> torch.Tensor:
+        """The row that reproduces the model's own constants ([32] on the CPU): unit mass scales, the model's friction,
+        motor gains and torque."""
+        p = self.model.meta["params"]
+        row = np.zeros(_native.ENV_PARAM_DIM, np.float32)
+        row[:26] = 1.0
+        row[26], row[27], row[28], row[29] = p["friction"], p["motor_kp"], p["motor_kd"], p["motor_max_torque"]
+        row[30] = np.float32(p["motor_max_torque"] * (p["time_step"] / self.num_substeps))
+        return torch.from_numpy(row)
+
+    def _row(self, spec, base) -> np.ndarray:
+        """A [32] row from an array, or from names (``mass_scale``: a scalar or {body: scale}; ``friction``, ``kp``,
+        ``kd``, ``max_torque``) applied on top of ``base``."""
+        if not isinstance(spec, dict):
+            row = np.asarray(spec.cpu() if isinstance(spec, torch.Tensor) else spec, np.float32).reshape(-1)
+            if row.shape != (_native.ENV_PARAM_DIM,):
+                raise ValueError("a parameter row has %d elements" % _native.ENV_PARAM_DIM)
+            return row.copy()
+        row = np.array(base, np.float32)
+        for k, v in spec.items():
+            if k == "mass_scale":
+                if isinstance(v, dict):
+                    for body, sc in v.items():
+                        row[self._body_index(body)] = sc
+                else:
+                    row[:26] = v
+            elif k in self._ROW_FIELDS:
+                row[self._ROW_FIELDS[k]] = v
+            else:
+                raise ValueError("unknown parameter %r (mass_scale, friction, kp, kd, max_torque)" % (k,))
+        return row
+
+    def _need_env_params(self):
+        if not self.env_params:
+            raise ValueError("the simulator was created with env_params=False")
+
+    def get_env_params(self) -> torch.Tensor:
+        """[N,32] copy of every environment's parameter row (element 30 as the library derived it)."""
+        self._need_env_params()
+        t = torch.empty(self.num_envs, _native.ENV_PARAM_DIM, device=self.device, dtype=torch.float32)
+        _native.check(self._L.trex_get_env_params(self._h, ctypes.c_void_p(t.data_ptr()), self._stream()), "trex_get_env_params")
+        return t
+
+    def set_env_params(self, t, mask: torch.Tensor | None = None) -> None:
+        """Set the rows of all (or the masked) environments: ``t`` is an [N,32] tensor, one [32] row for every
+        environment, or a dict of names (see ``_row``) applied to the default row.  Element 30 is derived by the library."""
+        self._need_env_params()
+        if isinstance(t, torch.Tensor) and t.dim() == 2:
+            rows = t.to(device=self.device, dtype=torch.float32).contiguous()
+        else:
+            rows = torch.from_numpy(self._row(t, self.default_env_params().numpy())).to(self.device).repeat(self.num_envs, 1)
+        self._check_tensor(rows, (self.num_envs, _native.ENV_PARAM_DIM), torch.float32, "env params")
+        if not bool(torch.isfinite(rows).all()):
+            raise ValueError("env params must be finite")
+        if bool((rows[:, :26] <= 0).any()) or bool((rows[:, 26:30] < 0).any()):
+            raise ValueError("mass scales must be > 0; friction, kp, kd and max_torque >= 0")
+        mp = None
+        if mask is not None:
+            mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
+            if mask.shape != (self.num_envs,):
+                raise ValueError("mask must have shape (num_envs,)")
+            mp = ctypes.c_void_p(mask.data_ptr())
+        _native.check(self._L.trex_set_env_params(self._h, ctypes.c_void_p(rows.data_ptr()), mp, self._stream()),
+                      "trex_set_env_params")
+        self._env_param_src = (rows, mask)  # kept alive until the stream has consumed them
+
+    def set_env_param_ranges(self, low=None, high=None) -> None:
+        """Randomizer: from now on every reset of an environment (``reset``, masked too, and the auto-reset) draws its row
+        uniformly in [low, high] (Philox keyed by the seed, global environment id and episode).  ``low`` / ``high``: [32]
+        rows, or dicts of names (see ``_row``) applied to the default row; elements 30-31 are ignored.  ``None, None``
+        turns the randomizer off."""
+        self._need_env_params()
+        if low is None and high is None:
+            _native.check(self._L.trex_set_env_param_ranges(self._h, None, None), "trex_set_env_param_ranges")
+            return
+        base = self.default_env_params().numpy()
+        lo, hi = self._row(low, base), self._row(high, base)
+        lo[30:] = 0.0
+        hi[30:] = 0.0
+        _native.check(self._L.trex_set_env_param_ranges(self._h, lo.ctypes.data, hi.ctypes.data), "trex_set_env_param_ranges")
 
     # -- state / diagnostics -----------------------------------------------------------------------
     def get_state(self) -> torch.Tensor:
