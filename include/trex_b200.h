@@ -114,7 +114,11 @@ typedef struct trex_config {
   int32_t env_params;        /* 0 (default): every environment simulates the model's own constants.  1: the handle owns a
                                 per-environment parameter record (trex_set_env_params below) and runs the kernel instances that
                                 read it; rows start as the model's constants, which reproduce the env_params = 0 results bit for bit */
-  int32_t reserved[6];       /* must be zero */
+  int32_t external_forces;   /* 0 (default): gravity is the only external load.  1: the handle owns a per-environment record of
+                                external wrenches on the bodies (trex_set_external_forces below) and an optional push schedule, and
+                                runs the dynamics-kernel instances that read them; the record starts at zero, which reproduces the
+                                external_forces = 0 results bit for bit */
+  int32_t reserved[5];       /* must be zero */
 } trex_config;
 
 typedef struct trex_stats {
@@ -189,6 +193,41 @@ int trex_get_env_params(trex_handle* h, float* params_dev, void* stream);
  * torque >= 0, elements 30 and 31 zero.  NULL / NULL turns the randomizer off.  Synchronises the device (resets already
  * enqueued use the previous ranges); a CUDA graph keeps the setting it was captured with. */
 int trex_set_env_param_ranges(trex_handle* h, const float* lo32_host, const float* hi32_host);
+
+/* External forces and torques on the bodies (handles created with trex_config.external_forces = 1; TREX_ERR_INVALID
+ * otherwise): what pybullet's applyExternalForce(robot, link, F, linkWorldCOM, WORLD_FRAME) and
+ * applyExternalTorque(robot, link, T, WORLD_FRAME) do, summed over the links of a merged body.
+ * The user layout is float32 [N][TREX_EXT_BODIES][6]: body k < 25 is the body moved by joint k (pybullet link order, fixed
+ * links folded in), body 25 the base -- the order of an env-param row.  A wrench is [fx fy fz tx ty tz] in the world
+ * frame (N, N m): the force acts at the body's centre of mass (the composite COM of the merged body; a mass scale leaves it
+ * unchanged), the torque is a free vector.
+ * PERSISTENCE DIFFERS FROM PYBULLET: pybullet clears external forces after every stepSimulation; here the record stays until
+ * it is set again.  It acts in every physics substep of every trex_step / trex_step_host*, never in the physics step of a
+ * reset (trex_reset and the auto-reset), and survives resets.  trex_get_state / trex_set_state do not carry it. */
+#define TREX_EXT_BODIES 26
+/* wrench_dev [N][26][6] (device) -> the record: all environments, or (mask_dev uint8[N] on the device, optional) those with
+ * mask != 0; every wrench of such an environment is replaced.  Stream ordered, capturable. */
+int trex_set_external_forces(trex_handle* h, const float* wrench_dev, const uint8_t* mask_dev, void* stream);
+int trex_get_external_forces(trex_handle* h, float* wrench_dev, void* stream);
+/* Push schedule: a horizontal push on one body, added to the record's force of that body while active.  Stateless: at env
+ * step t of episode e (steps completed in the episode when the step starts) of environment gid = env_offset + env, window
+ * w = t / interval draws u0..u3 from Philox4x32-10 keyed by the seed, counted by (gid, e, w), so pushes depend neither on
+ * the number of GPUs nor on when the schedule was set.  The window holds a push iff u0 < probability; it starts
+ * o = min(floor(u1 (interval - duration + 1)), interval - duration) steps into the window and lasts `duration` steps, and
+ * no push acts before step first_step.  Magnitude force_min + u2 (force_max - force_min) N, direction one of 32 horizontal
+ * unit vectors, index floor(32 u3), angle 2 pi index / 32 from the world x axis. */
+typedef struct trex_push_schedule {
+  int32_t body;              /* 0..25, numbered as above (25 = base) */
+  int32_t interval;          /* >= 1 env steps per window */
+  int32_t duration;          /* 1..interval env steps of a push */
+  int32_t first_step;        /* >= 0: no push before this step of an episode */
+  float probability;         /* [0, 1]: chance that a window holds a push */
+  float force_min, force_max;  /* 0 <= force_min <= force_max, finite (N) */
+  int32_t reserved[9];       /* must be zero */
+} trex_push_schedule;
+/* s_host NULL turns the schedule off.  The schedule is a kernel argument: it applies to the steps enqueued after the call,
+ * and a CUDA graph keeps the schedule it was captured with. */
+int trex_set_push_schedule(trex_handle* h, const trex_push_schedule* s_host);
 
 /* per-env diagnostics of the last step: head xyz (trex_robot.py:330-335), the three penalty terms
  * logged at trex_env.py:193-195 (lifting, station keeping, energy), PGS iterations, contacts. */

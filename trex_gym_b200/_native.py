@@ -18,12 +18,14 @@ OBS_DIM = 75
 STATE_DIM = 160
 AUX_DIM = 8
 ENV_PARAM_DIM = 32  # per-environment parameter row (include/trex_b200.h, trex_set_env_params)
+EXT_BODIES = 26  # bodies of the external-wrench layout [N][26][6] (include/trex_b200.h, trex_set_external_forces)
 
 EXPORTED_SYMBOLS = (
     "trex_create", "trex_destroy", "trex_reset", "trex_step", "trex_step_host", "trex_step_host_async", "trex_host_wait",
     "trex_reset_host",
     "trex_get_state", "trex_set_state", "trex_get_aux", "trex_get_joint_limits",
     "trex_set_env_params", "trex_get_env_params", "trex_set_env_param_ranges",
+    "trex_set_external_forces", "trex_get_external_forces", "trex_set_push_schedule",
     "trex_fill_random_actions", "trex_get_stats", "trex_measure_fp32_peak", "trex_gae", "trex_normalize",
     "trex_policy_param_count", "trex_policy_forward", "trex_kernel_launches", "trex_num_envs",
     "trex_last_error", "trex_version",
@@ -49,7 +51,21 @@ class TrexConfig(ctypes.Structure):
         ("chunk_envs", ctypes.c_int32),
         ("contact_memory", ctypes.c_int32),
         ("env_params", ctypes.c_int32),
-        ("reserved", ctypes.c_int32 * 6),
+        ("external_forces", ctypes.c_int32),
+        ("reserved", ctypes.c_int32 * 5),
+    ]
+
+
+class TrexPushSchedule(ctypes.Structure):
+    _fields_ = [
+        ("body", ctypes.c_int32),
+        ("interval", ctypes.c_int32),
+        ("duration", ctypes.c_int32),
+        ("first_step", ctypes.c_int32),
+        ("probability", ctypes.c_float),
+        ("force_min", ctypes.c_float),
+        ("force_max", ctypes.c_float),
+        ("reserved", ctypes.c_int32 * 9),
     ]
 
 
@@ -130,6 +146,12 @@ def lib():
     L.trex_get_env_params.argtypes = [vp, fp, vp]
     L.trex_set_env_param_ranges.restype = ctypes.c_int
     L.trex_set_env_param_ranges.argtypes = [vp, fp, fp]
+    L.trex_set_external_forces.restype = ctypes.c_int
+    L.trex_set_external_forces.argtypes = [vp, fp, u8p, vp]
+    L.trex_get_external_forces.restype = ctypes.c_int
+    L.trex_get_external_forces.argtypes = [vp, fp, vp]
+    L.trex_set_push_schedule.restype = ctypes.c_int
+    L.trex_set_push_schedule.argtypes = [vp, ctypes.POINTER(TrexPushSchedule)]
     L.trex_get_joint_limits.restype = ctypes.c_int
     L.trex_get_joint_limits.argtypes = [vp, fp, fp]
     L.trex_fill_random_actions.restype = ctypes.c_int

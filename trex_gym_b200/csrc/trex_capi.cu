@@ -39,6 +39,8 @@ static_assert(trex::F_COUNT == 32, "float field table");
 static_assert(TREX_ENV_PARAM_DIM == TREX_ENVP_DIM && TREX_ENVP_DIM == (int)trex_host::ENVP_DIM &&
               (int)trex::EP_MAX_IMPULSE == (int)trex_host::ENVP_MAX_IMPULSE && (int)trex::EP_MU == (int)trex_host::ENVP_MU &&
               (int)trex::EP_MAX_TORQUE == (int)trex_host::ENVP_MAX_TORQUE, "parameter row layout");
+static_assert(TREX_EXT_BODIES == trex_topo::NB && TREX_EXTF_DIM == 6 * 32, "wrench record layout");
+static_assert(sizeof(trex_push_schedule) == 16 * 4, "trex_push_schedule layout");
 
 namespace {
 
@@ -62,13 +64,16 @@ int fail(int code, const char* fmt, const char* detail = "") {
 // PACKED (4 warps per CTA): the inward pass of the CTA's four environments is done by warp 0, four environments at a time.
 // ENVP (trex_config.env_params): every environment's mass scales, friction and motor settings come from its row of envp
 // (indexed like state); without it envp is unused and the instance is the one the library had before the record existed.
-template <int WARPS, bool PACKED, bool ENVP>
+// EXTF (trex_config.external_forces): every environment's wrench record (extf, [6][32] per environment, indexed like state),
+// the COM table com [3][32] and the push schedule enter the bias forces; without it the three are unused.
+template <int WARPS, bool PACKED, bool ENVP, bool EXTF>
 __global__ void __launch_bounds__(32 * WARPS, TREX_MIN_BLOCKS / WARPS)
 trex_front_kernel(const trex::Uniform P, const float* __restrict__ mdl, const int* __restrict__ mdli,
                   const float* __restrict__ tasks, const float* __restrict__ cand_p, const int* __restrict__ cand_lane,
                   float* __restrict__ state, float* __restrict__ work, float* __restrict__ workh, const float* __restrict__ action,
                   int* __restrict__ list, int* __restrict__ list_count, const int* __restrict__ heavy_hint, int heavy_div, int n_envs,
-                  int first_round, const float* __restrict__ envp) {
+                  int first_round, const float* __restrict__ envp, const float* __restrict__ extf, const float* __restrict__ com,
+                  const __grid_constant__ trex::PushSchedule push) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   trex::WarpShared* slabs = reinterpret_cast<trex::WarpShared*>(smem_raw);
   const int warp = threadIdx.x >> 5;
@@ -88,12 +93,13 @@ trex_front_kernel(const trex::Uniform P, const float* __restrict__ mdl, const in
 #ifdef TREX_PHASES
   const long long t_entry = clock64();
 #endif
-  const int front_result = trex::front_phase<PACKED, ENVP>(P, mdl, mdli, tasks, cand_p, cand_lane, slabs[warp], state + (size_t)env * TREX_STATE_STRIDE,
+  const int front_result = trex::front_phase<PACKED, ENVP, EXTF>(P, mdl, mdli, tasks, cand_p, cand_lane, slabs[warp], state + (size_t)env * TREX_STATE_STRIDE,
                                                   work ? work + (size_t)env * TREX_WORK_STRIDE : nullptr, action + (size_t)env * trex::NJ,
                                                   first_round != 0, slabs, warp, valid_mask,
                                                   // class 5 (more than TREX_KC contacts) always goes to its own solver unless heavy_share_div asks for the batch-dependent rule
                                                   (workh != nullptr && (heavy_div <= 0 || (long long)(*heavy_hint) * heavy_div <= (long long)n_envs)) ? workh + (size_t)env * TREX_HEAVY_STRIDE : nullptr,
-                                                  ENVP ? envp + (size_t)env * TREX_ENVP_DIM : nullptr);
+                                                  ENVP ? envp + (size_t)env * TREX_ENVP_DIM : nullptr,
+                                                  EXTF ? extf + (size_t)env * TREX_EXTF_DIM : nullptr, com, &push, (long long)env);
   const int deferred = front_result & 255, n_contacts = front_result >> 8;
   // append to the list of its class of deferred environments (any order: the solver's lane groups are independent):
   // class 0 = contact-free substeps, classes 1..4 = 1 / 2 / 3-4 / 5-8 contacts, 5 = more; list c at list + c * n_envs, counters + 64 * c
@@ -247,6 +253,23 @@ trex_set_env_params_kernel(float* __restrict__ envp, const float* __restrict__ s
   if (env >= n_envs || (mask != nullptr && mask[env] == 0)) return;
   const float* row = src + (size_t)env * TREX_ENVP_DIM;
   envp[i] = k == trex::EP_MAX_IMPULSE ? (float)((double)row[trex::EP_MAX_TORQUE] * dt) : row[k];
+}
+
+// trex_set_external_forces / trex_get_external_forces: user layout [N][26][6] <-> the record [N][6][32] (lanes 26..31 zero).
+// One thread per record element; to_record: all environments, or those with mask != 0.
+__global__ void __launch_bounds__(256)
+trex_external_forces_kernel(float* __restrict__ rec, float* __restrict__ user, const uint8_t* __restrict__ mask, int n_envs,
+                            int to_record) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const long long env = i / TREX_EXTF_DIM;
+  const int c = (int)(i % TREX_EXTF_DIM) / 32, lane = (int)(i % 32);
+  if (env >= n_envs) return;
+  float* u = user + (size_t)env * (TREX_EXT_BODIES * 6) + lane * 6 + c;
+  if (to_record) {
+    if (mask == nullptr || mask[env] != 0) rec[i] = lane < TREX_EXT_BODIES ? *u : 0.0f;
+  } else if (lane < TREX_EXT_BODIES) {
+    *u = rec[i];
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -436,6 +459,11 @@ struct trex_handle {
   bool envp_on = false, ranges_on = false;
   float *d_envp = nullptr, *d_envp_ranges = nullptr;
   double dt = 0.0;              // physics substep in double (the motor impulse bound = torque * dt)
+  // external wrenches (trex_config.external_forces = 1): d_extf [n_envs][6][32], the COM table d_com [3][32], and the push
+  // schedule passed to every front kernel launch (push.on = 0: off)
+  bool extf_on = false;
+  float *d_extf = nullptr, *d_com = nullptr;
+  trex::PushSchedule push = {};
 };
 
 namespace {
@@ -461,7 +489,7 @@ struct HostIO {
   uint8_t* done;
 };
 
-template <int WF, int WS, bool ENVP>
+template <int WF, int WS, bool ENVP, bool EXTF>
 int launch_step(trex_handle* h, const float* action, float* obs, float* reward, uint8_t* done, const uint8_t* mask,
                 int mode, cudaStream_t st, const HostIO* io = nullptr) {
   static const size_t extra_c = getenv("TREX_SOLVEC_EXTRA_SMEM") ? (size_t)atoi(getenv("TREX_SOLVEC_EXTRA_SMEM")) : 0;  // measurement aid: fewer resident warps
@@ -475,7 +503,7 @@ int launch_step(trex_handle* h, const float* action, float* obs, float* reward, 
   std::lock_guard<std::mutex> guard(configure_lock);
   if (!configured[h->device & 15]) {
     int rc;
-    if ((rc = configure_kernel(trex_front_kernel<WF, WF == 4, ENVP>, smem_f)) != TREX_OK) return rc;
+    if ((rc = configure_kernel(trex_front_kernel<WF, WF == 4, ENVP, EXTF>, smem_f)) != TREX_OK) return rc;
     if ((rc = configure_kernel(trex_solve_kernel<WS, 0, 0, 0, ENVP>, smem_s)) != TREX_OK) return rc;
     if ((rc = configure_kernel(trex_solve_kernel<WS, TREX_KC, 1, TREX_CLASS_HEAVY - 1, ENVP>, smem_c)) != TREX_OK) return rc;
     if ((rc = configure_kernel(trex_solve_tm_kernel<1, TREX_CLASS_HEAVY - 1, ENVP>, smem_ct)) != TREX_OK) return rc;
@@ -517,10 +545,12 @@ int launch_step(trex_handle* h, const float* action, float* obs, float* reward, 
     float* work = h->d_work ? h->d_work + q.work_slot * TREX_WORK_STRIDE : nullptr;
     float* workh = h->d_workh ? h->d_workh + q.work_slot * TREX_HEAVY_STRIDE : nullptr;
     float* envp = ENVP ? h->d_envp + e0 * TREX_ENVP_DIM : nullptr;  // rows indexed like state
+    const float* extf = EXTF ? h->d_extf + e0 * TREX_EXTF_DIM : nullptr;  // wrench records indexed like state
     for (int r = 0; r < n_rounds; r++) {
-      trex_front_kernel<WF, WF == 4, ENVP><<<grid1, 32 * WF, smem_f, s>>>(Pc, h->d_mdl, h->d_mdli, h->d_tasks, h->d_cand_p, h->d_cand_lane,
+      trex_front_kernel<WF, WF == 4, ENVP, EXTF><<<grid1, 32 * WF, smem_f, s>>>(Pc, h->d_mdl, h->d_mdli, h->d_tasks, h->d_cand_p, h->d_cand_lane,
                                                           state, work, workh, action + e0 * trex::NJ, q.d_list, q.d_list_count + r,
-                                                          q.d_list_count + 64 * (TREX_NCLASS + 2), h->heavy_div, count, r == 0, envp);
+                                                          q.d_list_count + 64 * (TREX_NCLASS + 2), h->heavy_div, count, r == 0, envp,
+                                                          extf, h->d_com, h->push);
       CUDA_TRY(cudaGetLastError());
       h->launches++;
       if (stagger && c == 0 && r == 0) CUDA_TRY(cudaEventRecord(h->ev_stagger, s));
@@ -603,13 +633,19 @@ int launch_step(trex_handle* h, const float* action, float* obs, float* reward, 
 
 int dispatch_step(trex_handle* h, const float* action, float* obs, float* reward, uint8_t* done, const uint8_t* mask,
                   int mode, cudaStream_t st, const HostIO* io = nullptr) {
-  switch (h->warps_per_block * 2 + (h->envp_on ? 1 : 0)) {
-    case 2: return launch_step<1, 2, false>(h, action, obs, reward, done, mask, mode, st, io);
-    case 4: return launch_step<2, 1, false>(h, action, obs, reward, done, mask, mode, st, io);
-    case 8: return launch_step<4, 4, false>(h, action, obs, reward, done, mask, mode, st, io);
-    case 3: return launch_step<1, 2, true>(h, action, obs, reward, done, mask, mode, st, io);
-    case 5: return launch_step<2, 1, true>(h, action, obs, reward, done, mask, mode, st, io);
-    case 9: return launch_step<4, 4, true>(h, action, obs, reward, done, mask, mode, st, io);
+  switch (h->warps_per_block * 4 + (h->envp_on ? 1 : 0) + (h->extf_on ? 2 : 0)) {
+    case 4: return launch_step<1, 2, false, false>(h, action, obs, reward, done, mask, mode, st, io);
+    case 8: return launch_step<2, 1, false, false>(h, action, obs, reward, done, mask, mode, st, io);
+    case 16: return launch_step<4, 4, false, false>(h, action, obs, reward, done, mask, mode, st, io);
+    case 5: return launch_step<1, 2, true, false>(h, action, obs, reward, done, mask, mode, st, io);
+    case 9: return launch_step<2, 1, true, false>(h, action, obs, reward, done, mask, mode, st, io);
+    case 17: return launch_step<4, 4, true, false>(h, action, obs, reward, done, mask, mode, st, io);
+    case 6: return launch_step<1, 2, false, true>(h, action, obs, reward, done, mask, mode, st, io);
+    case 10: return launch_step<2, 1, false, true>(h, action, obs, reward, done, mask, mode, st, io);
+    case 18: return launch_step<4, 4, false, true>(h, action, obs, reward, done, mask, mode, st, io);
+    case 7: return launch_step<1, 2, true, true>(h, action, obs, reward, done, mask, mode, st, io);
+    case 11: return launch_step<2, 1, true, true>(h, action, obs, reward, done, mask, mode, st, io);
+    case 19: return launch_step<4, 4, true, true>(h, action, obs, reward, done, mask, mode, st, io);
     default: return fail(TREX_ERR_INVALID, "warps_per_block must be 1, 2 or 4%s");
   }
 }
@@ -695,7 +731,12 @@ int trex_create(const void* model_blob, size_t bytes, int32_t n_envs, int32_t de
       return fail(TREX_ERR_INVALID, "trex_config.env_params must be 0 or 1%s");
     }
     h->envp_on = cfg->env_params == 1;
-    for (int i = 0; i < 6; i++)
+    if (cfg->external_forces != 0 && cfg->external_forces != 1) {
+      delete h;
+      return fail(TREX_ERR_INVALID, "trex_config.external_forces must be 0 or 1%s");
+    }
+    h->extf_on = cfg->external_forces == 1;
+    for (int i = 0; i < 5; i++)
       if (cfg->reserved[i] != 0) {
         delete h;
         return fail(TREX_ERR_INVALID, "trex_config.reserved must be zero%s");
@@ -805,6 +846,12 @@ int trex_create(const void* model_blob, size_t bytes, int32_t n_envs, int32_t de
     CTRY(cudaMemcpy(h->d_envp, rows.data(), rows.size() * sizeof(float), cudaMemcpyHostToDevice));
     CTRY(cudaMalloc((void**)&h->d_envp_ranges, 2 * TREX_ENVP_DIM * sizeof(float)));
   }
+  if (h->extf_on) {  // the record starts at zero
+    CTRY(cudaMalloc((void**)&h->d_extf, N * TREX_EXTF_DIM * sizeof(float)));
+    CTRY(cudaMemset(h->d_extf, 0, N * TREX_EXTF_DIM * sizeof(float)));
+    CTRY(cudaMalloc((void**)&h->d_com, h->T.com.size() * sizeof(float)));
+    CTRY(cudaMemcpy(h->d_com, h->T.com.data(), h->T.com.size() * sizeof(float), cudaMemcpyHostToDevice));
+  }
 #undef CTRY
   // all environments start from the reference reset (TrexBulletEnv.__init__ calls reset(), trex_env.py:92)
   rc = trex_reset(h, nullptr, nullptr, nullptr);
@@ -824,6 +871,7 @@ void trex_destroy(trex_handle* h) {
   cudaFree(h->d_work); cudaFree(h->d_workh);
   cudaFree(h->d_lower); cudaFree(h->d_upper); cudaFree(h->d_state); cudaFree(h->d_aux); cudaFree(h->d_stats);
   cudaFree(h->d_envp); cudaFree(h->d_envp_ranges);
+  cudaFree(h->d_extf); cudaFree(h->d_com);
   for (int b = 0; b < 2; b++) {
     cudaFree(h->d_action[b]); cudaFree(h->d_obs[b]); cudaFree(h->d_reward[b]); cudaFree(h->d_done[b]);
     if (h->ev_step_done[b]) cudaEventDestroy(h->ev_step_done[b]);
@@ -1016,6 +1064,52 @@ int trex_set_env_param_ranges(trex_handle* h, const float* lo32_host, const floa
   CUDA_TRY(cudaDeviceSynchronize());
   CUDA_TRY(cudaMemcpy(h->d_envp_ranges, both, sizeof both, cudaMemcpyHostToDevice));
   h->ranges_on = true;
+  return TREX_OK;
+}
+
+int trex_set_external_forces(trex_handle* h, const float* wrench_dev, const uint8_t* mask_dev, void* stream) {
+  if (!h || !wrench_dev) return fail(TREX_ERR_INVALID, "NULL argument%s");
+  if (!h->extf_on) return fail(TREX_ERR_INVALID, "trex_set_external_forces: the handle was created with external_forces = 0%s");
+  CUDA_TRY(cudaSetDevice(h->device));
+  const long long total = (long long)h->n_envs * TREX_EXTF_DIM;
+  trex_external_forces_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+      h->d_extf, const_cast<float*>(wrench_dev), mask_dev, h->n_envs, 1);
+  CUDA_TRY(cudaGetLastError());
+  h->launches++;
+  return TREX_OK;
+}
+
+int trex_get_external_forces(trex_handle* h, float* wrench_dev, void* stream) {
+  if (!h || !wrench_dev) return fail(TREX_ERR_INVALID, "NULL argument%s");
+  if (!h->extf_on) return fail(TREX_ERR_INVALID, "trex_get_external_forces: the handle was created with external_forces = 0%s");
+  CUDA_TRY(cudaSetDevice(h->device));
+  const long long total = (long long)h->n_envs * TREX_EXTF_DIM;
+  trex_external_forces_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->d_extf, wrench_dev, nullptr,
+                                                                                                   h->n_envs, 0);
+  CUDA_TRY(cudaGetLastError());
+  h->launches++;
+  return TREX_OK;
+}
+
+int trex_set_push_schedule(trex_handle* h, const trex_push_schedule* s) {
+  if (!h) return fail(TREX_ERR_INVALID, "handle is NULL%s");
+  if (!h->extf_on) return fail(TREX_ERR_INVALID, "trex_set_push_schedule: the handle was created with external_forces = 0%s");
+  if (!s) {
+    h->push.on = 0;
+    return TREX_OK;
+  }
+  if (const char* why = trex_host::check_push_schedule(s->body, s->interval, s->duration, s->first_step, s->probability,
+                                                       s->force_min, s->force_max))
+    return fail(TREX_ERR_INVALID, "trex_set_push_schedule: %s", why);
+  for (int i = 0; i < 9; i++)
+    if (s->reserved[i] != 0) return fail(TREX_ERR_INVALID, "trex_set_push_schedule: reserved must be zero%s");
+  trex::PushSchedule p = {};
+  p.on = 1;
+  p.lane = s->body;  // record order = lane order
+  p.interval = s->interval; p.duration = s->duration; p.first_step = s->first_step;
+  p.probability = s->probability; p.force_min = s->force_min; p.force_max = s->force_max;
+  trex_host::push_directions(p.dir);
+  h->push = p;
   return TREX_OK;
 }
 

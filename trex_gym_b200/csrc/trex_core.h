@@ -231,6 +231,58 @@ enum { EP_MASS_BASE = 25, EP_MU = 26, EP_KP = 27, EP_KD = 28, EP_MAX_TORQUE = 29
 #define TREX_ENVP_PHILOX_KEY 0xe9a5u
 TREX_FN vf envp_mass_scale(const float* envp, vi lane) { return ld_if(envp, seli(lane <= EP_MASS_BASE, lane, 0), lane <= EP_MASS_BASE, 1.0f); }
 
+// ---- external wrenches (trex_config.external_forces = 1; the EXTF instances of the front kernel) ------------------------
+// Record of one environment, lane-major [6][32]: element c * 32 + L = component c of the wrench on the body of lane L (the
+// lane numbering of the kernels: L < 25 the body of joint L, 25 the base; lanes 26..31 hold zeros).  Components
+// fx fy fz tx ty tz in the world frame: the force acts at the body's centre of mass, the torque is a free vector.  A warp
+// reads it with six coalesced 128-byte loads per substep.  com: [3][32] body-frame centre of mass of each lane's body
+// (mc / mass of the model, rounded from double; a mass scale leaves it unchanged).
+#define TREX_EXTF_DIM (6 * 32)
+#define TREX_PUSH_DIRS 32
+// the push schedule's Philox key word (0xfa11: reset sampler, 0xe9a5: parameter randomizer)
+#define TREX_PUSH_PHILOX_KEY 0x9e57u
+// Push schedule (a kernel argument; on == 0: off).  dir: 32 horizontal unit vectors (cos, sin of 2 pi k / 32, rounded
+// from double on the host: a table keeps the device and the emulator bit-identical where sinf / cosf would not).
+struct PushSchedule {
+  int on, lane, interval, duration, first_step;
+  float probability, force_min, force_max;
+  float dir[TREX_PUSH_DIRS][2];
+};
+// The wrench inputs of one substep: the environment's record, the COM table, and the push of this substep (warp-uniform;
+// lane < 0: none) that is added to the record's force on that lane before the rotation into the body frame.
+struct ExtWrench {
+  const float* rec = nullptr;
+  const float* com = nullptr;
+  int push_lane = -1;
+  float push_fx = 0.0f, push_fy = 0.0f;
+};
+// The schedule of environment gid at env step t (steps completed in episode e): window w = t / interval; Philox4x32-10
+// keyed by (seed, TREX_PUSH_PHILOX_KEY), counter (gid lo, gid hi, e, w) -> u0..u3.  The window holds a push iff
+// u0 < probability, starting at onset o = min(floor(u1 (interval - duration + 1)), interval - duration) into the window
+// and lasting `duration` steps; steps before first_step never push.  Magnitude force_min + u2 (force_max - force_min)
+// (one fused multiply-add), direction dir[floor(32 u3)].  Stateless: a function of (seed, gid, e, t) only, so it
+// depends neither on the number of GPUs nor on when the schedule was set.  Called warp-uniformly.
+TREX_FN void push_of_step(const PushSchedule& S, unsigned seed, unsigned long long gid, float episode, float step, ExtWrench& X) {
+  const int t = (int)step;
+  if (!S.on || t < S.first_step) return;
+  const int w = t / S.interval;
+  vf u[4];
+  philox4_uniform(vi((int)(unsigned)(gid & 0xffffffffull)), vi((int)(unsigned)(gid >> 32)), vi((int)episode), vi(w), seed,
+                  TREX_PUSH_PHILOX_KEY, u);
+  const float u0 = lane_value(u[0], 0), u1 = lane_value(u[1], 0), u2 = lane_value(u[2], 0), u3 = lane_value(u[3], 0);
+  if (!(u0 < S.probability)) return;
+  const int span = S.interval - S.duration;
+  int o = (int)(u1 * (float)(span + 1));
+  o = o < span ? o : span;
+  const int r = t - w * S.interval;
+  if (r < o || r >= o + S.duration) return;
+  const float mag = fmaf(u2, S.force_max - S.force_min, S.force_min);
+  const int d = (int)(u3 * (float)TREX_PUSH_DIRS);
+  X.push_lane = S.lane;
+  X.push_fx = mag * S.dir[d][0];
+  X.push_fy = mag * S.dir[d][1];
+}
+
 // btClamp semantics: comparison based, so a NaN stays a NaN (fmin/fmax would launder it into a bound)
 TREX_FN vf clampv(vf x, float lo, float hi) { return sel(x < lo, lo, sel(x > hi, hi, x)); }
 TREX_FN float clampf(float x, float lo, float hi) { return x < lo ? lo : (x > hi ? hi : x); }
@@ -572,11 +624,12 @@ TREX_FN void inward_packed(const Uniform& P, const float* mdl, const int* mdli, 
 // PACKED (front kernel with 4-warp CTAs): the inward pass of the CTA's four environments is done by warp 0
 // (inward_packed) between two CTA barriers; cta_slabs = slab of warp 0, valid_mask = which warps hold an environment.
 // ENVP: envp = this environment's parameter row (mass scales and friction; the caller passes the row's motor settings)
-template <bool PACKED = false, bool ENVP = false>
+// EXTF: *xf = the external wrenches of this substep (record, COM table, scheduled push)
+template <bool PACKED = false, bool ENVP = false, bool EXTF = false>
 TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const float* tasks, const float* cand_p,
                      const int* cand_lane, WarpShared& S, EnvRegs& R, float kp, float kd, float max_imp,
                      StepStats& stats, float* work, WarpShared* cta_slabs = nullptr, int warp_in_cta = 0, int valid_mask = 0,
-                     float* workh = nullptr, const float* envp = nullptr) {
+                     float* workh = nullptr, const float* envp = nullptr, const ExtWrench* xf = nullptr) {
   const vi lane = lane_id();
   const vb is_joint = lane < NJ;
   const vb is_base = lane == 25;
@@ -632,6 +685,30 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
     pA[1] -= mc[2] * gx - mc[0] * gz;
     pA[2] -= mc[0] * gy - mc[1] * gx;
     pA[3] -= mass * gx; pA[4] -= mass * gy; pA[5] -= mass * gz;
+    if (EXTF) {
+      // external wrench (world force F at the COM c, world torque T), entering like gravity:
+      // f_b = Rw F, n_b = c x f_b + Rw T (Rw: world -> body; the gravity term above reads its third column)
+      vf F[3], T[3], c[3];
+      TREX_UNROLL for (int k = 0; k < 3; k++) {
+        F[k] = ld(xf->rec, lane + k * 32);
+        T[k] = ld(xf->rec, lane + (3 + k) * 32);
+        c[k] = ldg_ro(xf->com, lane + k * 32);
+      }
+      if (xf->push_lane >= 0) {  // the scheduled push joins the record's force before the rotation
+        const vb on = lane == xf->push_lane;
+        F[0] = sel(on, F[0] + xf->push_fx, F[0]);
+        F[1] = sel(on, F[1] + xf->push_fy, F[1]);
+      }
+      vf fb[3], nb[3];
+      TREX_UNROLL for (int i = 0; i < 3; i++) {
+        fb[i] = Rw[3 * i] * F[0] + Rw[3 * i + 1] * F[1] + Rw[3 * i + 2] * F[2];
+        nb[i] = Rw[3 * i] * T[0] + Rw[3 * i + 1] * T[1] + Rw[3 * i + 2] * T[2];
+      }
+      nb[0] += c[1] * fb[2] - c[2] * fb[1];
+      nb[1] += c[2] * fb[0] - c[0] * fb[2];
+      nb[2] += c[0] * fb[1] - c[1] * fb[0];
+      TREX_UNROLL for (int k = 0; k < 3; k++) { pA[k] -= nb[k]; pA[3 + k] -= fb[k]; }
+    }
     // angular damping of every URDF link of the body: (sum R I R^T) w (k + k|w|)
     vf dr[6];
     TREX_UNROLL for (int k = 0; k < 6; k++) dr[k] = ENVP ? MDL(F_DROT + k) * msc : MDL(F_DROT + k);
@@ -2541,11 +2618,14 @@ static_assert(ST_SIG == ST_ACC_ITERS + 3, "front_phase stores the four accumulat
 // contacts the substep is finished here (one-environment solver + integration); otherwise the solver inputs go to
 // `work` and the function returns 1 + class (solve_phase finishes the substep).   action: [25] name-sorted (trex_robot.py:311-314)
 // ENVP: envp = the environment's parameter row (mass scales, friction, motor gains and impulse bound)
-template <bool PACKED = false, bool ENVP = false>
+// EXTF: extf = the environment's wrench record [6][32], com = the COM table [3][32], push = the push schedule,
+// env_id = index of the environment in this launch (P.env_offset + env_id keys the schedule)
+template <bool PACKED = false, bool ENVP = false, bool EXTF = false>
 TREX_FN int front_phase(const Uniform& P, const float* mdl, const int* mdli, const float* tasks, const float* cand_p,
                          const int* cand_lane, WarpShared& S, float* rec, float* work, const float* action, bool first_round,
                          WarpShared* cta_slabs = nullptr, int warp_in_cta = 0, int valid_mask = 0, float* workh = nullptr,
-                         const float* envp = nullptr) {
+                         const float* envp = nullptr, const float* extf = nullptr, const float* com = nullptr,
+                         const PushSchedule* push = nullptr, long long env_id = 0) {
   const vi lane = lane_id();
   const vb is_joint = lane < NJ;
   const vi slot = seli(is_joint, MDLI(IF_OBS_SLOT), 0);
@@ -2562,8 +2642,15 @@ TREX_FN int front_phase(const Uniform& P, const float* mdl, const int* mdli, con
 #endif
   const float kp = ENVP ? ldu(envp, EP_KP) : P.kp, kd = ENVP ? ldu(envp, EP_KD) : P.kd;
   const float max_imp = ENVP ? ldu(envp, EP_MAX_IMPULSE) : P.max_impulse;
-  const int deferred = substep<PACKED, ENVP>(P, mdl, mdli, tasks, cand_p, cand_lane, S, R, kp, kd, max_imp, st, work, cta_slabs,
-                                             warp_in_cta, valid_mask, workh, envp);
+  ExtWrench xf;
+  if (EXTF) {
+    xf.rec = extf;
+    xf.com = com;
+    // the step count as the tail kernel left it: steps completed in this episode
+    push_of_step(*push, P.seed, (unsigned long long)(P.env_offset + env_id), ldu(rec, ST_EPISODE), ldu(rec, ST_STEP), xf);
+  }
+  const int deferred = substep<PACKED, ENVP, EXTF>(P, mdl, mdli, tasks, cand_p, cand_lane, S, R, kp, kd, max_imp, st, work, cta_slabs,
+                                                   warp_in_cta, valid_mask, workh, envp, EXTF ? &xf : nullptr);
   store_env(rec, lane, S, R);  // deferred: positions unchanged, velocities after the unconstrained update
   const float it0 = first_round ? 0.0f : ldu(rec, ST_ACC_ITERS), ov0 = first_round ? 0.0f : ldu(rec, ST_ACC_OVERFLOW);
   vf acc = 0.0f;

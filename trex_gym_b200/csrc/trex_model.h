@@ -2,6 +2,7 @@
 // as the lane-indexed tables trex_core.h consumes.  Plain C++ (no CUDA) so that both the
 // library (trex_capi.cu) and the CPU test emulator (tests/emu) build the tables identically.
 #pragma once
+#include <math.h>
 #include <stdint.h>
 #include <string.h>
 
@@ -79,6 +80,7 @@ struct ModelTables {
   std::vector<float> tasks;      // [rounds][4][32]  rx, ry, rz, mass
   std::vector<float> cand_p;     // [4][64]: candidate point / sphere centre x, y, z in body coordinates, sphere radius (0 = point)
   std::vector<int32_t> cand_lane;  // [64]
+  std::vector<float> com;        // [3][32]: body-frame centre of mass (mc / mass in double) of each lane's body, 0 elsewhere
   int n_rounds = 0, n_cand = 0, head_lane = 0;
   float head_p[3] = {0, 0, 0};
   float r0[trex_topo::NB][3];
@@ -135,6 +137,9 @@ static inline bool build_tables(const void* blob, size_t bytes, ModelTables& T, 
     for (int k = 0; k < 6; k++) F(22 + k, L) = (float)drot[6 * b + k];
     F(28, L) = (float)lower[b]; F(29, L) = (float)upper[b]; F(30, L) = (float)jdamp[b]; F(31, L) = (float)startq[b];
   }
+  T.com.assign(3 * 32, 0.0f);
+  for (int b = 0; b < NB; b++)
+    for (int k = 0; k < 3; k++) T.com[(size_t)k * 32 + body_lane(b)] = mass[b] > 0.0 ? (float)(mc[3 * b + k] / mass[b]) : 0.0f;
   // identity rotation for lanes without a body (harmless arithmetic)
   for (int L = 26; L < 32; L++) { F(0, L) = 1.0f; F(4, L) = 1.0f; F(8, L) = 1.0f; }
   // int fields
@@ -333,6 +338,29 @@ static inline const char* check_env_param_ranges(const float lo[ENVP_DIM], const
     if (k >= ENVP_MAX_IMPULSE && (lo[k] != 0.0f || hi[k] != 0.0f)) return "elements 30 and 31 of the ranges must be zero";
   }
   return nullptr;
+}
+
+// ---- push schedule (trex_core.h: PushSchedule, push_of_step) ----------------------------------------------------------
+// body 0..25 (wrench-record order: 25 = base), interval >= 1, 1 <= duration <= interval, first_step >= 0,
+// 0 <= probability <= 1, 0 <= force_min <= force_max, all finite.  Returns nullptr when valid, else what is wrong.
+static inline const char* check_push_schedule(int body, int interval, int duration, int first_step, float probability,
+                                              float force_min, float force_max) {
+  if (body < 0 || body > 25) return "body must be 0..25 (25 = base)";
+  if (interval < 1) return "interval must be >= 1";
+  if (duration < 1 || duration > interval) return "duration must be 1..interval";
+  if (first_step < 0) return "first_step must be >= 0";
+  if (!(probability >= 0.0f && probability <= 1.0f)) return "probability must be in [0, 1]";
+  if (!(force_min - force_min == 0.0f) || !(force_max - force_max == 0.0f)) return "forces must be finite";
+  if (!(force_min >= 0.0f && force_min <= force_max)) return "0 <= force_min <= force_max must hold";
+  return nullptr;
+}
+// the 32 horizontal push directions (cos, sin of 2 pi k / 32), computed in double and rounded once
+static inline void push_directions(float dir[32][2]) {
+  for (int k = 0; k < 32; k++) {
+    const double a = 6.283185307179586476925 * k / 32.0;
+    dir[k][0] = (float)cos(a);
+    dir[k][1] = (float)sin(a);
+  }
 }
 
 }  // namespace trex_host

@@ -897,6 +897,29 @@ def with_body_mass_scale(model: CompiledModel, scales) -> CompiledModel:
     return CompiledModel(S, dict(model.meta))
 
 
+def link_wrenches(model: CompiledModel, body_wrench) -> np.ndarray:
+    """The links' share of per-body external wrenches, for the reference simulator (``oracle``), which keeps every URDF link.
+
+    ``body_wrench``: [26, 6] in the order of an external-wrench record (``TrexBatchSim.set_external_forces``: ``[k]`` for
+    the body of joint ``k`` (body ``k + 1``), ``[25]`` for the base), world force at the body's COM then world torque.
+    Returns [n_links + 1, 6], base first: each link carries the body's force times its share of the body's mass (the
+    mass-weighted link COMs average to the body COM, so the split adds no moment), and the body's torque sits on its first
+    link."""
+    w = np.asarray(body_wrench, np.float64)
+    nb = int(model.sections["mb_n_bodies"][0])
+    if w.shape != (nb, 6):
+        raise ValueError("body_wrench must have shape (%d, 6)" % nb)
+    by_body = np.concatenate([w[nb - 1:], w[:nb - 1]])  # body index order: base first
+    task_body = np.asarray(model.sections["mb_task_body"])  # body of every link, in link order (base first)
+    mass = np.asarray(model.sections["full_mass"], np.float64)
+    body_mass = np.bincount(task_body, weights=mass, minlength=nb)
+    out = np.zeros((task_body.shape[0], 6))
+    out[:, :3] = by_body[task_body, :3] * (mass / body_mass[task_body])[:, None]
+    for b in range(nb):
+        out[int(np.flatnonzero(task_body == b)[0]), 3:] = by_body[b, 3:]
+    return out
+
+
 def emit_topology_header(model: CompiledModel) -> str:
     """C header with the merged tree as compile-time constants.
 

@@ -28,7 +28,7 @@ class TrexBatchSim:
                  seed: int = 0, warps_per_block: int | None = None, reset_mode: int = 0, env_offset: int = 0,
                  deferred_solve: bool = True, defer_contacts: bool = True, heavy_solver: bool = True,
                  heavy_share_div: int = 0, pipelines: int = 0, heavy_memory: int = 0, chunk_envs: int = 0, contact_memory: int = 0,
-                 env_params: bool = False):
+                 env_params: bool = False, external_forces: bool = False):
         if not torch.cuda.is_available():
             raise RuntimeError("trex_gym_b200 needs a CUDA device (no CPU fallback)")
         dev = torch.device(device if not isinstance(device, int) else "cuda:%d" % device)
@@ -61,6 +61,8 @@ class TrexBatchSim:
         cfg.chunk_envs = int(chunk_envs)  # 0 = default; L2-resident work records (include/trex_b200.h), -1 = off
         cfg.env_params = int(bool(env_params))  # per-environment dynamics parameters (set_env_params)
         self.env_params = bool(env_params)
+        cfg.external_forces = int(bool(external_forces))  # per-environment external wrenches (set_external_forces)
+        self.external_forces = bool(external_forces)
         blob = self.model.blob()
         h = ctypes.c_void_p()
         idx = dev.index if dev.index is not None else torch.cuda.current_device()
@@ -303,6 +305,89 @@ class TrexBatchSim:
         lo[30:] = 0.0
         hi[30:] = 0.0
         _native.check(self._L.trex_set_env_param_ranges(self._h, lo.ctypes.data, hi.ctypes.data), "trex_set_env_param_ranges")
+
+    # -- external forces and torques (external_forces=True) ------------------------------------------------------
+    # A wrench is [fx fy fz tx ty tz] in the world frame on one of 26 bodies (body k < 25: the body of joint k in pybullet link
+    # order, 25: the base); the force acts at the body's centre of mass (body_com), the torque is free.  Unlike pybullet's
+    # applyExternalForce, which lasts one stepSimulation, the wrenches stay until set again; they act in every physics
+    # substep of a step, never in the physics step of a reset, and survive resets.
+
+    def _need_external_forces(self):
+        if not self.external_forces:
+            raise ValueError("the simulator was created with external_forces=False")
+
+    def _mask_ptr(self, mask):
+        if mask is None:
+            return None, None
+        mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
+        if mask.shape != (self.num_envs,):
+            raise ValueError("mask must have shape (num_envs,)")
+        return mask, ctypes.c_void_p(mask.data_ptr())
+
+    def body_com(self) -> np.ndarray:
+        """[26, 3] centre of mass of every body in its own frame (the point the force of a wrench acts at), float32, in
+        wrench-body order.  A torque about another point p of body k is the torque at the COM plus (p - com) x F in world
+        coordinates."""
+        from .model_blob import unpack
+        sec = unpack(self.model.blob())
+        mass, mc = sec["mb_mass"], sec["mb_mc"].reshape(-1, 3)
+        bodies = [k + 1 for k in range(_native.EXT_BODIES - 1)] + [0]
+        return np.stack([(mc[b] / mass[b]) if mass[b] > 0 else np.zeros(3) for b in bodies]).astype(np.float32)
+
+    def set_external_forces(self, force, torque=None, bodies=None, mask: torch.Tensor | None = None) -> None:
+        """Replace the wrenches of all (or the masked) environments.  ``force`` / ``torque`` (None: zero): [N, 26, 3], or
+        [N, len(bodies), 3] with ``bodies`` a list of body names (joint names of ``meta["body_joint_names"]`` or
+        ``"base"``); bodies not named get zero."""
+        self._need_external_forces()
+        n = self.num_envs
+        cols = list(range(_native.EXT_BODIES)) if bodies is None else [self._body_index(b) for b in bodies]
+        if len(set(cols)) != len(cols):
+            raise ValueError("a body is named twice")
+
+        def part(x, what):
+            if x is None:
+                return torch.zeros(n, len(cols), 3, device=self.device, dtype=torch.float32)
+            x = torch.as_tensor(x, dtype=torch.float32).to(self.device)
+            if tuple(x.shape) != (n, len(cols), 3):
+                raise ValueError("%s must have shape %s" % (what, (n, len(cols), 3)))
+            return x
+        w = torch.zeros(n, _native.EXT_BODIES, 6, device=self.device, dtype=torch.float32)
+        w[:, cols, 0:3] = part(force, "force")
+        w[:, cols, 3:6] = part(torque, "torque")
+        if not bool(torch.isfinite(w).all()):
+            raise ValueError("external forces must be finite")
+        mask, mp = self._mask_ptr(mask)
+        _native.check(self._L.trex_set_external_forces(self._h, ctypes.c_void_p(w.data_ptr()), mp, self._stream()),
+                      "trex_set_external_forces")
+        self._extf_src = (w, mask)  # kept alive until the stream has consumed them
+
+    def get_external_forces(self) -> torch.Tensor:
+        """[N, 26, 6] copy of every environment's wrenches."""
+        self._need_external_forces()
+        t = torch.empty(self.num_envs, _native.EXT_BODIES, 6, device=self.device, dtype=torch.float32)
+        _native.check(self._L.trex_get_external_forces(self._h, ctypes.c_void_p(t.data_ptr()), self._stream()),
+                      "trex_get_external_forces")
+        return t
+
+    def clear_external_forces(self, mask: torch.Tensor | None = None) -> None:
+        """Zero the wrenches of all (or the masked) environments."""
+        self.set_external_forces(None, mask=mask)
+
+    def set_push_schedule(self, body="base", interval: int = 100, duration: int = 10, probability: float = 1.0,
+                          force=(0.0, 0.0), first_step: int = 0) -> None:
+        """Random horizontal pushes on ``body``, drawn on the device per environment and ``interval``-step window: with
+        chance ``probability`` a window holds one push of ``duration`` steps, magnitude uniform in ``force = (lo, hi)`` N and
+        one of 32 horizontal directions; none before ``first_step`` of an episode (include/trex_b200.h,
+        trex_set_push_schedule).  The push adds to the body's force in the record.  ``set_push_schedule(None)`` turns it off."""
+        self._need_external_forces()
+        if body is None:
+            _native.check(self._L.trex_set_push_schedule(self._h, None), "trex_set_push_schedule")
+            return
+        lo, hi = force
+        s = _native.TrexPushSchedule(body=self._body_index(body), interval=int(interval), duration=int(duration),
+                                     first_step=int(first_step), probability=float(probability), force_min=float(lo),
+                                     force_max=float(hi))
+        _native.check(self._L.trex_set_push_schedule(self._h, ctypes.byref(s)), "trex_set_push_schedule")
 
     # -- state / diagnostics -----------------------------------------------------------------------
     def get_state(self) -> torch.Tensor:

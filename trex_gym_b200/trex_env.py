@@ -141,10 +141,12 @@ class TrexVecEnv(object):
 
     def __init__(self, num_envs, urdf_path=None, distance_weight=1.0, energy_weight=0.005, drift_weight=0.002,
                  device=0, model=None, num_substeps=NUM_SUBSTEPS, max_episode_steps=0, contacts=True, seed=0, contact_model="points",
-                 literal_reference=False, randomize=None):
+                 literal_reference=False, randomize=None, pushes=None):
         """``randomize``: None, or a dict of parameter name -> (low, high) -- ``mass_scale`` (a scale, or {body: scale}),
         ``friction``, ``kp``, ``kd``, ``max_torque`` -- drawn per environment at every reset (``TrexBatchSim.set_env_param_ranges``);
-        parameters not named keep the model's value."""
+        parameters not named keep the model's value.
+        ``pushes``: None, or the keyword arguments of ``TrexBatchSim.set_push_schedule`` (``body``, ``interval``, ``duration``,
+        ``probability``, ``force=(lo, hi)``, ``first_step``): random horizontal pushes drawn on the device."""
         if literal_reference:  # see TrexBulletEnv
             contacts = False
             mdl = model if model is not None else load_builtin("literal")
@@ -152,9 +154,12 @@ class TrexVecEnv(object):
             mdl = model if model is not None else _load_model(urdf_path, contact_model)
         self.sim = TrexBatchSim(num_envs, device=device, model=mdl, num_substeps=num_substeps,
                                 distance_weight=distance_weight, energy_weight=energy_weight, drift_weight=drift_weight,
-                                max_episode_steps=max_episode_steps, contacts=contacts, seed=seed, env_params=randomize is not None)
+                                max_episode_steps=max_episode_steps, contacts=contacts, seed=seed, env_params=randomize is not None,
+                                external_forces=pushes is not None)
         if randomize is not None:
             self.sim.set_env_param_ranges({k: v[0] for k, v in randomize.items()}, {k: v[1] for k, v in randomize.items()})
+        if pushes is not None:
+            self.sim.set_push_schedule(**pushes)
         self.num_envs = int(num_envs)
         lo, hi = self.sim.action_low, self.sim.action_high
         self.action_space = spaces.Box(low=lo, high=hi, dtype=np.float32)
