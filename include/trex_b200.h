@@ -251,6 +251,34 @@ int trex_set_push_schedule(trex_handle* h, const trex_push_schedule* s_host);
 #define TREX_BODY_STATE_DIM 13
 int trex_get_body_states(trex_handle* h, float* states_dev, float* contact_force_dev, void* stream);
 
+/* Joint-space mass matrix, bias forces and body Jacobians, computed on the device from the environment records (pybullet's
+ * calculateMassMatrix, calculateInverseDynamics with zero accelerations and calculateJacobian at every body's COM; Isaac
+ * Gym's mass-matrix and Jacobian tensors).  Works on every handle; reads the records only (the step's results are
+ * unchanged); stream ordered, capturable.  Any output may be NULL, not all three (TREX_ERR_INVALID); a NULL output is not
+ * computed.  With trex_config.env_params = 1 the environment's mass scales apply (mass, first moment and inertia).
+ *   Generalized velocity u [TREX_NUM_DOFS] -- the record's own velocity layout:
+ *     u[0:3]  = record [7:10]:  base angular velocity, world frame
+ *     u[3:6]  = record [10:13]: velocity of the base link's COM (the record's position [0:3], the origin of the base frame),
+ *               world frame.  The merged base body (body 25 below) also holds the links fixed to the base, so its COM is
+ *               elsewhere
+ *     u[6:31] = record [38:63]: joint rates in pybullet link order (TrexBatchSim.dof_names()), NOT the name-sorted
+ *               action / observation order: action slot i drives joint obs_dof[i] (model section obs_dof), whose rate is
+ *               u[6 + obs_dof[i]]
+ *   mass_matrix_dev [N][31][31] float32: M with kinetic energy = 1/2 u^T M u; stored full and exactly symmetric (one triangle
+ *     is computed and mirrored)
+ *   bias_dev [N][31] float32: b with M du/dt + b = tau, du/dt the time derivative of u in the coordinates above: gravity plus
+ *     the Coriolis and centrifugal terms.  b does NOT contain link or joint damping, motors, joint limits, contacts or the
+ *     external-wrench record.  The generalized force tau of u[0:6] is the torque about the base link's COM, then the force
+ *     (world).  Joint torques of given accelerations: tau = M du/dt + b, in torch (M @ udot[..., None])[..., 0] + b
+ *   jacobian_dev [N][26][TREX_JACOBIAN_ROWS][31] float32: J_k of body k (numbered as in the wrench record and
+ *     trex_get_body_states: body k < 25 is the body moved by joint k, body 25 the base), rows [v_COM (3); w (3)] in the world
+ *     frame, linear first: J_k u = states[k][7:13] of trex_get_body_states.  The point is the body's COM as in the wrench
+ *     record and the body states (the composite COM of the merged body), so sum_k J_k^T [f_k; t_k] is the generalized force
+ *     of a wrench record.  A point p of body k moves with v_p = v_COM + w x (p - COM). */
+#define TREX_NUM_DOFS 31
+#define TREX_JACOBIAN_ROWS 6
+int trex_get_dynamics(trex_handle* h, float* mass_matrix_dev, float* bias_dev, float* jacobian_dev, void* stream);
+
 /* per-env diagnostics of the last step: head xyz (trex_robot.py:330-335), the three penalty terms
  * logged at trex_env.py:193-195 (lifting, station keeping, energy), PGS iterations, contacts. */
 int trex_get_aux(trex_handle* h, float* aux_dev, void* stream);

@@ -20,6 +20,8 @@ AUX_DIM = 8
 ENV_PARAM_DIM = 32  # per-environment parameter row (include/trex_b200.h, trex_set_env_params)
 EXT_BODIES = 26  # bodies of the external-wrench layout [N][26][6] (include/trex_b200.h, trex_set_external_forces)
 BODY_STATE_DIM = 13  # floats of a body row of trex_get_body_states: p | q | v | w
+NUM_DOFS = 31  # generalized coordinates of trex_get_dynamics: base angular | base linear | 25 joints in link order
+JACOBIAN_ROWS = 6  # rows of a body Jacobian: v_COM | w
 
 EXPORTED_SYMBOLS = (
     "trex_create", "trex_destroy", "trex_reset", "trex_step", "trex_step_host", "trex_step_host_async", "trex_host_wait",
@@ -27,7 +29,7 @@ EXPORTED_SYMBOLS = (
     "trex_get_state", "trex_set_state", "trex_get_aux", "trex_get_joint_limits",
     "trex_set_env_params", "trex_get_env_params", "trex_set_env_param_ranges",
     "trex_set_external_forces", "trex_get_external_forces", "trex_set_push_schedule",
-    "trex_get_body_states",
+    "trex_get_body_states", "trex_get_dynamics",
     "trex_fill_random_actions", "trex_get_stats", "trex_measure_fp32_peak", "trex_gae", "trex_normalize",
     "trex_policy_param_count", "trex_policy_forward", "trex_kernel_launches", "trex_num_envs",
     "trex_last_error", "trex_version",
@@ -154,6 +156,8 @@ def lib():
     L.trex_get_external_forces.argtypes = [vp, fp, vp]
     L.trex_get_body_states.restype = ctypes.c_int
     L.trex_get_body_states.argtypes = [vp, vp, vp, vp]
+    L.trex_get_dynamics.restype = ctypes.c_int
+    L.trex_get_dynamics.argtypes = [vp, vp, vp, vp, vp]
     L.trex_set_push_schedule.restype = ctypes.c_int
     L.trex_set_push_schedule.argtypes = [vp, ctypes.POINTER(TrexPushSchedule)]
     L.trex_get_joint_limits.restype = ctypes.c_int

@@ -42,6 +42,8 @@ static_assert(TREX_ENV_PARAM_DIM == TREX_ENVP_DIM && TREX_ENVP_DIM == (int)trex_
 static_assert(TREX_EXT_BODIES == trex_topo::NB && TREX_EXTF_DIM == 6 * 32, "wrench record layout");
 static_assert(sizeof(trex_push_schedule) == 16 * 4, "trex_push_schedule layout");
 static_assert(TREX_BODY_STATE_DIM == TREX_BODY_DIM && TREX_BODY_STAGE == TREX_EXT_BODIES * TREX_BODY_STATE_DIM, "body state layout");
+static_assert(TREX_NUM_DOFS == TREX_DYN_NDOF && TREX_NUM_DOFS == trex_topo::NDOF && TREX_JACOBIAN_ROWS == TREX_DYN_JROWS &&
+              (TREX_DYN_STAGE % 4) == 0, "dynamics layout");
 
 namespace {
 
@@ -288,6 +290,23 @@ trex_body_states_kernel(const trex::Uniform P, const float* __restrict__ mdl, co
                           states ? states + (size_t)env * TREX_BODY_STAGE : nullptr, forces ? forces + (size_t)env * trex::NB : nullptr);
 }
 
+// trex_get_dynamics: one warp per environment (trex_core.h: dynamics_phase); reads the records, the model tables and (with
+// env_params) the parameter rows, writes only the outputs.  The warp's subtree sums and its M are staged in a 5,136-byte
+// slice of static shared memory.
+#define TREX_DYN_WARPS 8
+__global__ void __launch_bounds__(32 * TREX_DYN_WARPS)
+trex_dynamics_kernel(const trex::Uniform P, const float* __restrict__ mdl, const int* __restrict__ mdli,
+                     const float* __restrict__ com, const float* __restrict__ envp, const float* __restrict__ state,
+                     float* __restrict__ M, float* __restrict__ b, float* __restrict__ J, int n_envs) {
+  __shared__ __align__(16) float stage[TREX_DYN_WARPS][TREX_DYN_STAGE];
+  const int warp = threadIdx.x >> 5;
+  const int env = blockIdx.x * TREX_DYN_WARPS + warp;
+  if (env >= n_envs) return;
+  trex::dynamics_phase(P, mdl, mdli, com, envp ? envp + (size_t)env * TREX_ENVP_DIM : nullptr,
+                       state + (size_t)env * TREX_STATE_STRIDE, stage[warp], M ? M + (size_t)env * TREX_DYN_MSIZE : nullptr,
+                       b ? b + (size_t)env * TREX_DYN_NDOF : nullptr, J ? J + (size_t)env * TREX_DYN_JSIZE : nullptr);
+}
+
 // ------------------------------------------------------------------------------------------------
 // synthetic actions: Philox4x32-10, key (seed, 0x5eed), counter (env lo, env hi, step lo, step hi ^ block)
 // ------------------------------------------------------------------------------------------------
@@ -476,7 +495,8 @@ struct trex_handle {
   float *d_envp = nullptr, *d_envp_ranges = nullptr;
   double dt = 0.0;              // physics substep in double (the motor impulse bound = torque * dt)
   // external wrenches (trex_config.external_forces = 1): d_extf [n_envs][6][32] and the push schedule passed to every front
-  // kernel launch (push.on = 0: off); the COM table d_com [3][32] (every handle: trex_get_body_states reads it too)
+  // kernel launch (push.on = 0: off); the COM table d_com [3][32] (every handle: trex_get_body_states and
+  // trex_get_dynamics read it too)
   bool extf_on = false;
   float *d_extf = nullptr, *d_com = nullptr;
   trex::PushSchedule push = {};
@@ -1137,6 +1157,18 @@ int trex_get_body_states(trex_handle* h, float* states_dev, float* contact_force
   trex_body_states_kernel<<<(unsigned)((h->n_envs + TREX_BODY_WARPS - 1) / TREX_BODY_WARPS), 32 * TREX_BODY_WARPS, 0,
                             (cudaStream_t)stream>>>(h->P, h->d_mdl, h->d_mdli, h->d_cand_lane, h->d_com, h->d_state, states_dev,
                                                     contact_force_dev, h->n_envs);
+  CUDA_TRY(cudaGetLastError());
+  h->launches++;
+  return TREX_OK;
+}
+
+int trex_get_dynamics(trex_handle* h, float* mass_matrix_dev, float* bias_dev, float* jacobian_dev, void* stream) {
+  if (!h) return fail(TREX_ERR_INVALID, "handle is NULL%s");
+  if (!mass_matrix_dev && !bias_dev && !jacobian_dev) return fail(TREX_ERR_INVALID, "trex_get_dynamics: all outputs are NULL%s");
+  CUDA_TRY(cudaSetDevice(h->device));
+  trex_dynamics_kernel<<<(unsigned)((h->n_envs + TREX_DYN_WARPS - 1) / TREX_DYN_WARPS), 32 * TREX_DYN_WARPS, 0, (cudaStream_t)stream>>>(
+      h->P, h->d_mdl, h->d_mdli, h->d_com, h->envp_on ? h->d_envp : nullptr, h->d_state, mass_matrix_dev, bias_dev, jacobian_dev,
+      h->n_envs);
   CUDA_TRY(cudaGetLastError());
   h->launches++;
   return TREX_OK;

@@ -2870,4 +2870,238 @@ TREX_FN void body_states_phase(const Uniform& P, const float* mdl, const int* md
   }
 }
 
+// ------------------------------------------------------------------------------------------
+// Joint-space mass matrix, bias forces and body Jacobians of ONE environment (trex_get_dynamics), one warp.  Reads the
+// record, writes nothing to it.  Generalized velocity u (31): [0:3] base angular velocity (world, record [7:10]), [3:6]
+// velocity of the base frame's origin p0 (world, record [10:13]), [6:31] joint rates in lane order (record [38:63]); lane
+// L < 25 owns coordinate 6 + L, lanes 25..30 own coordinates 0..5.
+//   M [31][31]: kinetic energy = u^T M u / 2; full, each entry below the diagonal a copy of its mirror image
+//   b [31]: M du/dt + b = tau: gravity, Coriolis and centrifugal terms only (no damping, motors, limits, contacts, wrenches)
+//   J [NB][6][31]: J_k u = [velocity of body k's COM; its angular velocity], world frame
+// All vectors are in world axes, positions relative to p0 (the values stay small where the base is far from the world
+// origin).  M and b come from subtree sums (dyn_composite, dyn_force_sum) that each lane takes about its own joint's origin:
+// the entries of a light distal joint are then not the small difference of large moments about p0.  envp: this
+// environment's parameter row (nullptr: the model's masses; a scale multiplies mass and inertia first, as in the step; the
+// COM stays).  com: the [3][32] COM table.  stage: TREX_DYN_STAGE floats of the warp's shared memory.  Any output may be
+// nullptr and is then not computed.
+// ------------------------------------------------------------------------------------------
+#define TREX_DYN_NDOF 31
+#define TREX_DYN_JROWS 6
+#define TREX_DYN_MSIZE (TREX_DYN_NDOF * TREX_DYN_NDOF)
+#define TREX_DYN_JSIZE (trex_topo::NB * TREX_DYN_JROWS * TREX_DYN_NDOF)
+#define TREX_DYN_SUMS 10                                            // rows of 32 floats for the subtree sums
+#define TREX_DYN_STAGE (TREX_DYN_SUMS * 32 + TREX_DYN_MSIZE + 3)  // + M staged row-major; + 3: a multiple of 16 bytes
+
+// whether body j (lane j) lies in the subtree of the lane's body (the base's lane: every body)
+TREX_FN vb dyn_in_subtree(const int* mdli, vi lane, int j) {
+  return lane == 25 || (((vi(ldui(mdli, IF_ANC_MASK * 32 + j)) >> lane) & 1) != 0);
+}
+
+// Composite inertia of the lane's subtree about the point r (from p0): B = the lane's body's COM inertia (xx xy xz yy yz zz,
+// world axes) | COM (from p0) | mass; C = inertia about r | first moment about r | mass, summed in ascending lane order.
+TREX_FN void dyn_composite(const int* mdli, vi lane, float* rows, const vf B[10], const vf r[3], vf C[10]) {
+  TREX_UNROLL for (int k = 0; k < 10; k++) { st(rows, lane + 32 * k, B[k]); C[k] = 0.0f; }
+  warp_sync();
+  TREX_ROLLED for (int j = 0; j < NB; j++) {
+    const vb in = dyn_in_subtree(mdli, lane, j);
+    vf x[10];
+    TREX_UNROLL for (int k = 0; k < 10; k++) x[k] = ld(rows, vi(32 * k + j));
+    const vf d0 = x[6] - r[0], d1 = x[7] - r[1], d2 = x[8] - r[2], m = x[9];
+    const vf t[10] = {x[0] + m * (d1 * d1 + d2 * d2), x[1] - m * (d0 * d1), x[2] - m * (d0 * d2), x[3] + m * (d0 * d0 + d2 * d2),
+                      x[4] - m * (d1 * d2), x[5] + m * (d0 * d0 + d1 * d1), m * d0, m * d1, m * d2, m};
+    TREX_UNROLL for (int k = 0; k < 10; k++) C[k] = sel(in, C[k] + t[k], C[k]);
+  }
+  warp_sync();
+}
+
+// Force of the lane's subtree about the point r: B = the lane's body's [n (about its COM); f] | COM (from p0); F = sum of
+// [n + (c - r) x f; f] in ascending lane order.
+TREX_FN void dyn_force_sum(const int* mdli, vi lane, float* rows, const vf B[9], const vf r[3], vf F[6]) {
+  TREX_UNROLL for (int k = 0; k < 9; k++) st(rows, lane + 32 * k, B[k]);
+  TREX_UNROLL for (int k = 0; k < 6; k++) F[k] = 0.0f;
+  warp_sync();
+  TREX_ROLLED for (int j = 0; j < NB; j++) {
+    const vb in = dyn_in_subtree(mdli, lane, j);
+    vf x[9];
+    TREX_UNROLL for (int k = 0; k < 9; k++) x[k] = ld(rows, vi(32 * k + j));
+    const vf d0 = x[6] - r[0], d1 = x[7] - r[1], d2 = x[8] - r[2];
+    const vf t[6] = {x[0] + (d1 * x[5] - d2 * x[4]), x[1] + (d2 * x[3] - d0 * x[5]), x[2] + (d0 * x[4] - d1 * x[3]), x[3], x[4], x[5]};
+    TREX_UNROLL for (int k = 0; k < 6; k++) F[k] = sel(in, F[k] + t[k], F[k]);
+  }
+  warp_sync();
+}
+
+TREX_FN void dynamics_phase(const Uniform& P, const float* mdl, const int* mdli, const float* com, const float* envp,
+                            const float* rec, float* stage, float* Mout, float* bout, float* Jout) {
+  const vi lane = lane_id();
+  const vb is_joint = lane < NJ;
+  const vb owns = lane < TREX_DYN_NDOF;
+  const vi col = seli(is_joint, lane + 6, lane - 25);  // the coordinate of u this lane owns
+  EnvRegs R;
+  load_env_regs(rec, lane, R);
+  float Rb[9];
+  quat_to_Rb(R.quat, Rb);
+  vf E[9], Rw[9], xw[3], v[6];
+  local_rotation(mdl, lane, R.q, E);
+  forward_pass<false>(mdl, mdli, lane, R, Rb, E, Rw, xw, v);
+  // joint axis a (world: the body's z axis) through the body origin r (from p0; the base's lane: r = 0), and the body's COM
+  // cw (from p0): c of the COM table in world axes
+  vf r[3], a[3], c[3], cw[3];
+  TREX_UNROLL for (int k = 0; k < 3; k++) { r[k] = xw[k] - R.pos[k]; a[k] = Rw[6 + k]; c[k] = ldg_ro(com, lane + k * 32); }
+  TREX_UNROLL for (int i = 0; i < 3; i++) cw[i] = r[i] + (Rw[i] * c[0] + Rw[3 + i] * c[1] + Rw[6 + i] * c[2]);
+
+  // the body's mass and COM inertia in world axes, Ic = Rw^T (I - m (|c|^2 1 - c c^T)) Rw (I: about the body origin)
+  vf m, Ic[6];
+  if (Mout || bout) {
+    const vf msc = envp ? envp_mass_scale(envp, lane) : vf(1.0f);
+    m = MDL(F_MASS) * msc;
+    vf I6[6];
+    TREX_UNROLL for (int k = 0; k < 6; k++) I6[k] = MDL(F_I + k) * msc;
+    const vf cc = c[0] * c[0] + c[1] * c[1] + c[2] * c[2];
+    const vf Ib[3][3] = {{I6[0] - m * (cc - c[0] * c[0]), I6[1] + m * (c[0] * c[1]), I6[2] + m * (c[0] * c[2])},
+                         {I6[1] + m * (c[0] * c[1]), I6[3] - m * (cc - c[1] * c[1]), I6[4] + m * (c[1] * c[2])},
+                         {I6[2] + m * (c[0] * c[2]), I6[4] + m * (c[1] * c[2]), I6[5] - m * (cc - c[2] * c[2])}};
+    vf T[3][3];
+    TREX_UNROLL for (int i = 0; i < 3; i++)
+      TREX_UNROLL for (int j = 0; j < 3; j++) T[i][j] = Ib[i][0] * Rw[j] + Ib[i][1] * Rw[3 + j] + Ib[i][2] * Rw[6 + j];
+    int n = 0;
+    TREX_UNROLL for (int i = 0; i < 3; i++)
+      TREX_UNROLL for (int j = i; j < 3; j++) Ic[n++] = Rw[i] * T[0][j] + Rw[3 + i] * T[1][j] + Rw[6 + i] * T[2][j];
+  }
+
+  if (Mout) {  // composite-rigid-body algorithm
+    vf C[10];
+    {
+      const vf B[10] = {Ic[0], Ic[1], Ic[2], Ic[3], Ic[4], Ic[5], cw[0], cw[1], cw[2], m};
+      dyn_composite(mdli, lane, stage, B, r, C);
+    }
+    float* Ms = stage + TREX_DYN_SUMS * 32;
+    TREX_UNROLL for (int i = 0; i < (TREX_DYN_MSIZE + 31) / 32; i++) {
+      const vi idx = lane + 32 * i;
+      st_if(Ms, seli(idx < TREX_DYN_MSIZE, idx, 0), 0.0f, idx < TREX_DYN_MSIZE);
+    }
+    warp_sync();
+    // joint lanes: F = [I a; a x h], the force about the joint's origin that moves the subtree with a unit joint rate.
+    // Row 6 + lane of M: F about p0 in the base columns, S_j . F for j the joint or one of its ancestors, 0 elsewhere.
+    vf F[6];
+    F[0] = C[0] * a[0] + C[1] * a[1] + C[2] * a[2];
+    F[1] = C[1] * a[0] + C[3] * a[1] + C[4] * a[2];
+    F[2] = C[2] * a[0] + C[4] * a[1] + C[5] * a[2];
+    F[3] = a[1] * C[8] - a[2] * C[7];
+    F[4] = a[2] * C[6] - a[0] * C[8];
+    F[5] = a[0] * C[7] - a[1] * C[6];
+    const vf Fb[6] = {F[0] + (r[1] * F[5] - r[2] * F[4]), F[1] + (r[2] * F[3] - r[0] * F[5]), F[2] + (r[0] * F[4] - r[1] * F[3]),
+                      F[3], F[4], F[5]};
+    const vi row = seli(is_joint, lane + 6, 0);
+    TREX_UNROLL for (int q = 0; q < 6; q++) {
+      st_if(Ms, row * TREX_DYN_NDOF + q, Fb[q], is_joint);
+      st_if(Ms, q * TREX_DYN_NDOF + row, Fb[q], is_joint);
+    }
+    vi anc = lane;
+    TREX_ROLLED for (int d = 0; d < MAX_DEPTH; d++) {
+      // joint j = anc moves the point r with a x (r - r_j)
+      const vb ok = is_joint && anc < NJ;
+      vf sa[3], e3[3];
+      TREX_UNROLL for (int k = 0; k < 3; k++) { sa[k] = shflv(a[k], anc); e3[k] = r[k] - shflv(r[k], anc); }
+      const vf l0 = sa[1] * e3[2] - sa[2] * e3[1], l1 = sa[2] * e3[0] - sa[0] * e3[2], l2 = sa[0] * e3[1] - sa[1] * e3[0];
+      const vf e = sa[0] * F[0] + sa[1] * F[1] + sa[2] * F[2] + (l0 * F[3] + l1 * F[4] + l2 * F[5]);
+      const vi other = seli(ok, anc + 6, 0);
+      st_if(Ms, row * TREX_DYN_NDOF + other, e, ok);
+      st_if(Ms, other * TREX_DYN_NDOF + row, e, ok);
+      anc = ldi(mdli, anc + IF_PARENT_LANE * 32);
+    }
+    // the base block: the whole tree's inertia about p0 [[I, [h]x], [[h]x^T, m 1]] (lane 25)
+    const vb is_base = lane == 25;
+    const vf hx[3][3] = {{0.0f, -C[8], C[7]}, {C[8], 0.0f, -C[6]}, {-C[7], C[6], 0.0f}};
+    const int si[3][3] = {{0, 1, 2}, {1, 3, 4}, {2, 4, 5}};
+    TREX_UNROLL for (int i = 0; i < 3; i++) {
+      TREX_UNROLL for (int j = 0; j < 3; j++) {
+        st_if(Ms, vi(i * TREX_DYN_NDOF + j), C[si[i][j]], is_base);
+        st_if(Ms, vi(i * TREX_DYN_NDOF + 3 + j), hx[i][j], is_base);
+        st_if(Ms, vi((3 + j) * TREX_DYN_NDOF + i), hx[i][j], is_base);
+      }
+      st_if(Ms, vi((3 + i) * TREX_DYN_NDOF + 3 + i), C[9], is_base);
+    }
+    warp_sync();
+    TREX_UNROLL for (int i = 0; i < (TREX_DYN_MSIZE + 31) / 32; i++) {  // coalesced, in flat-index order
+      const vi idx = lane + 32 * i;
+      const vb in = idx < TREX_DYN_MSIZE;
+      st_if(Mout, idx, ld_if(Ms, seli(in, idx, 0), in, 0.0f), in);
+    }
+    warp_sync();
+  }
+
+  if (bout) {  // Newton-Euler with du/dt = 0
+    // Motion V = [w; v at p0] and spatial acceleration A (at p0) of every body, gravity entering as an upward acceleration
+    // of the base.  The base's A is [0; -w x v] when its classical acceleration du/dt is 0; a joint adds (V x S) qd, with
+    // S = [a; r x a] its motion at p0 (the axis moves with the body).
+    vf s[3];
+    s[0] = r[1] * a[2] - r[2] * a[1];
+    s[1] = r[2] * a[0] - r[0] * a[2];
+    s[2] = r[0] * a[1] - r[1] * a[0];
+    vf V[6], A[6];
+    TREX_UNROLL for (int k = 0; k < 3; k++) { V[k] = vbroadcast(R.om[k]); V[3 + k] = vbroadcast(R.vl[k]); A[k] = 0.0f; }
+    A[3] = vbroadcast(-(R.om[1] * R.vl[2] - R.om[2] * R.vl[1]));
+    A[4] = vbroadcast(-(R.om[2] * R.vl[0] - R.om[0] * R.vl[2]));
+    A[5] = vbroadcast(P.g - (R.om[0] * R.vl[1] - R.om[1] * R.vl[0]));
+    const vi plane = MDLI(IF_PARENT_LANE);
+    const vi depth = MDLI(IF_DEPTH);
+    TREX_ROLLED for (int d = 1; d <= MAX_DEPTH; d++) {
+      const vb at = depth == d;
+      vf pV[6], pA[6];
+      TREX_UNROLL for (int k = 0; k < 6; k++) { pV[k] = shflv(V[k], plane); pA[k] = shflv(A[k], plane); }
+      vf cr[6];  // (pV x S) qd
+      cr[0] = (pV[1] * a[2] - pV[2] * a[1]) * R.qd;
+      cr[1] = (pV[2] * a[0] - pV[0] * a[2]) * R.qd;
+      cr[2] = (pV[0] * a[1] - pV[1] * a[0]) * R.qd;
+      cr[3] = ((pV[1] * s[2] - pV[2] * s[1]) + (pV[4] * a[2] - pV[5] * a[1])) * R.qd;
+      cr[4] = ((pV[2] * s[0] - pV[0] * s[2]) + (pV[5] * a[0] - pV[3] * a[2])) * R.qd;
+      cr[5] = ((pV[0] * s[1] - pV[1] * s[0]) + (pV[3] * a[1] - pV[4] * a[0])) * R.qd;
+      TREX_UNROLL for (int k = 0; k < 3; k++) {
+        V[k] = sel(at, pV[k] + a[k] * R.qd, V[k]);
+        V[3 + k] = sel(at, pV[3 + k] + s[k] * R.qd, V[3 + k]);
+      }
+      TREX_UNROLL for (int k = 0; k < 6; k++) A[k] = sel(at, pA[k] + cr[k], A[k]);
+    }
+    // at the COM: v_c = v + w x c, classical acceleration a_c = A_lin + alpha x c + w x v_c; f = m a_c, n = Ic alpha + w x Ic w
+    const vf vc[3] = {V[3] + (V[1] * cw[2] - V[2] * cw[1]), V[4] + (V[2] * cw[0] - V[0] * cw[2]), V[5] + (V[0] * cw[1] - V[1] * cw[0])};
+    const vf ac[3] = {A[3] + (A[1] * cw[2] - A[2] * cw[1]) + (V[1] * vc[2] - V[2] * vc[1]),
+                      A[4] + (A[2] * cw[0] - A[0] * cw[2]) + (V[2] * vc[0] - V[0] * vc[2]),
+                      A[5] + (A[0] * cw[1] - A[1] * cw[0]) + (V[0] * vc[1] - V[1] * vc[0])};
+    const vf L[3] = {Ic[0] * V[0] + Ic[1] * V[1] + Ic[2] * V[2], Ic[1] * V[0] + Ic[3] * V[1] + Ic[4] * V[2],
+                     Ic[2] * V[0] + Ic[4] * V[1] + Ic[5] * V[2]};
+    const vf B[9] = {Ic[0] * A[0] + Ic[1] * A[1] + Ic[2] * A[2] + (V[1] * L[2] - V[2] * L[1]),
+                     Ic[1] * A[0] + Ic[3] * A[1] + Ic[4] * A[2] + (V[2] * L[0] - V[0] * L[2]),
+                     Ic[2] * A[0] + Ic[4] * A[1] + Ic[5] * A[2] + (V[0] * L[1] - V[1] * L[0]),
+                     m * ac[0], m * ac[1], m * ac[2], cw[0], cw[1], cw[2]};
+    vf F[6];
+    dyn_force_sum(mdli, lane, stage, B, r, F);
+    // joint lanes: a . n of their subtree about the joint's origin; base lanes 25..30: component lane - 25 of the whole
+    // tree's [n about p0; f] (lane 25)
+    vf out = a[0] * F[0] + a[1] * F[1] + a[2] * F[2];
+    TREX_UNROLL for (int k = 0; k < 6; k++) out = sel(lane == 25 + k, shfl(F[k], 25), out);
+    st_if(bout, col, out, owns);
+  }
+
+  if (Jout) {
+    // lane L < 25: column 6 + L, the joint's [a x (c_k - r); a] where it moves body k; lanes 25..27: the base angular
+    // coordinate e = unit L - 25, [e x c_k; e]; lanes 28..30: the base linear coordinate, [e; 0]
+    vf u[3];
+    const vb wcol = lane >= 25 && lane < 28, vcol = lane >= 28 && lane < 31;
+    TREX_UNROLL for (int k = 0; k < 3; k++) u[k] = sel((wcol && lane == 25 + k) || (vcol && lane == 28 + k), 1.0f, 0.0f);
+    TREX_ROLLED for (int k = 0; k < NB; k++) {
+      vf ck[3], d[3], jr[6];
+      TREX_UNROLL for (int i = 0; i < 3; i++) { ck[i] = shfl(cw[i], k); d[i] = ck[i] - r[i]; }
+      const vb in = is_joint && dyn_in_subtree(mdli, lane, k);
+      const vf bv[3] = {u[1] * ck[2] - u[2] * ck[1], u[2] * ck[0] - u[0] * ck[2], u[0] * ck[1] - u[1] * ck[0]};
+      jr[0] = sel(in, a[1] * d[2] - a[2] * d[1], sel(wcol, bv[0], u[0]));
+      jr[1] = sel(in, a[2] * d[0] - a[0] * d[2], sel(wcol, bv[1], u[1]));
+      jr[2] = sel(in, a[0] * d[1] - a[1] * d[0], sel(wcol, bv[2], u[2]));
+      TREX_UNROLL for (int i = 0; i < 3; i++) jr[3 + i] = sel(in, a[i], sel(wcol, u[i], 0.0f));
+      float* Jk = Jout + k * (TREX_DYN_JROWS * TREX_DYN_NDOF);
+      TREX_UNROLL for (int i = 0; i < 6; i++) st_if(Jk, col + i * TREX_DYN_NDOF, jr[i], owns);
+    }
+  }
+}
+
 }  // namespace trex

@@ -439,6 +439,51 @@ class TrexBatchSim:
         self._body_query(None, out)
         return out
 
+    # -- joint-space dynamics (every simulator) ---------------------------------------------------------------------------
+    # Coordinates u of dof_names(): base angular velocity and the velocity of the base link's COM (world frame, the record's
+    # [7:13]), then the 25 joint rates in pybullet link order (the record's [38:63]; NOT the name-sorted action order).
+
+    def dof_names(self) -> list[str]:
+        """The 31 coordinate names of ``mass_matrix`` / ``bias_forces`` / ``jacobians``: six base coordinates, then the joint
+        names in pybullet link order (``meta["body_joint_names"]``)."""
+        return ["base_wx", "base_wy", "base_wz", "base_vx", "base_vy", "base_vz"] + list(self.model.meta["body_joint_names"][1:])
+
+    def _dynamics_query(self, mass_matrix, bias, jacobian):
+        ptrs = [None if t is None else ctypes.c_void_p(t.data_ptr()) for t in (mass_matrix, bias, jacobian)]
+        _native.check(self._L.trex_get_dynamics(self._h, *ptrs, self._stream()), "trex_get_dynamics")
+
+    def mass_matrix(self, out: torch.Tensor | None = None) -> torch.Tensor:
+        """[N, 31, 31] joint-space mass matrix M of the current records (include/trex_b200.h, trex_get_dynamics): kinetic
+        energy = u^T M u / 2 in the coordinates of ``dof_names()``, with the environments' mass scales; exactly symmetric."""
+        shape = (self.num_envs, _native.NUM_DOFS, _native.NUM_DOFS)
+        if out is None:
+            out = torch.empty(shape, device=self.device, dtype=torch.float32)
+        self._check_tensor(out, shape, torch.float32, "out")
+        self._dynamics_query(out, None, None)
+        return out
+
+    def bias_forces(self, out: torch.Tensor | None = None) -> torch.Tensor:
+        """[N, 31] b with M du/dt + b = tau: gravity, Coriolis and centrifugal terms (pybullet's calculateInverseDynamics with
+        zero accelerations).  Damping, motors, joint limits, contacts and external wrenches are not included.  Torques of
+        given accelerations: ``(sim.mass_matrix() @ udot[..., None])[..., 0] + sim.bias_forces()``."""
+        shape = (self.num_envs, _native.NUM_DOFS)
+        if out is None:
+            out = torch.empty(shape, device=self.device, dtype=torch.float32)
+        self._check_tensor(out, shape, torch.float32, "out")
+        self._dynamics_query(None, out, None)
+        return out
+
+    def jacobians(self, out: torch.Tensor | None = None) -> torch.Tensor:
+        """[N, 26, 6, 31] Jacobian of every body in ``body_names()`` order: rows [COM velocity; angular velocity] in the world
+        frame, so that ``J[:, k] @ u`` is ``body_states()[:, k, 7:13]`` and ``J[:, k].transpose(-1, -2) @ [f; t]`` is the
+        generalized force of a wrench on body k."""
+        shape = (self.num_envs, _native.EXT_BODIES, _native.JACOBIAN_ROWS, _native.NUM_DOFS)
+        if out is None:
+            out = torch.empty(shape, device=self.device, dtype=torch.float32)
+        self._check_tensor(out, shape, torch.float32, "out")
+        self._dynamics_query(None, None, out)
+        return out
+
     def random_actions(self, step: int, seed: int = 0, env_offset: int = 0, out: torch.Tensor | None = None) -> torch.Tensor:
         """U(low, high) actions from Philox keyed by (seed, env_offset + env, step)."""
         if out is None:
