@@ -67,6 +67,8 @@ typedef struct trex_handle trex_handle;
 #define TREX_HEAVY_TENSOR 2
 #define TREX_CONTACT_TENSOR 0
 #define TREX_CONTACT_SHARED 1
+#define TREX_ACTUATION_POSITION 0
+#define TREX_ACTUATION_TORQUE 1
 
 typedef struct trex_config {
   int32_t num_substeps;      /* trex_env.py:18 NUM_SUBSTEPS (5); dt = 0.01/n, iterations = int(300/n)  (:71-73) */
@@ -118,7 +120,24 @@ typedef struct trex_config {
                                 external wrenches on the bodies (trex_set_external_forces below) and an optional push schedule, and
                                 runs the dynamics-kernel instances that read them; the record starts at zero, which reproduces the
                                 external_forces = 0 results bit for bit */
-  int32_t reserved[5];       /* must be zero */
+  int32_t actuation;         /* what an action is (any other value: TREX_ERR_INVALID):
+                                TREX_ACTUATION_POSITION (0, default): a motor target, clipped to the joint limits (the reference's
+                                  trex_robot.set_actions; the motors bound the impulse by max_torque * dt).
+                                TREX_ACTUATION_TORQUE (1): joint torque control (pybullet's setJointMotorControlArray(TORQUE_CONTROL,
+                                  forces=tau) after VELOCITY_CONTROL with forces 0; Isaac Gym's DOF actuation-force tensor).
+                                  Action slot i (name-sorted) is the torque in N m on joint obs_dof[i], clipped to [-T, T] with T the
+                                  model's motor_max_torque (env_params = 1: the environment's row element [29]; elements [27] and
+                                  [28] are then ignored and the library keeps [30] at 0).  A NaN command is clipped to -T
+                                  (as a NaN target becomes the lower joint limit in position mode): pass finite torques.  It acts in EVERY physics substep of the
+                                  step, as an explicit joint torque next to pybullet's joint damping: Q = tau - d qd.  The motor
+                                  rows stay with kp = kd = 0 and impulse bound 0 (as in a reset step); joint limits, contacts,
+                                  damping, wrenches and pushes are unchanged.  Reset steps (trex_reset, the auto-reset) apply no
+                                  torque, as in position mode.  The applied joint torque that record [63:88], observation [50:75]
+                                  and the reward's energy term sum |qd tau| report is the CLIPPED COMMAND -- a deliberate
+                                  difference from pybullet, whose getJointState reports the motor's impulse / dt, i.e. 0 in torque
+                                  control (as far as we know), which would silently drop the reference's energy penalty.
+                                  trex_get_action_limits gives the bounds; trex_fill_random_actions draws U(-T, T). */
+  int32_t reserved[4];       /* must be zero */
 } trex_config;
 
 typedef struct trex_stats {
@@ -177,6 +196,8 @@ int trex_set_state(trex_handle* h, const float* state_dev, void* stream);
  *   [27]    motor position gain kp, [28] velocity gain kd                                      setJointMotorControlArray(positionGains=, velocityGains=)
  *   [29]    motor max torque, N m                                                              setJointMotorControlArray(forces=)
  *   [30]    motor impulse bound = [29] * dt, computed in double by the library (the value passed is ignored)
+ *   With TREX_ACTUATION_TORQUE: [27] and [28] are ignored, [29] is the bound the torque command is clipped to, and the library
+ *   keeps [30] at 0 (the motors have no strength) on create, on a set and on every randomized reset.
  *   [31]    reserved, 0
  * Defaults (every row after trex_create): scales 1, then the model's friction, motor_kp, motor_kd, motor_max_torque.  Reset
  * steps keep zero motor gains, as with env_params = 0; mass scales and friction apply to them.
@@ -268,7 +289,8 @@ int trex_get_body_states(trex_handle* h, float* states_dev, float* contact_force
  *     is computed and mirrored)
  *   bias_dev [N][31] float32: b with M du/dt + b = tau, du/dt the time derivative of u in the coordinates above: gravity plus
  *     the Coriolis and centrifugal terms.  b does NOT contain link or joint damping, motors, joint limits, contacts or the
- *     external-wrench record.  The generalized force tau of u[0:6] is the torque about the base link's COM, then the force
+ *     external-wrench record.  In particular a torque-mode step (TREX_ACTUATION_TORQUE) adds the joint damping -d qd to the
+ *     commanded torque, which b leaves out: a computed-torque controller adds d qd itself.  The generalized force tau of u[0:6] is the torque about the base link's COM, then the force
  *     (world).  Joint torques of given accelerations: tau = M du/dt + b, in torch (M @ udot[..., None])[..., 0] + b
  *   jacobian_dev [N][26][TREX_JACOBIAN_ROWS][31] float32: J_k of body k (numbered as in the wrench record and
  *     trex_get_body_states: body k < 25 is the body moved by joint k, body 25 the base), rows [v_COM (3); w (3)] in the world
@@ -283,10 +305,15 @@ int trex_get_dynamics(trex_handle* h, float* mass_matrix_dev, float* bias_dev, f
  * logged at trex_env.py:193-195 (lifting, station keeping, energy), PGS iterations, contacts. */
 int trex_get_aux(trex_handle* h, float* aux_dev, void* stream);
 
-/* action/observation limits in name-sorted joint order (trex_robot.py:337-357, 424-433); host pointers */
+/* action/observation limits in name-sorted joint order (trex_robot.py:337-357, 424-433); host pointers.  The observation
+ * space uses them in either actuation mode. */
 int trex_get_joint_limits(trex_handle* h, float* lower25_host, float* upper25_host);
+/* the action space in name-sorted joint order: the joint limits with TREX_ACTUATION_POSITION, -T / +T with
+ * TREX_ACTUATION_TORQUE (T = the model's motor_max_torque; per-environment bounds of env_params rows are not reflected);
+ * host pointers */
+int trex_get_action_limits(trex_handle* h, float* lo25_host, float* hi25_host);
 
-/* Synthetic benchmark input: action[i][k] ~ U(lower_k, upper_k) from a counter-based generator keyed by
+/* Synthetic benchmark input: action[i][k] ~ U(lo_k, hi_k) of trex_get_action_limits, from a counter-based generator keyed by
  * (seed, env_offset + i, step), so streams do not depend on the number of GPUs. */
 int trex_fill_random_actions(trex_handle* h, float* action_dev, uint32_t seed, uint64_t step, int64_t env_offset,
                              void* stream);

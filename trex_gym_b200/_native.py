@@ -26,7 +26,7 @@ JACOBIAN_ROWS = 6  # rows of a body Jacobian: v_COM | w
 EXPORTED_SYMBOLS = (
     "trex_create", "trex_destroy", "trex_reset", "trex_step", "trex_step_host", "trex_step_host_async", "trex_host_wait",
     "trex_reset_host",
-    "trex_get_state", "trex_set_state", "trex_get_aux", "trex_get_joint_limits",
+    "trex_get_state", "trex_set_state", "trex_get_aux", "trex_get_joint_limits", "trex_get_action_limits",
     "trex_set_env_params", "trex_get_env_params", "trex_set_env_param_ranges",
     "trex_set_external_forces", "trex_get_external_forces", "trex_set_push_schedule",
     "trex_get_body_states", "trex_get_dynamics",
@@ -56,7 +56,8 @@ class TrexConfig(ctypes.Structure):
         ("contact_memory", ctypes.c_int32),
         ("env_params", ctypes.c_int32),
         ("external_forces", ctypes.c_int32),
-        ("reserved", ctypes.c_int32 * 5),
+        ("actuation", ctypes.c_int32),
+        ("reserved", ctypes.c_int32 * 4),
     ]
 
 
@@ -76,6 +77,7 @@ class TrexPushSchedule(ctypes.Structure):
 SOLVE_DEFAULT, SOLVE_FRONT, SOLVE_FREE_ONLY, SOLVE_NO_HEAVY = 0, 1, 2, 3  # trex_config.solver_placement
 HEAVY_BOTH, HEAVY_SHARED, HEAVY_TENSOR = 0, 1, 2  # trex_config.heavy_memory
 CONTACT_TENSOR, CONTACT_SHARED = 0, 1  # trex_config.contact_memory
+ACTUATION = {"position": 0, "torque": 1}  # trex_config.actuation: TREX_ACTUATION_POSITION / TREX_ACTUATION_TORQUE
 
 
 class TrexStats(ctypes.Structure):
@@ -162,6 +164,8 @@ def lib():
     L.trex_set_push_schedule.argtypes = [vp, ctypes.POINTER(TrexPushSchedule)]
     L.trex_get_joint_limits.restype = ctypes.c_int
     L.trex_get_joint_limits.argtypes = [vp, fp, fp]
+    L.trex_get_action_limits.restype = ctypes.c_int
+    L.trex_get_action_limits.argtypes = [vp, fp, fp]
     L.trex_fill_random_actions.restype = ctypes.c_int
     L.trex_fill_random_actions.argtypes = [vp, fp, ctypes.c_uint32, ctypes.c_uint64, ctypes.c_int64, vp]
     L.trex_get_stats.restype = ctypes.c_int

@@ -69,14 +69,16 @@ int fail(int code, const char* fmt, const char* detail = "") {
 // (indexed like state); without it envp is unused and the instance is the one the library had before the record existed.
 // EXTF (trex_config.external_forces): every environment's wrench record (extf, [6][32] per environment, indexed like state),
 // the COM table com [3][32] and the push schedule enter the bias forces; without it the three are unused.
-template <int WARPS, bool PACKED, bool ENVP, bool EXTF>
+// TAU (trex_config.actuation = TREX_ACTUATION_TORQUE): the actions are joint torques, clipped to +-tau_max (ENVP: the row's
+// bound) and applied as explicit joint torques; the motors have no gain and no strength.  Without it tau_max is unused.
+template <int WARPS, bool PACKED, bool ENVP, bool EXTF, bool TAU>
 __global__ void __launch_bounds__(32 * WARPS, TREX_MIN_BLOCKS / WARPS)
 trex_front_kernel(const trex::Uniform P, const float* __restrict__ mdl, const int* __restrict__ mdli,
                   const float* __restrict__ tasks, const float* __restrict__ cand_p, const int* __restrict__ cand_lane,
                   float* __restrict__ state, float* __restrict__ work, float* __restrict__ workh, const float* __restrict__ action,
                   int* __restrict__ list, int* __restrict__ list_count, const int* __restrict__ heavy_hint, int heavy_div, int n_envs,
                   int first_round, const float* __restrict__ envp, const float* __restrict__ extf, const float* __restrict__ com,
-                  const __grid_constant__ trex::PushSchedule push) {
+                  const __grid_constant__ trex::PushSchedule push, float tau_max) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   trex::WarpShared* slabs = reinterpret_cast<trex::WarpShared*>(smem_raw);
   const int warp = threadIdx.x >> 5;
@@ -96,13 +98,13 @@ trex_front_kernel(const trex::Uniform P, const float* __restrict__ mdl, const in
 #ifdef TREX_PHASES
   const long long t_entry = clock64();
 #endif
-  const int front_result = trex::front_phase<PACKED, ENVP, EXTF>(P, mdl, mdli, tasks, cand_p, cand_lane, slabs[warp], state + (size_t)env * TREX_STATE_STRIDE,
+  const int front_result = trex::front_phase<PACKED, ENVP, EXTF, TAU>(P, mdl, mdli, tasks, cand_p, cand_lane, slabs[warp], state + (size_t)env * TREX_STATE_STRIDE,
                                                   work ? work + (size_t)env * TREX_WORK_STRIDE : nullptr, action + (size_t)env * trex::NJ,
                                                   first_round != 0, slabs, warp, valid_mask,
                                                   // class 5 (more than TREX_KC contacts) always goes to its own solver unless heavy_share_div asks for the batch-dependent rule
                                                   (workh != nullptr && (heavy_div <= 0 || (long long)(*heavy_hint) * heavy_div <= (long long)n_envs)) ? workh + (size_t)env * TREX_HEAVY_STRIDE : nullptr,
                                                   ENVP ? envp + (size_t)env * TREX_ENVP_DIM : nullptr,
-                                                  EXTF ? extf + (size_t)env * TREX_EXTF_DIM : nullptr, com, &push, (long long)env);
+                                                  EXTF ? extf + (size_t)env * TREX_EXTF_DIM : nullptr, com, &push, (long long)env, tau_max);
   const int deferred = front_result & 255, n_contacts = front_result >> 8;
   // append to the list of its class of deferred environments (any order: the solver's lane groups are independent):
   // class 0 = contact-free substeps, classes 1..4 = 1 / 2 / 3-4 / 5-8 contacts, 5 = more; list c at list + c * n_envs, counters + 64 * c
@@ -229,23 +231,25 @@ trex_heavy_kernel(const trex::Uniform P, float* __restrict__ state, const float*
 // one warp per environment: reward / done / auto-reset / observations (mode 0), or reset only (mode 1, optional mask)
 // ENVP: mass scales and friction of each environment's row apply to its reset step; ranges != nullptr: every reset first draws
 // the environment's row (the randomizer; dt = physics substep in double, for the impulse bound)
-template <int WARPS, bool ENVP>
+// TAU: the applied joint torque the step reports is the clipped action (action, tau_max); without it both are unused.
+template <int WARPS, bool ENVP, bool TAU>
 __global__ void __launch_bounds__(32 * WARPS, TREX_MIN_BLOCKS / WARPS)
 trex_tail_kernel(const trex::Uniform P, const float* __restrict__ mdl, const int* __restrict__ mdli,
                  const float* __restrict__ tasks, const float* __restrict__ cand_p, const int* __restrict__ cand_lane,
                  float* __restrict__ state, float* __restrict__ obs, float* __restrict__ reward, uint8_t* __restrict__ done,
                  float* __restrict__ aux, const uint8_t* __restrict__ mask, int n_envs, int mode, float* envp,
-                 const float* __restrict__ ranges, double dt) {
+                 const float* __restrict__ ranges, double dt, const float* __restrict__ action, float tau_max) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   trex::WarpShared* slabs = reinterpret_cast<trex::WarpShared*>(smem_raw);
   const int warp = threadIdx.x >> 5;
   const int env = blockIdx.x * WARPS + warp;
   if (env >= n_envs) return;
   if (mode == 1 && mask != nullptr && mask[env] == 0) return;
-  trex::tail_phase<ENVP>(P, mdl, mdli, tasks, cand_p, cand_lane, slabs[warp], state + (size_t)env * TREX_STATE_STRIDE,
+  trex::tail_phase<ENVP, TAU>(P, mdl, mdli, tasks, cand_p, cand_lane, slabs[warp], state + (size_t)env * TREX_STATE_STRIDE,
                    obs ? obs + (size_t)env * (3 * trex::NJ) : nullptr, (mode == 0 && reward) ? reward + env : nullptr,
                    (mode == 0 && done) ? done + env : nullptr, (mode == 0 && aux) ? aux + (size_t)env * TREX_AUX_STRIDE : nullptr,
-                   mode == 1, (long long)env, ENVP ? envp + (size_t)env * TREX_ENVP_DIM : nullptr, ranges, dt);
+                   mode == 1, (long long)env, ENVP ? envp + (size_t)env * TREX_ENVP_DIM : nullptr, ranges, dt,
+                   TAU && mode == 0 ? action + (size_t)env * trex::NJ : nullptr, tau_max);
 }
 
 // trex_set_env_params: rows (all, or those with mask != 0) from the caller's buffer, the impulse bound recomputed in double
@@ -500,6 +504,15 @@ struct trex_handle {
   bool extf_on = false;
   float *d_extf = nullptr, *d_com = nullptr;
   trex::PushSchedule push = {};
+  // joint torque control (trex_config.actuation = TREX_ACTUATION_TORQUE): the model's torque bound (the action limits +-tau_max,
+  // passed to the TAU kernel instances) and the action limits of trex_fill_random_actions (d_act_lo / d_act_hi, 25 floats each:
+  // the joint limits in position mode, +-tau_max in torque mode)
+  bool tau_on = false;
+  float tau_max = 0.0f;
+  float *d_act_lo = nullptr, *d_act_hi = nullptr;
+  // the impulse bound an env-param row derives from its torque: dt in position mode, 0 in torque mode (the motors have no
+  // strength there, so the shared solver instances read a zero bound from the row)
+  double imp_dt() const { return tau_on ? 0.0 : dt; }
 };
 
 namespace {
@@ -525,7 +538,7 @@ struct HostIO {
   uint8_t* done;
 };
 
-template <int WF, int WS, bool ENVP, bool EXTF>
+template <int WF, int WS, bool ENVP, bool EXTF, bool TAU>
 int launch_step(trex_handle* h, const float* action, float* obs, float* reward, uint8_t* done, const uint8_t* mask,
                 int mode, cudaStream_t st, const HostIO* io = nullptr) {
   static const size_t extra_c = getenv("TREX_SOLVEC_EXTRA_SMEM") ? (size_t)atoi(getenv("TREX_SOLVEC_EXTRA_SMEM")) : 0;  // measurement aid: fewer resident warps
@@ -539,13 +552,13 @@ int launch_step(trex_handle* h, const float* action, float* obs, float* reward, 
   std::lock_guard<std::mutex> guard(configure_lock);
   if (!configured[h->device & 15]) {
     int rc;
-    if ((rc = configure_kernel(trex_front_kernel<WF, WF == 4, ENVP, EXTF>, smem_f)) != TREX_OK) return rc;
+    if ((rc = configure_kernel(trex_front_kernel<WF, WF == 4, ENVP, EXTF, TAU>, smem_f)) != TREX_OK) return rc;
     if ((rc = configure_kernel(trex_solve_kernel<WS, 0, 0, 0, ENVP>, smem_s)) != TREX_OK) return rc;
     if ((rc = configure_kernel(trex_solve_kernel<WS, TREX_KC, 1, TREX_CLASS_HEAVY - 1, ENVP>, smem_c)) != TREX_OK) return rc;
     if ((rc = configure_kernel(trex_solve_tm_kernel<1, TREX_CLASS_HEAVY - 1, ENVP>, smem_ct)) != TREX_OK) return rc;
     if ((rc = configure_kernel(trex_heavy_kernel<1, false, ENVP>, smem_h)) != TREX_OK) return rc;
     if ((rc = configure_kernel(trex_heavy_kernel<4, true, ENVP>, smem_ht)) != TREX_OK) return rc;
-    if ((rc = configure_kernel(trex_tail_kernel<WF, ENVP>, smem_f)) != TREX_OK) return rc;
+    if ((rc = configure_kernel(trex_tail_kernel<WF, ENVP, TAU>, smem_f)) != TREX_OK) return rc;
     configured[h->device & 15] = true;
   }
   if (h->n_pipes > 1) CUDA_TRY(cudaEventRecord(h->ev_start, st));
@@ -583,10 +596,10 @@ int launch_step(trex_handle* h, const float* action, float* obs, float* reward, 
     float* envp = ENVP ? h->d_envp + e0 * TREX_ENVP_DIM : nullptr;  // rows indexed like state
     const float* extf = EXTF ? h->d_extf + e0 * TREX_EXTF_DIM : nullptr;  // wrench records indexed like state
     for (int r = 0; r < n_rounds; r++) {
-      trex_front_kernel<WF, WF == 4, ENVP, EXTF><<<grid1, 32 * WF, smem_f, s>>>(Pc, h->d_mdl, h->d_mdli, h->d_tasks, h->d_cand_p, h->d_cand_lane,
+      trex_front_kernel<WF, WF == 4, ENVP, EXTF, TAU><<<grid1, 32 * WF, smem_f, s>>>(Pc, h->d_mdl, h->d_mdli, h->d_tasks, h->d_cand_p, h->d_cand_lane,
                                                           state, work, workh, action + e0 * trex::NJ, q.d_list, q.d_list_count + r,
                                                           q.d_list_count + 64 * (TREX_NCLASS + 2), h->heavy_div, count, r == 0, envp,
-                                                          extf, h->d_com, h->push);
+                                                          extf, h->d_com, h->push, h->tau_max);
       CUDA_TRY(cudaGetLastError());
       h->launches++;
       if (stagger && c == 0 && r == 0) CUDA_TRY(cudaEventRecord(h->ev_stagger, s));
@@ -647,11 +660,12 @@ int launch_step(trex_handle* h, const float* action, float* obs, float* reward, 
       }
       if (heavy) CUDA_TRY(cudaStreamWaitEvent(s, q.ev_join, 0));
     }
-    trex_tail_kernel<WF, ENVP><<<grid1, 32 * WF, smem_f, s>>>(Pc, h->d_mdl, h->d_mdli, h->d_tasks, h->d_cand_p, h->d_cand_lane,
+    trex_tail_kernel<WF, ENVP, TAU><<<grid1, 32 * WF, smem_f, s>>>(Pc, h->d_mdl, h->d_mdli, h->d_tasks, h->d_cand_p, h->d_cand_lane,
                                                         h->d_state + e0 * TREX_STATE_STRIDE, obs ? obs + e0 * 3 * trex::NJ : nullptr,
                                                         reward ? reward + e0 : nullptr, done ? done + e0 : nullptr,
                                                         h->d_aux + e0 * TREX_AUX_STRIDE, mask ? mask + e0 : nullptr, count, mode, envp,
-                                                        ENVP && h->ranges_on ? h->d_envp_ranges : nullptr, h->dt);
+                                                        ENVP && h->ranges_on ? h->d_envp_ranges : nullptr, h->imp_dt(),
+                                                        action ? action + e0 * trex::NJ : nullptr, h->tau_max);
     CUDA_TRY(cudaGetLastError());
     h->launches++;
     if (io) {
@@ -667,23 +681,31 @@ int launch_step(trex_handle* h, const float* action, float* obs, float* reward, 
   return TREX_OK;
 }
 
-int dispatch_step(trex_handle* h, const float* action, float* obs, float* reward, uint8_t* done, const uint8_t* mask,
-                  int mode, cudaStream_t st, const HostIO* io = nullptr) {
+// warps per CTA (1, 2, 4) x ENVP x EXTF x TAU: 24 instances of the step
+template <bool TAU>
+int dispatch_actuation(trex_handle* h, const float* action, float* obs, float* reward, uint8_t* done, const uint8_t* mask,
+                       int mode, cudaStream_t st, const HostIO* io) {
   switch (h->warps_per_block * 4 + (h->envp_on ? 1 : 0) + (h->extf_on ? 2 : 0)) {
-    case 4: return launch_step<1, 2, false, false>(h, action, obs, reward, done, mask, mode, st, io);
-    case 8: return launch_step<2, 1, false, false>(h, action, obs, reward, done, mask, mode, st, io);
-    case 16: return launch_step<4, 4, false, false>(h, action, obs, reward, done, mask, mode, st, io);
-    case 5: return launch_step<1, 2, true, false>(h, action, obs, reward, done, mask, mode, st, io);
-    case 9: return launch_step<2, 1, true, false>(h, action, obs, reward, done, mask, mode, st, io);
-    case 17: return launch_step<4, 4, true, false>(h, action, obs, reward, done, mask, mode, st, io);
-    case 6: return launch_step<1, 2, false, true>(h, action, obs, reward, done, mask, mode, st, io);
-    case 10: return launch_step<2, 1, false, true>(h, action, obs, reward, done, mask, mode, st, io);
-    case 18: return launch_step<4, 4, false, true>(h, action, obs, reward, done, mask, mode, st, io);
-    case 7: return launch_step<1, 2, true, true>(h, action, obs, reward, done, mask, mode, st, io);
-    case 11: return launch_step<2, 1, true, true>(h, action, obs, reward, done, mask, mode, st, io);
-    case 19: return launch_step<4, 4, true, true>(h, action, obs, reward, done, mask, mode, st, io);
+    case 4: return launch_step<1, 2, false, false, TAU>(h, action, obs, reward, done, mask, mode, st, io);
+    case 8: return launch_step<2, 1, false, false, TAU>(h, action, obs, reward, done, mask, mode, st, io);
+    case 16: return launch_step<4, 4, false, false, TAU>(h, action, obs, reward, done, mask, mode, st, io);
+    case 5: return launch_step<1, 2, true, false, TAU>(h, action, obs, reward, done, mask, mode, st, io);
+    case 9: return launch_step<2, 1, true, false, TAU>(h, action, obs, reward, done, mask, mode, st, io);
+    case 17: return launch_step<4, 4, true, false, TAU>(h, action, obs, reward, done, mask, mode, st, io);
+    case 6: return launch_step<1, 2, false, true, TAU>(h, action, obs, reward, done, mask, mode, st, io);
+    case 10: return launch_step<2, 1, false, true, TAU>(h, action, obs, reward, done, mask, mode, st, io);
+    case 18: return launch_step<4, 4, false, true, TAU>(h, action, obs, reward, done, mask, mode, st, io);
+    case 7: return launch_step<1, 2, true, true, TAU>(h, action, obs, reward, done, mask, mode, st, io);
+    case 11: return launch_step<2, 1, true, true, TAU>(h, action, obs, reward, done, mask, mode, st, io);
+    case 19: return launch_step<4, 4, true, true, TAU>(h, action, obs, reward, done, mask, mode, st, io);
     default: return fail(TREX_ERR_INVALID, "warps_per_block must be 1, 2 or 4%s");
   }
+}
+
+int dispatch_step(trex_handle* h, const float* action, float* obs, float* reward, uint8_t* done, const uint8_t* mask,
+                  int mode, cudaStream_t st, const HostIO* io = nullptr) {
+  return h->tau_on ? dispatch_actuation<true>(h, action, obs, reward, done, mask, mode, st, io)
+                   : dispatch_actuation<false>(h, action, obs, reward, done, mask, mode, st, io);
 }
 
 template <class Tp>
@@ -772,7 +794,12 @@ int trex_create(const void* model_blob, size_t bytes, int32_t n_envs, int32_t de
       return fail(TREX_ERR_INVALID, "trex_config.external_forces must be 0 or 1%s");
     }
     h->extf_on = cfg->external_forces == 1;
-    for (int i = 0; i < 5; i++)
+    if (cfg->actuation != TREX_ACTUATION_POSITION && cfg->actuation != TREX_ACTUATION_TORQUE) {
+      delete h;
+      return fail(TREX_ERR_INVALID, "trex_config.actuation must be TREX_ACTUATION_POSITION or TREX_ACTUATION_TORQUE%s");
+    }
+    h->tau_on = cfg->actuation == TREX_ACTUATION_TORQUE;
+    for (int i = 0; i < 4; i++)
       if (cfg->reserved[i] != 0) {
         delete h;
         return fail(TREX_ERR_INVALID, "trex_config.reserved must be zero%s");
@@ -798,6 +825,10 @@ int trex_create(const void* model_blob, size_t bytes, int32_t n_envs, int32_t de
   }
   trex_host::fill_uniform(h->T, h->C, h->P);
   h->dt = trex_host::substep_dt(h->T, h->C.num_substeps);
+  h->tau_max = (float)h->T.params[trex_host::P_MAX_TORQUE];
+  if (h->tau_on) {  // the motors of every kernel that reads the uniform settings: no gain, no strength
+    h->P.kp = 0.0f; h->P.kd = 0.0f; h->P.max_impulse = 0.0f;
+  }
   {
     // trex_heavy_kernel strides over its list with a fixed grid: exactly the CTAs that are resident at once (a larger
     // grid would run its surplus CTAs as a second wave after the first has walked the whole list)
@@ -830,6 +861,9 @@ int trex_create(const void* model_blob, size_t bytes, int32_t n_envs, int32_t de
   {
     std::vector<float> lo(h->T.lower_sorted, h->T.lower_sorted + trex::NJ), hi(h->T.upper_sorted, h->T.upper_sorted + trex::NJ);
     TRY(upload(&h->d_lower, lo)); TRY(upload(&h->d_upper, hi));
+    float alo[trex::NJ], ahi[trex::NJ];
+    trex_get_action_limits(h, alo, ahi);
+    TRY(upload(&h->d_act_lo, std::vector<float>(alo, alo + trex::NJ))); TRY(upload(&h->d_act_hi, std::vector<float>(ahi, ahi + trex::NJ)));
   }
 #undef TRY
 #define CTRY(expr) { cudaError_t _e = (expr); if (_e != cudaSuccess) { int r_ = fail(TREX_ERR_CUDA, #expr ": %s", cudaGetErrorString(_e)); trex_destroy(h); return r_; } }
@@ -876,6 +910,7 @@ int trex_create(const void* model_blob, size_t bytes, int32_t n_envs, int32_t de
   if (h->envp_on) {  // every row starts as the model's own constants
     float row[TREX_ENVP_DIM];
     trex_host::default_env_params(h->T, h->C.num_substeps, row);
+    if (h->tau_on) row[trex_host::ENVP_MAX_IMPULSE] = 0.0f;
     std::vector<float> rows(N * TREX_ENVP_DIM);
     for (size_t i = 0; i < rows.size(); i++) rows[i] = row[i % TREX_ENVP_DIM];
     CTRY(cudaMalloc((void**)&h->d_envp, rows.size() * sizeof(float)));
@@ -909,6 +944,7 @@ void trex_destroy(trex_handle* h) {
   cudaFree(h->d_lower); cudaFree(h->d_upper); cudaFree(h->d_state); cudaFree(h->d_aux); cudaFree(h->d_stats);
   cudaFree(h->d_envp); cudaFree(h->d_envp_ranges);
   cudaFree(h->d_extf); cudaFree(h->d_com);
+  cudaFree(h->d_act_lo); cudaFree(h->d_act_hi);
   for (int b = 0; b < 2; b++) {
     cudaFree(h->d_action[b]); cudaFree(h->d_obs[b]); cudaFree(h->d_reward[b]); cudaFree(h->d_done[b]);
     if (h->ev_step_done[b]) cudaEventDestroy(h->ev_step_done[b]);
@@ -1069,7 +1105,7 @@ int trex_set_env_params(trex_handle* h, const float* params_dev, const uint8_t* 
   if (!h->envp_on) return fail(TREX_ERR_INVALID, "trex_set_env_params: the handle was created with env_params = 0%s");
   CUDA_TRY(cudaSetDevice(h->device));
   const int total = h->n_envs * TREX_ENVP_DIM;
-  trex_set_env_params_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(h->d_envp, params_dev, mask_dev, h->dt, h->n_envs);
+  trex_set_env_params_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(h->d_envp, params_dev, mask_dev, h->imp_dt(), h->n_envs);
   CUDA_TRY(cudaGetLastError());
   h->launches++;
   return TREX_OK;
@@ -1189,11 +1225,18 @@ int trex_get_joint_limits(trex_handle* h, float* lower25_host, float* upper25_ho
   return TREX_OK;
 }
 
+int trex_get_action_limits(trex_handle* h, float* lo25_host, float* hi25_host) {
+  if (!h || !lo25_host || !hi25_host) return fail(TREX_ERR_INVALID, "NULL argument%s");
+  if (!h->tau_on) return trex_get_joint_limits(h, lo25_host, hi25_host);
+  for (int i = 0; i < trex::NJ; i++) { lo25_host[i] = -h->tau_max; hi25_host[i] = h->tau_max; }
+  return TREX_OK;
+}
+
 int trex_fill_random_actions(trex_handle* h, float* action_dev, uint32_t seed, uint64_t step, int64_t env_offset, void* stream) {
   if (!h || !action_dev) return fail(TREX_ERR_INVALID, "NULL argument%s");
   CUDA_TRY(cudaSetDevice(h->device));
   const int total = h->n_envs * 7;
-  trex_random_action_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(action_dev, h->d_lower, h->d_upper, seed, step,
+  trex_random_action_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(action_dev, h->d_act_lo, h->d_act_hi, seed, step,
                                                                                      env_offset, h->n_envs);
   CUDA_TRY(cudaGetLastError());
   h->launches++;

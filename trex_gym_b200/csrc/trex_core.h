@@ -286,6 +286,10 @@ TREX_FN void push_of_step(const PushSchedule& S, unsigned seed, unsigned long lo
 // btClamp semantics: comparison based, so a NaN stays a NaN (fmin/fmax would launder it into a bound)
 TREX_FN vf clampv(vf x, float lo, float hi) { return sel(x < lo, lo, sel(x > hi, hi, x)); }
 TREX_FN float clampf(float x, float lo, float hi) { return x < lo ? lo : (x > hi ? hi : x); }
+// joint torque mode: the commanded torque of a joint lane, clipped to [-bound, bound] with fmin / fmax as the targets are
+// clipped; 0 elsewhere.  Unlike np.clip, a NaN command becomes -bound (a NaN target becomes the lower joint limit).  The
+// front phase (applied torque) and the tail phase (reported torque) both call it, so the two agree bit for bit.
+TREX_FN vf clip_torque(vf a, vb is_joint, float bound) { return sel(is_joint, vmin(vmax(a, -bound), bound), 0.0f); }
 
 // world -> base rotation from the base -> world quaternion (x,y,z,w)
 TREX_FN void quat_to_Rb(const float q[4], float Rb[9]) {
@@ -625,11 +629,14 @@ TREX_FN void inward_packed(const Uniform& P, const float* mdl, const int* mdli, 
 // (inward_packed) between two CTA barriers; cta_slabs = slab of warp 0, valid_mask = which warps hold an environment.
 // ENVP: envp = this environment's parameter row (mass scales and friction; the caller passes the row's motor settings)
 // EXTF: *xf = the external wrenches of this substep (record, COM table, scheduled push)
-template <bool PACKED = false, bool ENVP = false, bool EXTF = false>
+// TAU: tau_action = the step's actions [25] name-sorted, the joint torques; clipped to +-tau_bound they enter as explicit joint
+// torques next to the damping (read where they are added, not held in registers across the kinematics)
+template <bool PACKED = false, bool ENVP = false, bool EXTF = false, bool TAU = false>
 TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const float* tasks, const float* cand_p,
                      const int* cand_lane, WarpShared& S, EnvRegs& R, float kp, float kd, float max_imp,
                      StepStats& stats, float* work, WarpShared* cta_slabs = nullptr, int warp_in_cta = 0, int valid_mask = 0,
-                     float* workh = nullptr, const float* envp = nullptr, const ExtWrench* xf = nullptr) {
+                     float* workh = nullptr, const float* envp = nullptr, const ExtWrench* xf = nullptr,
+                     const float* tau_action = nullptr, float tau_bound = 0.0f) {
   const vi lane = lane_id();
   const vb is_joint = lane < NJ;
   const vb is_base = lane == 25;
@@ -755,8 +762,10 @@ TREX_FN int substep(const Uniform& P, const float* mdl, const int* mdli, const f
 
   // Coriolis term c = v x (S qd), S = z rotation: only 4 non-zero components
   const vf c0 = R.qd * v[1], c1 = -(R.qd * v[0]), c3 = R.qd * v[4], c4 = -(R.qd * v[3]);
-  // explicit joint damping torque (pybullet adds -damping*qd before each step)
-  const vf tau_j = -(MDL(F_JDAMP) * R.qd);
+  // explicit joint damping torque (pybullet adds -damping*qd before each step); TAU: plus the commanded torque, written
+  // -(d qd - tau) so that a zero command gives the bits of -(d qd), signed zeros included (tau - d qd would turn -0 into +0)
+  const vf tau_cmd = TAU ? clip_torque(ld_if(tau_action, seli(is_joint, MDLI(IF_OBS_SLOT), 0), is_joint, 0.0f), is_joint, tau_bound) : vf(0.0f);
+  const vf tau_j = TAU ? -(MDL(F_JDAMP) * R.qd - tau_cmd) : -(MDL(F_JDAMP) * R.qd);
 
   TREX_TICK(1)
   // ---- 5. inward pass: articulated inertias ---------------------------------------------------
@@ -2620,12 +2629,14 @@ static_assert(ST_SIG == ST_ACC_ITERS + 3, "front_phase stores the four accumulat
 // ENVP: envp = the environment's parameter row (mass scales, friction, motor gains and impulse bound)
 // EXTF: extf = the environment's wrench record [6][32], com = the COM table [3][32], push = the push schedule,
 // env_id = index of the environment in this launch (P.env_offset + env_id keys the schedule)
-template <bool PACKED = false, bool ENVP = false, bool EXTF = false>
+// TAU (trex_config.actuation = TREX_ACTUATION_TORQUE): the action is the joint torque, clipped to +-tau_max (ENVP: +-the row's
+// element EP_MAX_TORQUE) and applied in this substep; the motors run with kp = kd = 0 and impulse bound 0
+template <bool PACKED = false, bool ENVP = false, bool EXTF = false, bool TAU = false>
 TREX_FN int front_phase(const Uniform& P, const float* mdl, const int* mdli, const float* tasks, const float* cand_p,
                          const int* cand_lane, WarpShared& S, float* rec, float* work, const float* action, bool first_round,
                          WarpShared* cta_slabs = nullptr, int warp_in_cta = 0, int valid_mask = 0, float* workh = nullptr,
                          const float* envp = nullptr, const float* extf = nullptr, const float* com = nullptr,
-                         const PushSchedule* push = nullptr, long long env_id = 0) {
+                         const PushSchedule* push = nullptr, long long env_id = 0, float tau_max = 0.0f) {
   const vi lane = lane_id();
   const vb is_joint = lane < NJ;
   const vi slot = seli(is_joint, MDLI(IF_OBS_SLOT), 0);
@@ -2633,15 +2644,15 @@ TREX_FN int front_phase(const Uniform& P, const float* mdl, const int* mdli, con
   load_env(rec, lane, S, R);
   // np.clip(action, low, high)  (trex_env.py:147); the targets are re-applied every substep (:148-150)
   const vf a = ld_if(action, slot, is_joint, 0.0f);
-  R.tgt = vmin(vmax(a, MDL(F_LOWER)), MDL(F_UPPER));
+  if (!TAU) R.tgt = vmin(vmax(a, MDL(F_LOWER)), MDL(F_UPPER));  // (TAU: R.tgt stays 0, the motors have no gain)
   StepStats st;
   st.iters = 0; st.contacts = 0; st.overflow = 0;
   st.sig = first_round ? 0u : (uint32_t)ldu(rec, ST_SIG);
 #ifdef TREX_PHASES
   for (int i = 0; i < 8; i++) st.phase[i] = 0.0f;
 #endif
-  const float kp = ENVP ? ldu(envp, EP_KP) : P.kp, kd = ENVP ? ldu(envp, EP_KD) : P.kd;
-  const float max_imp = ENVP ? ldu(envp, EP_MAX_IMPULSE) : P.max_impulse;
+  const float kp = TAU ? 0.0f : (ENVP ? ldu(envp, EP_KP) : P.kp), kd = TAU ? 0.0f : (ENVP ? ldu(envp, EP_KD) : P.kd);
+  const float max_imp = TAU ? 0.0f : (ENVP ? ldu(envp, EP_MAX_IMPULSE) : P.max_impulse);
   ExtWrench xf;
   if (EXTF) {
     xf.rec = extf;
@@ -2649,8 +2660,9 @@ TREX_FN int front_phase(const Uniform& P, const float* mdl, const int* mdli, con
     // the step count as the tail kernel left it: steps completed in this episode
     push_of_step(*push, P.seed, (unsigned long long)(P.env_offset + env_id), ldu(rec, ST_EPISODE), ldu(rec, ST_STEP), xf);
   }
-  const int deferred = substep<PACKED, ENVP, EXTF>(P, mdl, mdli, tasks, cand_p, cand_lane, S, R, kp, kd, max_imp, st, work, cta_slabs,
-                                                   warp_in_cta, valid_mask, workh, envp, EXTF ? &xf : nullptr);
+  const int deferred = substep<PACKED, ENVP, EXTF, TAU>(P, mdl, mdli, tasks, cand_p, cand_lane, S, R, kp, kd, max_imp, st, work,
+                                                        cta_slabs, warp_in_cta, valid_mask, workh, envp, EXTF ? &xf : nullptr, action,
+                                                        TAU ? (ENVP ? ldu(envp, EP_MAX_TORQUE) : tau_max) : 0.0f);
   store_env(rec, lane, S, R);  // deferred: positions unchanged, velocities after the unconstrained update
   const float it0 = first_round ? 0.0f : ldu(rec, ST_ACC_ITERS), ov0 = first_round ? 0.0f : ldu(rec, ST_ACC_OVERFLOW);
   vf acc = 0.0f;
@@ -2719,11 +2731,14 @@ TREX_FN void heavy_phase(const Uniform& P, float* scratch, tmem_t tm, const floa
 //   obs : [75] q | qd | motor torque   aux : [TREX_AUX_STRIDE] head xyz, lifting/station/energy, PGS iterations, contacts
 // ENVP: envp = the environment's parameter row (mass scales and friction apply to the reset step; its motor gains stay zero).
 // ranges != nullptr: the randomizer is on -- every reset first draws a new row (draw_env_params).
-template <bool ENVP = false>
+// TAU: action = the step's actions [25] name-sorted, tau_max = the torque bound without ENVP: the applied torque the reward and
+// the observation report (and record [63:88] keeps) is the clipped command, not the motors' impulse / dt.  A reset reports
+// the reset step's own value.
+template <bool ENVP = false, bool TAU = false>
 TREX_FN void tail_phase(const Uniform& P, const float* mdl, const int* mdli, const float* tasks, const float* cand_p,
                         const int* cand_lane, WarpShared& S, float* rec, float* obs, float* reward, uint8_t* done,
                         float* aux, bool force_reset, long long env_id, float* envp = nullptr, const float* ranges = nullptr,
-                        double dt = 0.0) {
+                        double dt = 0.0, const float* action = nullptr, float tau_max = 0.0f) {
   const vi lane = lane_id();
   const vb is_joint = lane < NJ;
   const vi slot = seli(is_joint, MDLI(IF_OBS_SLOT), 0);
@@ -2731,6 +2746,10 @@ TREX_FN void tail_phase(const Uniform& P, const float* mdl, const int* mdli, con
   load_env(rec, lane, S, R);
   bool is_done = false;
   if (!force_reset) {
+    if (TAU) {
+      R.tau = clip_torque(ld_if(action, slot, is_joint, 0.0f), is_joint, ENVP ? ldu(envp, EP_MAX_TORQUE) : tau_max);
+      st_if(rec, seli(is_joint, lane, 0) + ST_TAU, R.tau, is_joint);
+    }
     const float step_count = ldu(rec, ST_STEP) + 1.0f;
     float head[3], terms[3], rew;
     bool bad;

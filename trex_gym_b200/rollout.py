@@ -38,6 +38,10 @@ class RolloutBuffer:
     """Time-major device buffers ``[T, N, ...]`` filled in place by :class:`TrexBatchSim`."""
 
     def __init__(self, sim: TrexBatchSim, horizon: int):
+        if getattr(sim, "actuation", "position") != "position":
+            # the on-device PPO loop drives motor targets only
+            raise ValueError("RolloutBuffer supports position-actuated simulators only; this one was created with "
+                             "actuation=%r" % (sim.actuation,))
         self.sim, self.T, self.N = sim, int(horizon), sim.num_envs
         dev = sim.device
         f32, u8 = torch.float32, torch.uint8

@@ -28,7 +28,13 @@ class TrexBatchSim:
                  seed: int = 0, warps_per_block: int | None = None, reset_mode: int = 0, env_offset: int = 0,
                  deferred_solve: bool = True, defer_contacts: bool = True, heavy_solver: bool = True,
                  heavy_share_div: int = 0, pipelines: int = 0, heavy_memory: int = 0, chunk_envs: int = 0, contact_memory: int = 0,
-                 env_params: bool = False, external_forces: bool = False):
+                 env_params: bool = False, external_forces: bool = False, actuation: str = "position"):
+        """``actuation``: ``"position"`` (default: an action is a motor target, clipped to the joint limits) or ``"torque"``
+        (joint torque control: an action is the joint torque in N m, clipped to the model's ``motor_max_torque`` -- or an
+        ``env_params`` row's element 29 -- and applied in every physics substep; the motors have no gain or strength; the
+        observation's torque block and the energy term report the clipped command).  See ``include/trex_b200.h``."""
+        if actuation not in _native.ACTUATION:
+            raise ValueError("actuation must be 'position' or 'torque', not %r" % (actuation,))
         if not torch.cuda.is_available():
             raise RuntimeError("trex_gym_b200 needs a CUDA device (no CPU fallback)")
         dev = torch.device(device if not isinstance(device, int) else "cuda:%d" % device)
@@ -63,6 +69,8 @@ class TrexBatchSim:
         self.env_params = bool(env_params)
         cfg.external_forces = int(bool(external_forces))  # per-environment external wrenches (set_external_forces)
         self.external_forces = bool(external_forces)
+        cfg.actuation = _native.ACTUATION[actuation]
+        self.actuation = actuation
         blob = self.model.blob()
         h = ctypes.c_void_p()
         idx = dev.index if dev.index is not None else torch.cuda.current_device()
@@ -80,7 +88,15 @@ class TrexBatchSim:
         lo = np.zeros(_native.NUM_JOINTS, np.float32)
         hi = np.zeros(_native.NUM_JOINTS, np.float32)
         _native.check(self._L.trex_get_joint_limits(self._h, lo.ctypes.data, hi.ctypes.data), "trex_get_joint_limits")
-        self.action_low, self.action_high = lo, hi
+        self.action_low, self.action_high = lo, hi  # the joint limits (the observation space uses them in both modes)
+
+    def action_limits(self) -> tuple[np.ndarray, np.ndarray]:
+        """(low, high) [25] of the action space, name-sorted: the joint limits in position mode, -/+ the model's
+        ``motor_max_torque`` in torque mode."""
+        lo = np.zeros(_native.NUM_JOINTS, np.float32)
+        hi = np.zeros(_native.NUM_JOINTS, np.float32)
+        _native.check(self._L.trex_get_action_limits(self._h, lo.ctypes.data, hi.ctypes.data), "trex_get_action_limits")
+        return lo, hi
 
     # -- lifetime ---------------------------------------------------------------------------
     def close(self):

@@ -47,7 +47,10 @@ class TrexBulletEnv(spaces.Env):
     metadata = {"render.modes": ["human", "rgb_array"], "video.frames_per_second": 50}
 
     def __init__(self, urdf_path=None, action_repeat=1, distance_weight=1.0, energy_weight=0.005, drift_weight=0.002,
-                 render=False, device=0, model=None, contacts=True, contact_model="points", literal_reference=False):
+                 render=False, device=0, model=None, contacts=True, contact_model="points", literal_reference=False,
+                 actuation="position"):
+        """``actuation="torque"``: an action is the joint torque (N m) of every joint, applied in every physics substep
+        (``TrexBatchSim``); ``action_space`` is then -/+ the motor torque bound."""
         self._time_step = 0.01
         self._urdf_path = urdf_path
         self._action_repeat = action_repeat
@@ -81,7 +84,7 @@ class TrexBulletEnv(spaces.Env):
         # action_repeat * NUM_SUBSTEPS physics steps (trex_env.py:148-150)
         self._sim = TrexBatchSim(1, device=device, model=mdl, num_substeps=NUM_SUBSTEPS,
                                  distance_weight=distance_weight, energy_weight=energy_weight,
-                                 drift_weight=drift_weight, contacts=contacts)
+                                 drift_weight=drift_weight, contacts=contacts, actuation=actuation)
         self._repeat_env_steps = int(action_repeat)
         self.model = None
         self.np_random = None
@@ -141,12 +144,14 @@ class TrexVecEnv(object):
 
     def __init__(self, num_envs, urdf_path=None, distance_weight=1.0, energy_weight=0.005, drift_weight=0.002,
                  device=0, model=None, num_substeps=NUM_SUBSTEPS, max_episode_steps=0, contacts=True, seed=0, contact_model="points",
-                 literal_reference=False, randomize=None, pushes=None):
+                 literal_reference=False, randomize=None, pushes=None, actuation="position"):
         """``randomize``: None, or a dict of parameter name -> (low, high) -- ``mass_scale`` (a scale, or {body: scale}),
         ``friction``, ``kp``, ``kd``, ``max_torque`` -- drawn per environment at every reset (``TrexBatchSim.set_env_param_ranges``);
         parameters not named keep the model's value.
         ``pushes``: None, or the keyword arguments of ``TrexBatchSim.set_push_schedule`` (``body``, ``interval``, ``duration``,
-        ``probability``, ``force=(lo, hi)``, ``first_step``): random horizontal pushes drawn on the device."""
+        ``probability``, ``force=(lo, hi)``, ``first_step``): random horizontal pushes drawn on the device.
+        ``actuation``: ``"position"`` (motor targets) or ``"torque"`` (joint torques, ``action_space`` -/+ the motor torque
+        bound; see ``TrexBatchSim``)."""
         if literal_reference:  # see TrexBulletEnv
             contacts = False
             mdl = model if model is not None else load_builtin("literal")
@@ -155,14 +160,15 @@ class TrexVecEnv(object):
         self.sim = TrexBatchSim(num_envs, device=device, model=mdl, num_substeps=num_substeps,
                                 distance_weight=distance_weight, energy_weight=energy_weight, drift_weight=drift_weight,
                                 max_episode_steps=max_episode_steps, contacts=contacts, seed=seed, env_params=randomize is not None,
-                                external_forces=pushes is not None)
+                                external_forces=pushes is not None, actuation=actuation)
         if randomize is not None:
             self.sim.set_env_param_ranges({k: v[0] for k, v in randomize.items()}, {k: v[1] for k, v in randomize.items()})
         if pushes is not None:
             self.sim.set_push_schedule(**pushes)
         self.num_envs = int(num_envs)
-        lo, hi = self.sim.action_low, self.sim.action_high
-        self.action_space = spaces.Box(low=lo, high=hi, dtype=np.float32)
+        alo, ahi = self.sim.action_limits()
+        self.action_space = spaces.Box(low=alo, high=ahi, dtype=np.float32)
+        lo, hi = self.sim.action_low, self.sim.action_high  # the joint limits bound the observed positions in either mode
         n = lo.shape[0]
         self.observation_space = spaces.Box(low=np.concatenate([lo, np.full(2 * n, -1.0e12, np.float32)]),
                                             high=np.concatenate([hi, np.full(2 * n, 1.0e12, np.float32)]), dtype=np.float32)

@@ -76,8 +76,9 @@ class TrexRobot(object):
         return self.sim.action_low.astype(np.float64).tolist(), self.sim.action_high.astype(np.float64).tolist()
 
     def get_action_limits(self):
-        lo, hi = self._get_joint_limits()  # trex_robot.py:424-433
-        return np.array(lo), np.array(hi)
+        """The joint limits (trex_robot.py:424-433); -/+ the motor torque bound on a torque-actuated simulator."""
+        lo, hi = self.sim.action_limits()
+        return lo.astype(np.float64), hi.astype(np.float64)
 
     def get_observation_limits(self):
         n = len(self._revolute_joint_indices)  # trex_robot.py:348-357
@@ -91,7 +92,8 @@ class TrexRobot(object):
         """trex_robot.py:413-422: position targets for the 25 motors (kp = 5e-3, kd = 0.1, 3e5 N m), name-sorted order.
         Like ``setJointMotorControlArray`` the targets persist: they are written to this environment's row of the
         simulator's target buffer and every following physics substep (``sim.step()`` without an argument, which is
-        what ``TrexBulletEnv.step`` calls, trex_env.py:148-150) servoes towards them until the next call."""
+        what ``TrexBulletEnv.step`` calls, trex_env.py:148-150) servoes towards them until the next call.  On a simulator
+        created with ``actuation="torque"`` the values are joint torques (N m), applied in every substep instead."""
         n = len(self._revolute_joint_indices)
         a = np.asarray(actions, dtype=np.float32).reshape(-1)[:n]  # the reference slices actions[:num_joints]
         if a.shape != (n,):
